@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the typing hot path (stage a: per-read allele compatibility -> Gene_cmpt/Gene_counts, stage b: EM).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--samples S] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--samples S] [--impl reference] [--dump-outputs DIR]
 
 Workload = BASELINE.json configs[1]: HLA-A/B/C/DQA1/DQB1/DRB1, paired-end 2x100 bp, 30x, synthetic database of the
 named shape (SURVEY.md 8d) and reads drawn from a random diploid genotype per sample with 0.5 % sequencing
@@ -308,6 +308,9 @@ def run_oversized(args):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench: --dump-outputs of the oversized workload needs one GPU (with more, the EM of the "
+                         "read-sharded unit runs outside the batch)")
     if world > 1:
         import torch.distributed as dist
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
@@ -390,6 +393,8 @@ def run_oversized(args):
     h2d, d2h = ctypes.c_int64(0), ctypes.c_int64(0)
     L.hgt_profile_read(ctx, stage_ms, stage_n, ctypes.byref(h2d), ctypes.byref(d2h))
     stage = {n: stage_ms[i] / args.steps for i, n in enumerate(STAGES)}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [batch])
     summ = batch.unit_summary(0)
     C, it = summ["n_classes"][0], (em_state["iters"] if world > 1 else summ["em_iters"][0])
     em_bytes = it * (3 * C * (table.wp * 8 + 8) + 6 * table.A * 8)
@@ -651,6 +656,8 @@ def run_workload(args):
     h2d, d2h = ctypes.c_int64(0), ctypes.c_int64(0)
     L.hgt_profile_read(ctx, stage_ms, stage_n, ctypes.byref(h2d), ctypes.byref(d2h))
     stage = {n: stage_ms[i] / args.steps for i, n in enumerate(STAGES)}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, batches)
     example = batches[0].top_calls(2)[0]
     parity_batch = batches[0]
     for b in batches[1:]:
@@ -773,6 +780,75 @@ def oversized_subrecord(args, rank, world):
     return sub
 
 
+DUMP_LIMIT = 64 << 20  # bytes of all arrays --dump-outputs writes
+DUMP_UNITS = 64  # units whose per-allele and per-class arrays are written (a seeded sample when the step has more)
+DUMP_TOP = 5  # calls per unit in top_calls.npy
+
+
+def dump_outputs(out_dir, batches):
+    """--dump-outputs: what the timed path computed in its last step (the prepared batches after execute + finish), as
+    float64 arrays out_dir/<name>.npy, so that two builds can be compared output for output on the same seeded inputs.
+    Units are numbered in batch order.  For every unit:
+      unit_summary   [U, 10]     reads, pairs, classes of the 4 tables, EM iterations (2 levels), EM status (2 levels)
+      top_calls      [U, 5, 2]   allele index and abundance of the 5 best calls; -1 and 0 where the unit has fewer
+    For a fixed sample of at most DUMP_UNITS units (sample_units: their numbers, ascending):
+      abundance      [sum A]     Gene_prob of every allele of the unit's locus, 0 where the allele has none
+      allele_counts  [sum A, 4]  Gene_counts of each table
+      classes        [sum C, 4]  per class, table after table: read pairs, member alleles, first pair, and a 48-bit
+                                 BLAKE2b hash of its member bitset (the packed words would exceed the size budget)"""
+    import hashlib
+
+    import numpy as np
+    units = [(b, u) for b in batches for u in range(len(b.unit_locus))]
+    index = {}
+
+    def allele_index(t):
+        if id(t) not in index:
+            index[id(t)] = {n: i for i, n in enumerate(t.names)}
+        return index[id(t)]
+
+    summary = np.zeros((len(units), 10))
+    top = np.zeros((len(units), DUMP_TOP, 2))
+    top[:, :, 0] = -1
+    k = 0
+    for b in batches:
+        for u, calls in enumerate(b.top_calls(DUMP_TOP)):
+            s = b.unit_summary(u)
+            summary[k] = [s["num_reads"], s["num_pairs"]] + s["n_classes"] + s["em_iters"] + s["em_status"]
+            names = allele_index(b.loci[b.unit_locus[u]])
+            for j, (allele, prob) in enumerate(calls):
+                top[k, j] = names[allele], prob
+            k += 1
+    pick = np.sort(np.random.default_rng(0).choice(len(units), min(len(units), DUMP_UNITS), replace=False))
+    abundance, counts, classes = [], [], []
+    for k in pick:
+        b, u = units[k]
+        t = b.loci[b.unit_locus[u]]
+        names = allele_index(t)
+        prob = np.zeros(t.A)
+        for allele, p in b.unit_calls(u):
+            prob[names[allele]] = p
+        abundance.append(prob)
+        cnt = np.zeros((t.A, 4))
+        for tb in range(4):
+            bits, n_pairs, first, acount, _ = b.unit_table(u, tb)
+            cnt[:, tb] = acount
+            members = [int.from_bytes(hashlib.blake2b(row.tobytes(), digest_size=6).digest(), "little") for row in bits]
+            classes.append(np.stack([n_pairs, np.bitwise_count(bits).sum(axis=1), first, np.asarray(members, np.float64)],
+                                    axis=1))
+        counts.append(cnt)
+    out = {"unit_summary": summary, "top_calls": top, "sample_units": pick, "abundance": np.concatenate(abundance),
+           "allele_counts": np.concatenate(counts), "classes": np.concatenate(classes)}
+    out = {n: np.ascontiguousarray(a, np.float64) for n, a in out.items()}
+    size = sum(a.nbytes for a in out.values())
+    if size > DUMP_LIMIT:
+        raise SystemExit("bench: --dump-outputs would write %d bytes, more than %d" % (size, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in out.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a)
+    sys.stderr.write("bench: %d arrays, %d bytes, in %s\n" % (len(out), size, out_dir))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -791,7 +867,14 @@ def main():
     ap.add_argument("--oversized-sub-reads", type=int, default=10000000,
                     help="reads of the read-sharded oversized locus reported as the `oversized` sub-record of the default "
                          "line (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's units) as DIR/<name>.npy; "
+                         "the oversized workload on one GPU only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path, not of --impl reference")
     if args.impl == "reference":
         return run_reference_arm(args)
     if args.workload == "oversized":
@@ -881,6 +964,8 @@ def main():
     h2d, d2h = ctypes.c_int64(0), ctypes.c_int64(0)
     L.hgt_profile_read(ctx, stage_ms, stage_n, ctypes.byref(h2d), ctypes.byref(d2h))
     stage = {n: stage_ms[i] / args.steps for i, n in enumerate(STAGES)}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [batch])
     # EM bookkeeping
     # SURVEY.md 8d: per loop iteration min(bit matrix, CSR) evaluated on the actual class tables:
     #   bit matrix 3 C (wp 8 + 8) + 6 A 8,   CSR 3 (4 nnz + 12 C) + 6 A 8   (nnz = members over all classes)

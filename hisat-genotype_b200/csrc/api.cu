@@ -2,10 +2,26 @@
 #include <stdarg.h>
 
 #include <algorithm>
+#include <mutex>
+#include <utility>
 
 #include "common.cuh"
 
 static thread_local char g_err[1024] = "";
+
+cudaError_t hgt_smem_at_least(const void *kernel, size_t bytes) {
+    static std::mutex mu;
+    static std::map<std::pair<int, const void *>, size_t> limit;  // (device, kernel) -> limit set so far
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    std::lock_guard<std::mutex> lock(mu);
+    size_t &cur = limit[{dev, kernel}];
+    if (cur >= bytes) return cudaSuccess;
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e == cudaSuccess) cur = bytes;
+    return e;
+}
 
 void hgt_set_error(const char *fmt, ...) {
     va_list ap;

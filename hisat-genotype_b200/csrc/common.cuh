@@ -49,6 +49,12 @@ void hgt_set_error(const char *fmt, ...);
 // the stream has passed this point (the rule of cudaMemcpyAsync).
 cudaError_t hgt_small_h2d(void *dst_dev, const void *src_pinned, size_t bytes, cudaStream_t st);
 
+// Raises the dynamic shared-memory limit of `kernel` on the current device to at least `bytes`; never lowers it.  The
+// limit is a property of the kernel for the whole process, and batches on other host threads (one context each,
+// typing_core.BatchPipeline) launch the same kernels with their own sizes: a thread that set the exact size of its own
+// launch could lower the limit between another thread's set and launch, and that launch would fail.
+cudaError_t hgt_smem_at_least(const void *kernel, size_t bytes);
+
 #include <chrono>
 struct HostTimer {  // wall-clock bracket of one host stage, accumulated into ctx->host_ms (bench.py reads it)
     hgt_ctx *ctx;

@@ -1629,7 +1629,7 @@ int em_launch(hgt_ctx *ctx, cudaStream_t st, const EmArgs *d_args, int grid, int
         case 8: kern = em_kernel<8, COOP>; break;
         default: kern = em_kernel<16, COOP>; break;
     }
-    HGT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    HGT_CUDA(hgt_smem_at_least((const void *)kern, smem));
     if (COOP) {
         void *params[] = {(void *)&d_args};
         HGT_CUDA(cudaLaunchCooperativeKernel((void *)kern, dim3(grid), dim3(EM_THREADS), params, smem, st));
@@ -2134,7 +2134,7 @@ static int em_partial_impl(hgt_ctx *ctx, void *stream, const uint64_t *class_bit
         case 8: kern = em_part_kernel<8>; break;
         default: kern = em_part_kernel<16>; break;
     }
-    HGT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem));
+    HGT_CUDA(hgt_smem_at_least((const void *)kern, plan.smem));
     kern<<<G, EM_THREADS, plan.smem, st>>>(a, mode, p_in);
     HGT_CUDA(cudaGetLastError());
     em_part_reduce_kernel<<<(n_alleles + 255) / 256, 256, 0, st>>>(G, n_alleles, (int)Apad, mode, a.part_acc, a.part_aux,

@@ -1953,12 +1953,8 @@ static int reads_execute(hgt_batch *b, cudaStream_t st) {
     // the walk reads its lines straight from global memory: after the three-pass split the TMA-staged image measured
     // slower for it (5.97 vs 4.69 ms of walk per step); HGT_WALK_STAGE=1 brings it back for A/B runs
     static const int walk_stage_off = !getenv("HGT_WALK_STAGE") && !getenv("HGT_WALK_STAGE_ON");
-    static int stage_attr = 0;
-    if (stage_attr < stage_bytes) {
-        HGT_CUDA(cudaFuncSetAttribute(hgtk::parse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, stage_bytes));
-        HGT_CUDA(cudaFuncSetAttribute(hgtk::walk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, stage_bytes));
-        stage_attr = stage_bytes;
-    }
+    HGT_CUDA(hgt_smem_at_least((const void *)hgtk::parse_kernel, stage_bytes));
+    HGT_CUDA(hgt_smem_at_least((const void *)hgtk::walk_kernel, stage_bytes));
     const int stage_grid = (int)std::max<int64_t>(1, std::min<int64_t>((N + hgtk::STAGE_LINES - 1) / hgtk::STAGE_LINES,
                                                                      (int64_t)ctx->sm_count * stage_ctas));
     // The pileup is its own pass (warp per line, 8 CTAs of 256 threads per SM).  HGT_PILEUP_FUSED=1 runs it inside the parse
@@ -2427,12 +2423,7 @@ static void em_problems(hgt_ctx *ctx, int n_launch, LocusBatch &lb, int table, c
 }
 
 static int launch_class_sort(hgt_ctx *ctx, cudaStream_t st, LocusBatch &lb, int table) {
-    static bool attr = false;
-    const int smem = 2 * CLASS_SORT_MAX * 4;
-    if (!attr) {
-        HGT_CUDA(cudaFuncSetAttribute(class_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        attr = true;
-    }
+    HGT_CUDA(hgt_smem_at_least((const void *)class_sort_kernel, 2 * CLASS_SORT_MAX * 4));
     int64_t max_pairs = 1;
     for (size_t ut = 0; ut + 1 < lb.ut_base.size(); ut++) max_pairs = std::max<int64_t>(max_pairs, lb.ut_base[ut + 1] - lb.ut_base[ut]);
     const int need = 2 * 4 * (int)std::min<int64_t>(max_pairs, CLASS_SORT_MAX);  // classes of a region <= its pairs

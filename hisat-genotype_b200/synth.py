@@ -311,12 +311,20 @@ _sim = None
 def _simlib():
     global _sim
     if _sim is None:
+        import atexit
         import ctypes
+        import shutil
         import subprocess
+        import tempfile
         tools = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools")
         so = os.path.join(tools, "libhgtsim.so")
         if not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(os.path.join(tools, "simgen.cpp")):
-            subprocess.check_call(["make", "-s", "-C", tools])
+            # not built by __graft_entry__.build() or older than its source: compile a private copy, because the
+            # source tree may be read-only
+            tmp = tempfile.mkdtemp(prefix="hgtsim-")
+            atexit.register(shutil.rmtree, tmp, True)
+            so = os.path.join(tmp, "libhgtsim.so")
+            subprocess.check_call(["make", "-s", "-C", tools, "OUT=" + so])
         L = ctypes.CDLL(so)
         L.hgtsim_locus_create.restype = ctypes.c_void_p
         L.hgtsim_locus_create.argtypes = [ctypes.c_char_p, ctypes.c_int, ctypes.c_char_p, ctypes.c_int] + \

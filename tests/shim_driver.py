@@ -1,6 +1,6 @@
 """Child process of tests/test_gpu_shim.py: the drop-in modules (hisat-genotype_b200/shim) in front of a STAND-IN reference
-tree (the GPU box has no /root/reference), typing() called the way genotyping_locus calls it, golden alignments as the
-"BAM" behind the rig's stand-in samtools; prints the report files as JSON.
+tree, typing() called the way genotyping_locus calls it, golden alignments as the "BAM" behind the rig's stand-in
+samtools; prints the report files as JSON.
 
 usage: shim_driver.py <golden name> <work dir> [native]"""
 import json
@@ -37,6 +37,15 @@ def genotyping_locus(*args, **kwargs):
 '''
 
 
+def write_stand_in_modules(mods):
+    """The three reference modules the drop-in modules load, with the attributes their path touches."""
+    os.makedirs(mods, exist_ok=True)
+    for fn, text in (("hisatgenotype_typing_common.py", FAKE_COMMON), ("hisatgenotype_typing_process.py", FAKE_PROCESS),
+                     ("hisatgenotype_typing_core.py", FAKE_CORE)):
+        with open(os.path.join(mods, fn), "w") as f:
+            f.write(text)
+
+
 def main():
     name, work = sys.argv[1], sys.argv[2]
     native = len(sys.argv) > 3 and sys.argv[3] == "native"  # HGT_NATIVE_INTAKE=1 and NO samtools anywhere
@@ -50,13 +59,10 @@ def main():
     ref = os.path.join(work, "reference")
     mods = os.path.join(ref, "hisatgenotype_modules")
     os.makedirs(os.path.join(ref, "hisat2"), exist_ok=True)
-    os.makedirs(mods, exist_ok=True)
+    write_stand_in_modules(mods)
     first = g["reports"][sorted(g["reports"])[0]].split("\n")
     open(os.path.join(ref, "hisat2", "VERSION"), "w").write(first[1][len("# HISAT2 - "):] + "\n")
     open(os.path.join(ref, "VERSION"), "w").write(first[3][len("# HISAT-genotype - "):] + "\n")
-    for fn, text in (("hisatgenotype_typing_common.py", FAKE_COMMON), ("hisatgenotype_typing_process.py", FAKE_PROCESS),
-                     ("hisatgenotype_typing_core.py", FAKE_CORE)):
-        open(os.path.join(mods, fn), "w").write(text)
     bindir = os.path.join(work, "bin")
     os.makedirs(bindir, exist_ok=True)
     tool = os.path.join(bindir, "samtools")

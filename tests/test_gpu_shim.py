@@ -1,8 +1,8 @@
 """Drop-in boundary on the GPU: hisat-genotype_b200/shim in front of a reference tree, typing() reached through the
 reference's genotyping_locus -> module-global typing (core:2582, 2655), golden alignments as the alignment file, the
-FULL `.report` (header included) equal to what the unmodified reference wrote (tests/golden).  The GPU box has no
-/root/reference, so the child process builds a stand-in tree with the attributes the path touches (shim_driver.py);
-tests/test_shim.py runs the same modules against the real reference on the CPU side."""
+FULL `.report` (header included) equal to what the unmodified reference wrote (tests/golden).  The child process builds
+a stand-in reference tree with the attributes the path touches (shim_driver.py); tests/test_shim.py checks names,
+dispatch and the CLI on the CPU side, against a real reference tree when $HGT_REFERENCE names one."""
 import json
 import os
 import subprocess

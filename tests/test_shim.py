@@ -1,6 +1,12 @@
-"""CPU-side checks of the drop-in modules (hisat-genotype_b200/shim) against the REAL reference tree, when it is present
-(this container: /root/reference; the GPU box has none - there tests/test_gpu_shim.py uses a stand-in tree).  No GPU call
-is made: the checks are about names, dispatch and the unchanged CLI."""
+"""CPU-side checks of the drop-in modules (hisat-genotype_b200/shim) in front of a reference tree.  No GPU call is made:
+the checks are about names, dispatch and the unchanged CLI.  The tree is $HGT_REFERENCE when set (a hisat-genotype
+checkout); otherwise a stand-in holding the modules of tests/shim_driver.py and an entry script that imports
+genotyping_locus by name and parses its options, as the reference's `hisatgenotype` does (hisatgenotype:36).
+
+What the stand-in can and cannot show: the dispatch, pass-through and re-export checks run on the shim's own code
+either way, but "no name of the reference is missing" is then checked against the stand-in's few names, and the CLI
+test then only shows that `from hisatgenotype_typing_core import genotyping_locus` resolves through the shim (the
+stand-in script declares --locus-list itself).  Set $HGT_REFERENCE to a reference checkout for those two checks."""
 import json
 import os
 import subprocess
@@ -9,13 +15,32 @@ import sys
 import pytest
 
 from conftest import ROOT
+from shim_driver import write_stand_in_modules
 
-REF = os.environ.get("HGT_REFERENCE", "/root/reference")
-MODS = os.path.join(REF, "hisatgenotype_modules")
 SHIM = os.path.join(ROOT, "hisat-genotype_b200", "shim")
 
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(MODS, "hisatgenotype_typing_core.py")),
-                                reason="reference tree not present")
+STAND_IN_CLI = r'''
+import argparse
+import hisatgenotype_typing_common as typing_common
+from hisatgenotype_typing_core import genotyping_locus
+parser = argparse.ArgumentParser(description="HISAT-genotype")
+parser.add_argument("--base", default="hla")
+parser.add_argument("--locus-list", default="")
+args = parser.parse_args()
+'''
+
+
+@pytest.fixture(scope="module")
+def mods(tmp_path_factory):
+    """The reference tree's hisatgenotype_modules directory."""
+    ref = os.environ.get("HGT_REFERENCE", "")
+    if not ref:
+        ref = str(tmp_path_factory.mktemp("reference"))
+        write_stand_in_modules(os.path.join(ref, "hisatgenotype_modules"))
+        with open(os.path.join(ref, "hisatgenotype"), "w") as f:
+            f.write(STAND_IN_CLI)
+    return os.path.join(ref, "hisatgenotype_modules")
+
 
 CHILD = r'''
 import json, sys, warnings
@@ -65,8 +90,8 @@ print("CHILD " + json.dumps(out))
 '''
 
 
-def run_child(disable):
-    env = dict(os.environ, PYTHONPATH=SHIM + os.pathsep + MODS, PYTHONHASHSEED="0")
+def run_child(mods, disable):
+    env = dict(os.environ, PYTHONPATH=SHIM + os.pathsep + mods, PYTHONHASHSEED="0")
     env.pop("HGT_DISABLE", None)
     if disable:
         env["HGT_DISABLE"] = "1"
@@ -75,8 +100,8 @@ def run_child(disable):
     return json.loads([x for x in r.stdout.splitlines() if x.startswith("CHILD ")][-1][6:])
 
 
-def test_drop_in_modules_wrap_the_reference():
-    o = run_child(False)
+def test_drop_in_modules_wrap_the_reference(mods):
+    o = run_child(mods, False)
     assert o["common_file"].startswith(SHIM) and o["core_file"].startswith(SHIM)
     assert o["missing_common"] == [] and o["missing_core"] == []
     assert o["single_abundance_module"] == "hisatgenotype_b200.typing_common"
@@ -89,19 +114,19 @@ def test_drop_in_modules_wrap_the_reference():
     assert o["short_call"] == "TypeError"
 
 
-def test_hgt_disable_is_a_pure_pass_through():
-    o = run_child(True)
+def test_hgt_disable_is_a_pure_pass_through(mods):
+    o = run_child(mods, True)
     assert o["missing_common"] == [] and o["missing_core"] == []
     assert o["single_abundance_module"].startswith("_hgt_ref_")
     assert o["typing_module"].startswith("_hgt_ref_")
     assert o["other_names_identical"]
 
 
-def test_reference_cli_starts_with_the_drop_in_modules_first():
+def test_reference_cli_starts_with_the_drop_in_modules_first(mods):
     """`hisatgenotype` imports genotyping_locus by name (hisatgenotype:36): with the shim directory first on PYTHONPATH the
     unchanged CLI must still come up (argument parser only; no database, no GPU)."""
-    cli = os.path.join(REF, "hisatgenotype")
-    env = dict(os.environ, PYTHONPATH=SHIM + os.pathsep + MODS)
+    cli = os.path.join(os.path.dirname(mods), "hisatgenotype")
+    env = dict(os.environ, PYTHONPATH=SHIM + os.pathsep + mods)
     r = subprocess.run([sys.executable, "-W", "ignore", cli, "--help"], env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr[-2000:]
     assert "--locus-list" in r.stdout
