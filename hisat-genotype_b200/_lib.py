@@ -24,6 +24,17 @@ class HgtError(RuntimeError):
         self.code = code
 
 
+EM_FORM_COMPACT, EM_FORM_STREAM, EM_FORM_COOP = 0, 1, 2
+EM_FORM_NAMES = {EM_FORM_COMPACT: "compact", EM_FORM_STREAM: "stream", EM_FORM_COOP: "coop"}
+
+
+class EmForm(ctypes.Structure):
+    """hgt_em_form_info (include/hgt.h)."""
+    _fields_ = [("form", ctypes.c_int32), ("grid", ctypes.c_int32), ("na", ctypes.c_int32), ("slab_rows", ctypes.c_int32),
+                ("slab_bytes", ctypes.c_int64), ("merge", ctypes.c_int32), ("collapse", ctypes.c_int32),
+                ("batch_coop", ctypes.c_int32)]
+
+
 _lib = None
 _ctx = {}
 
@@ -61,6 +72,8 @@ def lib():
         L.hgt_em_dev.restype = c_int
         L.hgt_em_dev.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_i32, c_i32, c_i32, c_void_p, c_i32, c_i32,
                                  c_i32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]
+        L.hgt_em_form.restype = c_int
+        L.hgt_em_form.argtypes = [c_void_p, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, P(EmForm)]
         L.hgt_batch_add_units.restype = c_i64
         L.hgt_batch_add_units.argtypes = [c_void_p, c_i64, c_void_p, c_void_p, c_void_p]
         L.hgt_batch_abundances.restype = c_int
@@ -168,6 +181,14 @@ class PinnedText:
             self.close()
         except Exception:
             pass
+
+
+def em_form(n_classes, n_alleles, wp=None, has_lengths=False, n_ctas=0, a_live_max=0, n_problems=1, device=None):
+    """The form hgt_em_dev runs a problem of this size in (hgt_em_form): EmForm."""
+    out = EmForm()
+    check(lib().hgt_em_form(ctx(device), int(n_classes), int(n_alleles), int(wp or row_pitch(n_alleles)),
+                            1 if has_lengths else 0, int(n_ctas), int(a_live_max), int(n_problems), ctypes.byref(out)))
+    return out
 
 
 def ptr(a):

@@ -875,6 +875,16 @@ __device__ void compact_loop(const EmArgs &a, Compact &c, double &diff, int &ite
 constexpr int DEDUP_CAP = 8192;         // hash slots; at most 6144 live alleles (load factor 0.75)
 constexpr int DEDUP_MAX_LIVE = 6144;
 constexpr int DEDUP_COLS = 4;           // 64-allele word columns per warp: wp <= 128
+// Sizes under which an allele-compacted problem without lengths merges identical columns (kernel and hgt_em_form).
+__host__ __device__ inline bool em_merge_fits(int wp, int A_live_max, size_t slab_bytes) {
+    return wp <= DEDUP_COLS * EM_WARPS && A_live_max <= DEDUP_MAX_LIVE && slab_bytes >= (size_t)wp * 64 * 12 + DEDUP_CAP * 4 &&
+           slab_bytes >= (size_t)wp * 8 * 32;
+}
+// Whether a one-CTA problem can switch to the <= 64-key loop: the allele-compacted layout has buffers for it, the
+// streaming layout re-uses its staged vector and slab (C class masks, counts and weights) (kernel and hgt_em_form).
+__host__ __device__ inline bool em_collapse_fits(bool compacted, int C, int wp, int slab_rows) {
+    return compacted || (size_t)C * 24 + 64 * 64 <= p_slots((size_t)wp * 64) * 8 + (size_t)slab_rows * 8 + (size_t)slab_rows * wp * 8;
+}
 __device__ __forceinline__ unsigned long long dedup_mix(unsigned long long x) {
     x ^= x >> 33; x *= 0xff51afd7ed558ccdULL; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53ULL; x ^= x >> 33;
     return x;
@@ -1249,8 +1259,7 @@ __global__ void __launch_bounds__(EM_THREADS, 1) em_kernel(const EmArgs *__restr
         }
         // identical columns are merged when there are no allele lengths (lengths differ inside a set) and the sizes fit
         // the merge tables
-        const bool dedup = !a.len && a.rep_ws && a.wp <= DEDUP_COLS * EM_WARPS && a.A_live_max <= DEDUP_MAX_LIVE &&
-                           a.slab_bytes >= (size_t)a.wp * 64 * 12 + DEDUP_CAP * 4 && a.slab_bytes >= (size_t)a.wp * 8 * 32;
+        const bool dedup = !a.len && a.rep_ws && em_merge_fits(a.wp, a.A_live_max, a.slab_bytes);
         const int An = em_compact_build(a, sm, lv, a.C, &s_int, dedup, tr);
         if (An > a.A_live_max) {
             if (tid == 0) {
@@ -1303,8 +1312,7 @@ __global__ void __launch_bounds__(EM_THREADS, 1) em_kernel(const EmArgs *__restr
     bool have_last = false;
     // bytes from sm.p to the end of the slab buffer can be re-used by the compact mode
     // (the allele-compacted layout has dedicated buffers for it instead, so its slab stays intact)
-    const size_t compact_room = p_slots(Apad) * 8 + (size_t)a.slab_rows * 8 + (size_t)a.slab_rows * a.wp * 8;
-    const bool compact_ok = !COOP && (compacted || (size_t)a.C * 24 + 64 * 64 <= compact_room);
+    const bool compact_ok = !COOP && em_collapse_fits(compacted, a.C, a.wp, a.slab_rows);
     while (a.fixed_iters > 0 ? iter < a.fixed_iters : (diff > 0.0001 && iter < 1000)) {
         if (s_status != HGT_OK) break;
         if (compact_ok && (iter == 0 || (iter > 10 && a.remove_low))) {
@@ -1761,6 +1769,34 @@ EmWs em_ws_carve(void *ws, int sm_count, int A) {
     return w;
 }
 
+// Grid and plan of hgt_em_dev (hgt_em_form reports the same decisions).  One CTA takes the batched plan: the
+// allele-compacted layout when it fits, else one streaming CTA; more CTAs run the cooperative streaming plan.
+int em_dev_plan(const hgt_ctx *ctx, int n_classes, int n_alleles, int wp, int n_ctas, int A_live_max, EmArgs *a,
+                EmPlan *plan, int *grid) {
+    int G = n_ctas;
+    if (G <= 0) {
+        // one CTA until the matrix stops fitting comfortably in a single SM's shared memory
+        const size_t bytes = (size_t)n_classes * wp * 8;
+        G = bytes <= 160 * 1024 ? 1 : ctx->sm_count;
+    }
+    if (G > ctx->sm_count) G = ctx->sm_count;
+    if (G > n_classes) G = n_classes;
+    if (G < 1) G = 1;
+    if (G == 1) {
+        const EmShape sh{n_classes, n_alleles, wp, A_live_max};
+        int na = 1;
+        size_t smem = 0;
+        HGT_CHECK(em_plan_batched(ctx, sh, a, &na, &smem));
+        plan->na = na; plan->smem = smem; plan->slab_rows = a->slab_rows;
+    } else {
+        HGT_CHECK(em_plan(ctx, (n_classes + G - 1) / G, n_alleles, wp, plan));
+        a->compact = 0; a->A_live_max = n_alleles; a->slab_bytes = 0;
+        a->slab_rows = plan->slab_rows;
+    }
+    *grid = G;
+    return HGT_OK;
+}
+
 }  // namespace
 
 extern "C" size_t hgt_em_workspace_bytes(const hgt_ctx *ctx, int32_t n_classes, int32_t n_alleles) {
@@ -1781,16 +1817,6 @@ extern "C" int hgt_em_dev(hgt_ctx *ctx, void *stream, const uint64_t *class_bits
         return HGT_ERR_ARG;
     }
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    int G = n_ctas;
-    if (G <= 0) {
-        // one CTA until the matrix stops fitting comfortably in a single SM's shared memory
-        const size_t bytes = (size_t)n_classes * wp * 8;
-        G = bytes <= 160 * 1024 ? 1 : ctx->sm_count;
-    }
-    if (G > ctx->sm_count) G = ctx->sm_count;
-    if (G > n_classes) G = n_classes;
-    if (G < 1) G = 1;
-    const int rows_per_cta = (n_classes + G - 1) / G;
     EmPlan plan;
     EmWs w = em_ws_carve(workspace, ctx->sm_count, n_alleles);
     EmArgs a;
@@ -1801,17 +1827,8 @@ extern "C" int hgt_em_dev(hgt_ctx *ctx, void *stream, const uint64_t *class_bits
     a.vec = w.vec; a.live = w.live; a.part_acc = w.part_acc; a.part_aux = w.part_aux;
     a.red_acc = w.red_acc; a.red_aux = w.red_aux;
     em_set_scratch(&a, w.scratch);
-    if (G == 1) {
-        const EmShape sh{n_classes, n_alleles, wp, n_alleles};
-        int na = 1;
-        size_t smem = 0;
-        HGT_CHECK(em_plan_batched(ctx, sh, &a, &na, &smem));
-        plan.na = na; plan.smem = smem; plan.slab_rows = a.slab_rows;
-    } else {
-        HGT_CHECK(em_plan(ctx, rows_per_cta, n_alleles, wp, &plan));
-        a.compact = 0; a.A_live_max = n_alleles; a.slab_bytes = 0;
-        a.slab_rows = plan.slab_rows;
-    }
+    int G = 1;
+    HGT_CHECK(em_dev_plan(ctx, n_classes, n_alleles, wp, n_ctas, n_alleles, &a, &plan, &G));
     HGT_CUDA(cudaMemcpyAsync(w.d_args, &a, sizeof(a), cudaMemcpyHostToDevice, st));
     if (G == 1) return em_launch<false>(ctx, st, w.d_args, 1, plan.na, plan.smem);
     return em_launch<true>(ctx, st, w.d_args, G, plan.na, plan.smem);
@@ -2359,6 +2376,29 @@ bool hgt_em_wants_coop(const hgt_ctx *ctx, int C, int A, int wp, int A_live_max,
     return bytes > ((size_t)4 << 20) || (n_problems <= 6 && bytes > ((size_t)256 << 10));
 }
 size_t hgt_em_coop_ws_bytes(const hgt_ctx *ctx, int A) { return em_ws_bytes(ctx->sm_count, A); }
+
+extern "C" int hgt_em_form(const hgt_ctx *ctx, int32_t n_classes, int32_t n_alleles, int32_t wp, int32_t has_lengths,
+                           int32_t n_ctas, int32_t a_live_max, int32_t n_problems, hgt_em_form_info *out) {
+    if (!ctx || !out || n_classes < 1 || n_alleles < 1 || wp < hgt_row_pitch(n_alleles) || (wp & 1)) {
+        hgt_set_error("hgt_em_form: need a context, an output, n_classes >= 1, n_alleles >= 1 and an even wp >= "
+                      "hgt_row_pitch(n_alleles)");
+        return HGT_ERR_ARG;
+    }
+    if (a_live_max < 1 || a_live_max > n_alleles) a_live_max = n_alleles;
+    EmArgs a;
+    EmPlan plan;
+    int G = 1;
+    HGT_CHECK(em_dev_plan(ctx, n_classes, n_alleles, wp, n_ctas, a_live_max, &a, &plan, &G));
+    out->form = G > 1 ? HGT_EM_FORM_COOP : (a.compact ? HGT_EM_FORM_COMPACT : HGT_EM_FORM_STREAM);
+    out->grid = G;
+    out->na = plan.na;
+    out->slab_rows = plan.slab_rows;
+    out->slab_bytes = a.slab_bytes;
+    out->merge = a.compact && !has_lengths && em_merge_fits(wp, a.A_live_max, a.slab_bytes);
+    out->collapse = G == 1 && em_collapse_fits(a.compact, n_classes, wp, plan.slab_rows);
+    out->batch_coop = hgt_em_wants_coop(ctx, n_classes, n_alleles, wp, a_live_max, n_problems);
+    return HGT_OK;
+}
 
 int hgt_em_batch_dev(hgt_ctx *ctx, cudaStream_t st, int n_problems, const EmDevProblem *pr, void *h_args, void *d_args) {
     if (n_problems <= 0) return HGT_OK;

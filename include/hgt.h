@@ -113,7 +113,26 @@ size_t hgt_em_workspace_bytes(const hgt_ctx *ctx, int32_t n_classes, int32_t n_a
 int hgt_em_dev(hgt_ctx *ctx, void *stream, const uint64_t *class_bits, const double *class_count,
                int32_t n_classes, int32_t n_alleles, int32_t wp, const double *allele_len, int32_t remove_low,
                int32_t fixed_iters, int32_t n_ctas, double *prob, uint8_t *in_result, int32_t *first_class,
-               int32_t *iters_status /* [2]: iters, status */, void *workspace);
+               int32_t *iters_status /* [3]: iters, status, next_prob sweeps */, void *workspace);
+
+/* The execution form hgt_em_dev chooses for a problem of this size, from the host's planning alone (nothing is launched):
+ * the allele-compacted shared-memory layout (one CTA), one CTA streaming the class rows in slabs of slab_rows rows, or
+ * a cooperative launch over `grid` CTAs (each owns ceil(n_classes / grid) rows, streamed when that exceeds slab_rows).
+ * na = allele slots per thread of the kernel variant.  slab_bytes = shared-memory bytes of the compacted matrix (0 for
+ * the streaming forms); the kernel stores that matrix sparse (16 bytes per non-zero 32-bit word plus an index) when it
+ * fits there, dense otherwise.  merge = a compacted problem merges alleles with identical columns (no lengths,
+ * a_live_max <= 6144, wp <= 128 and room for the tables).  collapse = one CTA can switch to the <= 64-key loop.
+ * batch_coop = typing's batched launch of n_problems problems would run this one cooperatively on all SMs.
+ * wp may be wider than hgt_row_pitch(n_alleles) (batched problems share the widest pitch); a_live_max < 1 means
+ * n_alleles.  Fails like hgt_em_dev on sizes the kernel does not support. */
+enum { HGT_EM_FORM_COMPACT = 0, HGT_EM_FORM_STREAM = 1, HGT_EM_FORM_COOP = 2 };
+typedef struct {
+    int32_t form, grid, na, slab_rows;
+    int64_t slab_bytes;
+    int32_t merge, collapse, batch_coop;
+} hgt_em_form_info;
+int hgt_em_form(const hgt_ctx *ctx, int32_t n_classes, int32_t n_alleles, int32_t wp, int32_t has_lengths, int32_t n_ctas,
+                int32_t a_live_max, int32_t n_problems, hgt_em_form_info *out);
 
 /* Read-sharded locus (SURVEY.md 8e): ONE partial sweep of next_prob() over the class rows that live on this device.
  * mode 0: initial mass (common:1299-1309; p_in unused), 1: next_prob E/M sums (common:1311-1331), 2: smallest class

@@ -45,7 +45,8 @@ static int normalize(pdict *d, const double *len) {
     double total = 0.0;
     if (len) {
         for (int32_t i = 0; i < d->n; i++) total += d->val[d->ord[i]] / len[d->ord[i]];
-        if (total == 0.0) return -3; /* ZeroDivisionError in the reference */
+        /* ZeroDivisionError in the reference; an empty dict divides by nothing (e.g. an empty Gene_cmpt with lengths) */
+        if (total == 0.0 && d->n > 0) return -3;
         for (int32_t i = 0; i < d->n; i++) { int32_t a = d->ord[i]; d->val[a] = d->val[a] / len[a] / total; }
     } else {
         /* `sum(prob.values())`: CPython >= 3.12 sums floats with Neumaier compensation (Python/bltinmodule.c,
