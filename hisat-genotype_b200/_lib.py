@@ -86,6 +86,20 @@ def lib():
         L.hgt_sam_split_write.argtypes = [c_void_p, c_i32, c_void_p]
         L.hgt_sam_split_free.restype = None
         L.hgt_sam_split_free.argtypes = [c_void_p]
+        L.hgt_bam_split_create.restype = c_int
+        L.hgt_bam_split_create.argtypes = [c_void_p, c_size_t, c_i32, c_void_p, c_i32, c_i32, P(c_void_p)]
+        L.hgt_bam_split_sizes.restype = c_int
+        L.hgt_bam_split_sizes.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p]
+        L.hgt_bam_split_write_records.restype = c_int
+        L.hgt_bam_split_write_records.argtypes = [c_void_p, c_i32, c_void_p]
+        L.hgt_bam_split_write_text.restype = c_int
+        L.hgt_bam_split_write_text.argtypes = [c_void_p, c_i32, c_void_p]
+        L.hgt_bam_split_free.restype = None
+        L.hgt_bam_split_free.argtypes = [c_void_p]
+        L.hgt_batch_add_unit_bam.restype = c_i64
+        L.hgt_batch_add_unit_bam.argtypes = [c_void_p, c_i32, c_void_p, c_size_t]
+        L.hgt_batch_unit_text.restype = c_int
+        L.hgt_batch_unit_text.argtypes = [c_void_p, c_i64, c_void_p, P(c_size_t)]
         L.hgt_batch_unit_reads.restype = c_int
         L.hgt_batch_unit_reads.argtypes = [c_void_p, c_i64] + [c_void_p] * 10
         L.hgt_pair_em.restype = c_int

@@ -9,11 +9,13 @@
 #include <algorithm>
 #include <atomic>
 #include <string>
-#include <thread>
 #include <unordered_map>
 #include <vector>
 
 #include "common.cuh"
+#include "split_order.hpp"
+
+using hgt_split::run_threads;
 
 struct hgt_sam_split {
     const char *text = nullptr;
@@ -31,30 +33,6 @@ struct hgt_sam_split {
     bool drop_qual = false;  // write '*' for the QUAL column (the typing path never reads it: 27 % of a 2x100 bp record)
 };
 
-namespace {
-
-template <class F>
-void run_threads(int n_threads, size_t n, F f) {
-    if (n_threads <= 1 || n <= 1) {
-        for (size_t i = 0; i < n; i++) f(i);
-        return;
-    }
-    std::atomic<size_t> next{0};
-    std::vector<std::thread> th;
-    const int nt = (int)std::min<size_t>((size_t)n_threads, n);
-    for (int t = 0; t < nt; t++)
-        th.emplace_back([&]() {
-            while (true) {
-                const size_t i = next.fetch_add(1);
-                if (i >= n) break;
-                f(i);
-            }
-        });
-    for (auto &x : th) x.join();
-}
-
-}  // namespace
-
 extern "C" int hgt_sam_split_create(const char *sam_text, size_t n_bytes, int32_t n_refs, const char *const *ref_names,
                                     int32_t n_threads, hgt_sam_split **out) {
     return hgt_sam_split_create_opts(sam_text, n_bytes, n_refs, ref_names, n_threads, 0, out);
@@ -67,10 +45,7 @@ extern "C" int hgt_sam_split_create_opts(const char *sam_text, size_t n_bytes, i
         return HGT_ERR_ARG;
     }
     *out = nullptr;
-    if (n_threads <= 0) {
-        const unsigned hc = std::thread::hardware_concurrency();
-        n_threads = hc ? (int)hc : 1;
-    }
+    n_threads = hgt_split::default_threads(n_threads);
     std::unordered_map<std::string, int> ref_index;
     for (int r = 0; r < n_refs; r++) ref_index[ref_names[r]] = r;
     hgt_sam_split *s = new hgt_sam_split();
@@ -145,24 +120,12 @@ extern "C" int hgt_sam_split_create_opts(const char *sam_text, size_t n_bytes, i
     }
     s->last_needs_newline = n_bytes > 0 && sam_text[n_bytes - 1] != '\n';
     // pass 2: per reference - concatenate the slices (input order), stable sort by (name, pos)
-    run_threads(n_threads, (size_t)n_refs, [&](size_t r) {
-        std::vector<hgt_sam_split::Rec> &b = s->bucket[r];
-        size_t total = 0;
-        for (size_t k = 0; k < n_slices; k++) total += part[k][r].size();
-        b.reserve(total);
-        for (size_t k = 0; k < n_slices; k++) b.insert(b.end(), part[k][r].begin(), part[k][r].end());
-        const char *text = sam_text;
-        std::stable_sort(b.begin(), b.end(), [text](const hgt_sam_split::Rec &x, const hgt_sam_split::Rec &y) {
-            const uint32_t m = std::min(x.name_len, y.name_len);
-            const int c = memcmp(text + x.off, text + y.off, m);
-            if (c != 0) return c < 0;
-            if (x.name_len != y.name_len) return x.name_len < y.name_len;
-            return x.pos < y.pos;
-        });
-        size_t bytes = 0;
-        for (const auto &rec : b) bytes += rec.len - (rec.q_len ? rec.q_len - 1 : 0);
-        s->bytes[r] = bytes;
-    });
+    hgt_split::bucket_and_order(n_threads, part, s->bucket, [sam_text](const hgt_sam_split::Rec &x) { return sam_text + x.off; },
+                                [s](size_t r) {
+                                    size_t bytes = 0;
+                                    for (const auto &rec : s->bucket[r]) bytes += rec.len - (rec.q_len ? rec.q_len - 1 : 0);
+                                    s->bytes[r] = bytes;
+                                });
     *out = s;
     return HGT_OK;
 }

@@ -35,6 +35,7 @@
 #include "walk.hpp"
 #include "walk_dev.cuh"
 #include "reads.cuh"
+#include "bam_dev.cuh"
 
 using namespace hgt;
 
@@ -1481,7 +1482,10 @@ static int wpl_of(int wp) {
 struct UnitHost {
     int locus = 0;
     const char *sam = nullptr;
-    size_t n_bytes = 0;
+    size_t n_bytes = 0;             // text bytes (a BAM unit: its rendered text, known after the length pass of prepare)
+    const void *blob = nullptr;     // BAM unit: packed records (bam_dev.cuh), rendered into the arena by prepare
+    size_t blob_bytes = 0;
+    int64_t n_records = 0;
     int local = 0;  // index inside its locus batch
     int arena = 0;  // index in arena order (loci-major, add order inside a locus)
     int64_t num_reads = 0, num_pairs = 0;
@@ -1500,6 +1504,8 @@ struct ReadsDev {
     DevBuf d_text, d_chunk, d_line_off, d_unit, d_rec, d_st, d_hdr, d_hids, d_slow, d_slow_list, d_units, d_loci, d_small,
         d_scan, d_partial, d_jobs_desc, d_cnt, d_mf;
     PinBuf h_units, h_small, h_stage, h_loci, h_jobs_desc;
+    DevBuf d_blob, d_blen, d_bunits;  // BAM units: blob arena, per-record text offsets, unit descriptors (prepare only)
+    PinBuf h_bstage, h_bunits;
     size_t o_uoff = 0, o_uline0 = 0, o_upos0 = 0, o_ulocus = 0, o_ulocal = 0, o_lu0 = 0, units_bytes = 0;
     size_t s_reads = 0, s_pairs = 0, s_totals = 0, small_bytes = 0;  // offsets inside the small result block
     void release() {
@@ -1508,6 +1514,11 @@ struct ReadsDev {
         for (DevBuf *x : all) x->release();
         PinBuf *pins[] = {&h_units, &h_small, &h_stage, &h_loci, &h_jobs_desc};
         for (PinBuf *x : pins) x->release();
+        release_bam();
+    }
+    void release_bam() {
+        d_blob.release(); d_blen.release(); d_bunits.release();
+        h_bstage.release(); h_bunits.release();
     }
 };
 
@@ -1676,6 +1687,218 @@ static bool is_pinned_host(const void *p) {
     return at.type == cudaMemoryTypeHost;
 }
 
+// ---- BAM units: packed records (bam_dev.cuh) -> text in the arena ---------------------------------------------------------
+namespace hgtk {
+
+constexpr int BAM_THREADS = 256;
+
+struct BamUnitDev {  // one BAM unit of a batch: blob in the blob arena, first record (batch-wide), slice of the text arena
+    int64_t blob_off, rec0, text_off, pad;
+};
+
+// unit of batch-wide record g: the last unit whose first record is <= g (units without records are skipped that way)
+__device__ __forceinline__ int bam_unit_of(const BamUnitDev *__restrict__ u, int nb, int64_t g) {
+    int lo = 0, hi = nb - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (u[mid].rec0 <= g) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
+__device__ __forceinline__ void bam_view(const unsigned char *__restrict__ blobs, const BamUnitDev &U, int64_t i, hgtb::BamRec *r,
+                                         hgtb::BamNames *nm) {
+    using namespace hgtb;
+    const unsigned char *blob = blobs + U.blob_off;
+    const BamUnitHeader h = *reinterpret_cast<const BamUnitHeader *>(blob);
+    nm->off = reinterpret_cast<const uint32_t *>(blob + unit_name_off_at());
+    nm->bytes = blob + unit_names_at(h.n_names);
+    nm->n = h.n_names;
+    const uint64_t *ro = reinterpret_cast<const uint64_t *>(blob + unit_rec_off_at(h.n_names, h.names_bytes));
+    const uint64_t a = ro[i], e = ro[i + 1];
+    bam_decode(blob + a, e - a, (h.flags & UNIT_DROP_QUAL) != 0, r);
+}
+
+// text length of every record (one thread per record)
+__global__ void __launch_bounds__(BAM_THREADS) bam_text_len_kernel(const unsigned char *__restrict__ blobs,
+                                                                   const BamUnitDev *__restrict__ u, int nb, int64_t n_rec,
+                                                                   int64_t *__restrict__ len) {
+    const int64_t g = (int64_t)blockIdx.x * BAM_THREADS + threadIdx.x;
+    if (g >= n_rec) return;
+    const int k = bam_unit_of(u, nb, g);
+    hgtb::BamRec r;
+    hgtb::BamNames nm;
+    bam_view(blobs, u[k], g - u[k].rec0, &r, &nm);
+    len[g] = hgtb::bam_line_len(r, nm);
+}
+
+// text offset of every unit's first record (k = 0 .. nb; u[nb].rec0 = n_rec): the per-unit sizes the host lays out with
+__global__ void bam_unit_text_kernel(const int64_t *__restrict__ off, const BamUnitDev *__restrict__ u, int nb,
+                                     int64_t *__restrict__ out) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k <= nb) out[k] = off[u[k].rec0];
+}
+
+// one warp per record: QNAME, SEQ and QUAL lane-parallel, the other columns and the tags by lane 0 (bam_dev.cuh)
+__global__ void __launch_bounds__(BAM_THREADS) bam_render_kernel(const unsigned char *__restrict__ blobs,
+                                                                 const BamUnitDev *__restrict__ u, int nb, int64_t n_rec,
+                                                                 const int64_t *__restrict__ off, char *__restrict__ text) {
+    const int64_t g = ((int64_t)blockIdx.x * BAM_THREADS + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (g >= n_rec) return;
+    const int k = bam_unit_of(u, nb, g);
+    hgtb::BamRec r;
+    hgtb::BamNames nm;
+    bam_view(blobs, u[k], g - u[k].rec0, &r, &nm);
+    char *dst = text + u[k].text_off + (off[g] - off[u[k].rec0]);
+    const uint32_t qn = hgtb::qname_len(r);
+    for (uint32_t i = lane; i < qn; i += 32) dst[i] = (char)r.p[hgtb::REC_FIXED + i];
+    dst += qn;
+    int64_t hl = 0;
+    if (lane == 0) {
+        hgtb::WriteSink w{dst};
+        hgtb::bam_head(r, nm, w);
+        hl = w.o - dst;
+    }
+    dst += __shfl_sync(0xffffffffu, hl, 0);
+    if (r.l_seq == 0) {
+        if (lane == 0) dst[0] = '*';
+        dst += 1;
+    } else {
+        for (uint32_t i = lane; i < r.l_seq; i += 32) dst[i] = hgtb::seq_base(r, i);
+        dst += r.l_seq;
+    }
+    if (lane == 0) dst[0] = '\t';
+    dst += 1;
+    if (!r.has_qual) {
+        if (lane == 0) dst[0] = '*';
+        dst += 1;
+    } else {
+        for (uint32_t i = lane; i < r.l_seq; i += 32) dst[i] = (char)(r.p[r.o_qual + i] + 33);
+        dst += r.l_seq;
+    }
+    if (lane == 0) {
+        hgtb::WriteSink w{dst};
+        hgtb::bam_tags(r, w);
+        *w.o = '\n';
+    }
+}
+
+}  // namespace hgtk
+
+// Length pass of the BAM units (prepare, only when the batch holds one): blobs to the device, text length per record,
+// scan, per-unit sizes back to the host (one synchronisation).  Sets n_bytes of every BAM unit.
+static int bam_units_measure(hgt_batch *b, std::vector<int> &bam_arena, int64_t *n_rec) {
+    hgt_ctx *ctx = b->ctx;
+    cudaStream_t st = ctx->stream;
+    ReadsDev &rd = b->rd;
+    const int nb = (int)bam_arena.size();
+    std::vector<int64_t> blob_off((size_t)nb + 1, 0);
+    HGT_CHECK(rd.h_bunits.alloc((size_t)(nb + 1) * sizeof(hgtk::BamUnitDev) + (size_t)(nb + 1) * 8));
+    hgtk::BamUnitDev *hu = rd.h_bunits.as<hgtk::BamUnitDev>();
+    int64_t R = 0;
+    bool all_pinned = true;
+    for (int k = 0; k < nb; k++) {
+        const UnitHost &U = b->units[rd.unit_of_arena[bam_arena[k]]];
+        hu[k] = {blob_off[k], R, 0, 0};
+        blob_off[k + 1] = blob_off[k] + (int64_t)a16(U.blob_bytes);
+        R += U.n_records;
+        all_pinned &= is_pinned_host(U.blob);
+    }
+    hu[nb] = {blob_off[nb], R, 0, 0};
+    *n_rec = R;
+    HGT_CHECK(rd.d_blob.alloc((size_t)std::max<int64_t>(blob_off[nb], 16)));
+    unsigned char *db = rd.d_blob.as<unsigned char>();
+    if (all_pinned) {
+        for (int k = 0; k < nb; k++) {
+            const UnitHost &U = b->units[rd.unit_of_arena[bam_arena[k]]];
+            HGT_CUDA(cudaMemcpyAsync(db + blob_off[k], U.blob, U.blob_bytes, cudaMemcpyHostToDevice, st));
+            ctx->h2d_bytes += (int64_t)U.blob_bytes;
+        }
+    } else {  // pageable blobs: host threads assemble the blob arena in page-locked memory, one copy
+        HGT_CHECK(rd.h_bstage.alloc((size_t)std::max<int64_t>(blob_off[nb], 16)));
+        unsigned char *hs = rd.h_bstage.as<unsigned char>();
+        parallel_units(batch_threads(b->params), (size_t)nb, [&](size_t k) {
+            const UnitHost &U = b->units[rd.unit_of_arena[bam_arena[k]]];
+            memcpy(hs + blob_off[k], U.blob, U.blob_bytes);
+        });
+        HGT_CUDA(cudaMemcpyAsync(db, hs, (size_t)blob_off[nb], cudaMemcpyHostToDevice, st));
+        ctx->h2d_bytes += blob_off[nb];
+    }
+    const size_t desc = (size_t)(nb + 1) * sizeof(hgtk::BamUnitDev);
+    HGT_CHECK(rd.d_bunits.alloc(desc + (size_t)(nb + 1) * 8));
+    HGT_CUDA(cudaMemcpyAsync(rd.d_bunits.p, hu, desc, cudaMemcpyHostToDevice, st));
+    ctx->h2d_bytes += (int64_t)desc;
+    HGT_CHECK(rd.d_blen.alloc((size_t)(R + 1) * 8));
+    if (R > 0) {
+        hgtk::bam_text_len_kernel<<<(unsigned)((R + hgtk::BAM_THREADS - 1) / hgtk::BAM_THREADS), hgtk::BAM_THREADS, 0, st>>>(
+            db, rd.d_bunits.as<hgtk::BamUnitDev>(), nb, R, rd.d_blen.as<int64_t>());
+        ctx->launches++;
+        HGT_CUDA(cudaGetLastError());
+    }
+    HGT_CHECK(dev_scan(ctx, st, rd.d_blen.as<int64_t>(), R, rd.d_blen.as<int64_t>(), &rd.d_partial));
+    int64_t *d_sz = reinterpret_cast<int64_t *>(static_cast<unsigned char *>(rd.d_bunits.p) + desc);
+    hgtk::bam_unit_text_kernel<<<(unsigned)((nb + 1 + 255) / 256), 256, 0, st>>>(rd.d_blen.as<int64_t>(),
+                                                                                rd.d_bunits.as<hgtk::BamUnitDev>(), nb, d_sz);
+    ctx->launches++;
+    HGT_CUDA(cudaGetLastError());
+    int64_t *h_sz = reinterpret_cast<int64_t *>(reinterpret_cast<unsigned char *>(hu) + desc);
+    HGT_CUDA(d2h(h_sz, d_sz, (size_t)(nb + 1) * 8, st));
+    HGT_CUDA(cudaStreamSynchronize(st));
+    for (int k = 0; k < nb; k++) b->units[rd.unit_of_arena[bam_arena[k]]].n_bytes = (size_t)(h_sz[k + 1] - h_sz[k]);
+    return HGT_OK;
+}
+
+// Text arena of a batch with BAM units: '\n' everywhere, text units copied (page-locked directly, pageable staged), BAM
+// units rendered into their slices.
+static int bam_units_fill(hgt_batch *b, const std::vector<int> &bam_arena, int64_t R) {
+    hgt_ctx *ctx = b->ctx;
+    cudaStream_t st = ctx->stream;
+    ReadsDev &rd = b->rd;
+    const size_t nu = b->units.size();
+    char *dt = rd.d_text.as<char>();
+    HGT_CUDA(cudaMemsetAsync(dt, '\n', (size_t)rd.text_bytes, st));
+    std::vector<size_t> stage_off(nu + 1, 0);
+    for (size_t a = 0; a < nu; a++) {
+        const UnitHost &U = b->units[rd.unit_of_arena[a]];
+        const bool staged = !U.blob && U.n_bytes && !is_pinned_host(U.sam);
+        stage_off[a + 1] = stage_off[a] + (staged ? a16(U.n_bytes) : 0);
+        if (!U.blob && U.n_bytes && !staged) {
+            HGT_CUDA(cudaMemcpyAsync(dt + rd.unit_off[a], U.sam, U.n_bytes, cudaMemcpyHostToDevice, st));
+            ctx->h2d_bytes += (int64_t)U.n_bytes;
+        }
+    }
+    if (stage_off[nu]) {
+        HGT_CHECK(rd.h_stage.alloc(stage_off[nu]));
+        char *hs = rd.h_stage.as<char>();
+        parallel_units(batch_threads(b->params), nu, [&](size_t a) {
+            const UnitHost &U = b->units[rd.unit_of_arena[a]];
+            if (stage_off[a + 1] > stage_off[a]) memcpy(hs + stage_off[a], U.sam, U.n_bytes);
+        });
+        for (size_t a = 0; a < nu; a++) {
+            const UnitHost &U = b->units[rd.unit_of_arena[a]];
+            if (stage_off[a + 1] == stage_off[a]) continue;
+            HGT_CUDA(cudaMemcpyAsync(dt + rd.unit_off[a], hs + stage_off[a], U.n_bytes, cudaMemcpyHostToDevice, st));
+            ctx->h2d_bytes += (int64_t)U.n_bytes;
+        }
+    }
+    if (R == 0) return HGT_OK;
+    // the descriptors again, now with the arena slices (the length pass synchronised: the staging copy is idle)
+    const int nb = (int)bam_arena.size();
+    hgtk::BamUnitDev *hu = rd.h_bunits.as<hgtk::BamUnitDev>();
+    for (int k = 0; k < nb; k++) hu[k].text_off = rd.unit_off[bam_arena[k]];
+    const size_t desc = (size_t)(nb + 1) * sizeof(hgtk::BamUnitDev);
+    HGT_CUDA(cudaMemcpyAsync(rd.d_bunits.p, hu, desc, cudaMemcpyHostToDevice, st));
+    ctx->h2d_bytes += (int64_t)desc;
+    const int64_t warps_per_cta = hgtk::BAM_THREADS / 32;
+    hgtk::bam_render_kernel<<<(unsigned)((R + warps_per_cta - 1) / warps_per_cta), hgtk::BAM_THREADS, 0, st>>>(
+        rd.d_blob.as<unsigned char>(), rd.d_bunits.as<hgtk::BamUnitDev>(), nb, R, rd.d_blen.as<int64_t>(), dt);
+    ctx->launches++;
+    HGT_CUDA(cudaGetLastError());
+    return HGT_OK;
+}
+
 static int batch_prepare(hgt_batch *b) {
     hgt_ctx *ctx = b->ctx;
     cudaStream_t st = ctx->stream;
@@ -1700,6 +1923,14 @@ static int batch_prepare(hgt_batch *b) {
         }
     }
     rd.locus_unit0[b->loci.size()] = (int32_t)nu;
+    std::vector<int> bam_arena;  // arena indices of the BAM units
+    for (size_t a = 0; a < nu; a++)
+        if (b->units[rd.unit_of_arena[a]].blob) bam_arena.push_back((int)a);
+    int64_t n_bam_rec = 0;
+    if (!bam_arena.empty()) {
+        HostTimer ht(ctx, 0);
+        HGT_CHECK(bam_units_measure(b, bam_arena, &n_bam_rec));
+    }
     rd.unit_off.assign(nu + 1, 0);
     rd.POS = 0;
     for (size_t a = 0; a < nu; a++) {
@@ -1719,15 +1950,18 @@ static int batch_prepare(hgt_batch *b) {
         HGT_CHECK(rd.d_text.alloc((size_t)rd.text_bytes));
         char *dt = rd.d_text.as<char>();
         bool all_pinned = true;
-        for (const UnitHost &U : b->units) all_pinned &= U.n_bytes == 0 || is_pinned_host(U.sam);
-        ctx->h2d_bytes += rd.text_bytes;
-        if (all_pinned) {  // page-locked input: the DMA engine reads the caller's buffers directly
+        for (const UnitHost &U : b->units) all_pinned &= U.blob || U.n_bytes == 0 || is_pinned_host(U.sam);
+        if (!bam_arena.empty()) {  // text units copied, BAM units rendered (h2d_bytes: the bytes actually copied)
+            HGT_CHECK(bam_units_fill(b, bam_arena, n_bam_rec));
+        } else if (all_pinned) {  // page-locked input: the DMA engine reads the caller's buffers directly
+            ctx->h2d_bytes += rd.text_bytes;
             HGT_CUDA(cudaMemsetAsync(dt, '\n', (size_t)rd.text_bytes, st));
             for (size_t a = 0; a < nu; a++) {
                 const UnitHost &U = b->units[rd.unit_of_arena[a]];
                 if (U.n_bytes) HGT_CUDA(cudaMemcpyAsync(dt + rd.unit_off[a], U.sam, U.n_bytes, cudaMemcpyHostToDevice, st));
             }
         } else {  // pageable input: host threads assemble the arena image in page-locked memory, one copy
+            ctx->h2d_bytes += rd.text_bytes;
             HGT_CHECK(rd.h_stage.alloc((size_t)rd.text_bytes));
             char *hs = rd.h_stage.as<char>();
             parallel_units(batch_threads(b->params), nu, [&](size_t a) {
@@ -1779,6 +2013,7 @@ static int batch_prepare(hgt_batch *b) {
         HGT_CUDA(d2h(rd.h_small.p, rd.d_chunk.as<int64_t>() + rd.n_chunks, 8, st));
         HGT_CUDA(cudaStreamSynchronize(st));
         rd.n_lines = *rd.h_small.as<int64_t>();
+        rd.release_bam();  // the blob arena goes back to the pool: the render has run
     }
     if (rd.n_lines > 0x7fffffff) {
         hgt_set_error("more than 2^31 alignment lines in one batch: split the batch");
@@ -2667,6 +2902,48 @@ extern "C" int64_t hgt_batch_add_unit(hgt_batch *b, int32_t locus_index, const c
     u.n_bytes = n_bytes;
     b->units.push_back(std::move(u));
     return (int64_t)b->units.size() - 1;
+}
+
+extern "C" int64_t hgt_batch_add_unit_bam(hgt_batch *b, int32_t locus_index, const void *blob, size_t n_bytes) {
+    if (!b || locus_index < 0 || locus_index >= (int)b->loci.size() || b->prepared) {
+        hgt_set_error("hgt_batch_add_unit_bam: bad argument");
+        return HGT_ERR_ARG;
+    }
+    hgtb::BamUnitHeader h;
+    if (const char *why = hgtb::bam_unit_check(blob, n_bytes, &h)) {
+        hgt_set_error("hgt_batch_add_unit_bam: not a packed BAM unit: %s", why);
+        return HGT_ERR_ARG;
+    }
+    UnitHost u;
+    u.locus = locus_index;
+    u.blob = blob;
+    u.blob_bytes = n_bytes;
+    u.n_records = h.n_records;
+    b->units.push_back(std::move(u));
+    return (int64_t)b->units.size() - 1;
+}
+
+extern "C" int hgt_batch_unit_text(const hgt_batch *b, int64_t unit, char *dst, size_t *n_bytes) {
+    if (!b || !b->prepared || unit < 0 || unit >= (int64_t)b->units.size() || !n_bytes) {
+        hgt_set_error("hgt_batch_unit_text: bad argument or batch not prepared");
+        return HGT_ERR_ARG;
+    }
+    const UnitHost &U = b->units[(size_t)unit];
+    if (!dst) {
+        *n_bytes = U.n_bytes;
+        return HGT_OK;
+    }
+    if (*n_bytes < U.n_bytes) {
+        hgt_set_error("hgt_batch_unit_text: buffer of %zu bytes for %zu bytes of text", *n_bytes, U.n_bytes);
+        return HGT_ERR_ARG;
+    }
+    *n_bytes = U.n_bytes;
+    if (!U.n_bytes) return HGT_OK;
+    HGT_CUDA(cudaSetDevice(b->ctx->device));
+    g_acct = b->ctx;
+    HGT_CUDA(d2h(dst, b->rd.d_text.as<char>() + b->rd.unit_off[(size_t)U.arena], U.n_bytes, b->ctx->stream));
+    HGT_CUDA(cudaStreamSynchronize(b->ctx->stream));
+    return HGT_OK;
 }
 
 extern "C" int64_t hgt_batch_add_units(hgt_batch *b, int64_t n, const int32_t *locus_index, const char *const *sam_text,

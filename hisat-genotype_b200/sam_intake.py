@@ -1,11 +1,15 @@
-"""Native SAM intake: the aligner's SAM text -> per-locus, name-grouped alignment text, without samtools.
+"""Native SAM / BAM intake: the aligner's SAM text or a BAM file -> per-locus, name-grouped alignment units, without
+samtools.
 
 Replaces `samtools view <bam> <backbone> | sort -k1,1 -s` (reference hisatgenotype_typing_core.py:436-468) and the BAM
 round trip in front of it (hisatgenotype_typing_common.py:1038-1054) for every locus of a sample in one pass (libhgt
-hgt_sam_split_*, host threads)."""
+hgt_sam_split_* / hgt_bam_split_*, host threads).  A BAM unit travels to the GPU as packed records and is rendered into
+alignment text there (hgt_batch_add_unit_bam)."""
 from __future__ import annotations
 
 import ctypes
+import struct
+import zlib
 
 import numpy as np
 
@@ -49,6 +53,118 @@ def split_sam(sam_text, ref_names, n_threads=0, pinned=None, drop_qual=False):
         L.hgt_sam_split_free(h)
 
 
+class BamUnit(bytes):
+    """A packed BAM unit (hgt_bam_split_write_records; layout in csrc/bam_dev.cuh): what split_bam returns per reference, and
+    what Batch.add_unit_bam / typing_from_alignments take in place of alignment text."""
+
+
+_BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
+
+
+def _bgzf_blocks(data):
+    """(start, end) of every BGZF block: gzip members whose extra field carries BC with BSIZE = block size - 1."""
+    blocks = []
+    o, n = 0, len(data)
+    while o < n:
+        assert n - o >= 18, "truncated BGZF block header at byte %d" % o
+        assert data[o] == 31 and data[o + 1] == 139 and data[o + 2] == 8 and data[o + 3] & 4, \
+            "not a BGZF block at byte %d" % o
+        xlen = struct.unpack_from("<H", data, o + 10)[0]
+        assert o + 12 + xlen <= n, "truncated BGZF block header at byte %d" % o
+        x, bsize = o + 12, None
+        while x + 4 <= o + 12 + xlen:
+            si1, si2, slen = data[x], data[x + 1], struct.unpack_from("<H", data, x + 2)[0]
+            if si1 == 66 and si2 == 67 and slen == 2:
+                bsize = struct.unpack_from("<H", data, x + 4)[0]
+            x += 4 + slen
+        assert bsize is not None, "gzip member without the BGZF BC field at byte %d" % o
+        end = o + bsize + 1
+        assert 12 + xlen + 8 <= bsize + 1 and end <= n, "truncated BGZF block at byte %d" % o
+        blocks.append((o, end, 12 + xlen))
+        o = end
+    return blocks
+
+
+def _inflate_blocks(data, blocks):
+    out = []
+    for o, end, head in blocks:
+        crc, isize = struct.unpack_from("<II", data, end - 8)
+        d = zlib.decompressobj(-15)
+        try:
+            raw = d.decompress(bytes(data[o + head:end - 8]))
+        except zlib.error as e:
+            raise AssertionError("corrupt BGZF block at byte %d: %s" % (o, e))
+        assert d.eof and not d.unused_data, "corrupt BGZF block at byte %d (deflate stream does not end with the block)" % o
+        assert len(raw) == isize, "BGZF block at byte %d: ISIZE %d, inflated %d bytes" % (o, isize, len(raw))
+        assert zlib.crc32(raw) == crc, "BGZF block at byte %d: CRC32 mismatch" % o
+        out.append(raw)
+    return b"".join(out)
+
+
+def read_bgzf(data, n_threads=0):
+    """Inflate a BGZF file (BAM's compression) to its uncompressed bytes: blocks inflate in parallel on a thread pool
+    (zlib releases the GIL), every block's CRC32 and ISIZE are checked.  A missing EOF marker block is accepted, as
+    samtools accepts it (with a warning); a truncated or corrupt block raises AssertionError."""
+    import os
+    from concurrent.futures import ThreadPoolExecutor
+    data = memoryview(data)
+    blocks = _bgzf_blocks(data)
+    if not bytes(data[-len(_BGZF_EOF):]) == _BGZF_EOF:
+        import warnings
+        warnings.warn("BGZF input has no EOF marker block; it may be truncated")
+    n_threads = int(n_threads) or os.cpu_count() or 1
+    if n_threads <= 1 or len(blocks) < 64:
+        return _inflate_blocks(data, blocks)
+    per = max(16, (len(blocks) + 4 * n_threads - 1) // (4 * n_threads))
+    chunks = [blocks[i:i + per] for i in range(0, len(blocks), per)]
+    with ThreadPoolExecutor(n_threads) as pool:
+        return b"".join(pool.map(lambda c: _inflate_blocks(data, c), chunks))
+
+
+def split_bam(bam_bytes, ref_names, n_threads=0, pinned=None, drop_qual=False, text=False):
+    """bam_bytes: a BAM file (BGZF, inflated first by read_bgzf) or its decompressed stream.  ref_names: backbone names.
+    Returns {ref_name: BamUnit} (packed records for Batch.add_unit_bam), with text=True {ref_name: bytes} (the SAM text
+    `samtools view` prints for the same records, in the same order as split_sam), or with pinned=_lib.PinnedText
+    {ref_name: (address, n_bytes)} of either written into it.  Records are bucketed and ordered as split_sam does.
+    drop_qual: the QUAL bytes are left out ('*' in the text).  Malformed input raises AssertionError; float tags and the
+    CG long-CIGAR tag raise HgtError (HGT_ERR_UNSUPPORTED)."""
+    if bytes(bam_bytes[:2]) == b"\x1f\x8b":
+        bam_bytes = read_bgzf(bam_bytes, n_threads)
+    bam_bytes = bytes(bam_bytes)
+    L = _lib.lib()
+    n = len(ref_names)
+    enc = [r.encode() for r in ref_names]
+    arr = (ctypes.c_char_p * n)(*enc)
+    h = ctypes.c_void_p()
+    rc = L.hgt_bam_split_create(bam_bytes, len(bam_bytes), n, arr, int(n_threads), 1 if drop_qual else 0,
+                                ctypes.byref(h))
+    if rc == _lib.HGT_ERR_PARSE:
+        raise AssertionError(_lib.last_error())
+    _lib.check(rc)
+    try:
+        sizes = (ctypes.c_size_t * n)()
+        if text:
+            _lib.check(L.hgt_bam_split_sizes(h, None, sizes, None))
+            write = L.hgt_bam_split_write_text
+        else:
+            _lib.check(L.hgt_bam_split_sizes(h, sizes, None, None))
+            write = L.hgt_bam_split_write_records
+        out = {}
+        for r, name in enumerate(ref_names):
+            if pinned is not None:  # PinnedText hands out 16-byte aligned slices
+                addr, nb = pinned.reserve(sizes[r])
+                _lib.check(write(h, r, ctypes.c_void_p(addr)))
+                out[name] = (addr, nb)
+            else:
+                buf = np.empty(max(int(sizes[r]), 8) // 8 + 1, np.uint64)  # 8-byte aligned
+                _lib.check(write(h, r, buf.ctypes.data_as(ctypes.c_void_p)))
+                data = buf.view(np.uint8)[:sizes[r]].tobytes()
+                out[name] = data if text else BamUnit(data)
+        return out
+    finally:
+        L.hgt_bam_split_free(h)
+
+
 def hisat2_command(simulation, index_name, base_fname, read_fname, fastq, threads):
     """The command line of the reference's align_reads() for aligner == "hisat2" on a graph index
     (hisatgenotype_typing_common.py:995-1024), without the samtools stages behind it."""
@@ -81,10 +197,16 @@ def align_to_sam(simulation, index_name, base_fname, read_fname, fastq, threads,
     return proc.stdout
 
 
-def read_alignment_text(path):
-    """SAM text of an alignment file; None when the file is BGZF / BAM (it then goes through samtools, like the reference)."""
+def read_alignment(path, n_threads=0):
+    """The alignment file as the native intake takes it: ("sam", text), ("bam", decompressed BAM stream), or (None, None)
+    for what stays with samtools, like the reference: CRAM, and BGZF that is not BAM."""
     with open(path, "rb") as f:
-        head = f.read(2)
-        if head == b"\x1f\x8b":
-            return None
-        return head + f.read()
+        data = f.read()
+    if data[:4] == b"CRAM":
+        return None, None
+    if data[:2] == b"\x1f\x8b":
+        raw = read_bgzf(data, n_threads) if data[3:4] and data[3] & 4 else b""
+        if raw[:4] != b"BAM\1":
+            return None, None
+        return "bam", raw
+    return "sam", data

@@ -198,6 +198,31 @@ class Batch:
         self.unit_locus.append(locus_index)
         return int(u)
 
+    def add_unit_bam(self, locus_index, blob):
+        """A packed BAM unit (sam_intake.split_bam): prepare() renders its records into alignment text on the GPU."""
+        buf = np.frombuffer(blob, np.uint8)
+        if buf.ctypes.data % 8:
+            buf = np.frombuffer(np.frombuffer(blob + b"\0" * (-len(blob) % 8), np.uint64).copy(), np.uint8)[:len(blob)]
+        self._texts.append(buf)  # must outlive prepare()
+        return self.add_unit_bam_ptr(locus_index, buf.ctypes.data, len(blob))
+
+    def add_unit_bam_ptr(self, locus_index, address, n_bytes):
+        """A packed BAM unit already in (ideally page-locked, _lib.PinnedText) host memory, 8-byte aligned; the caller keeps
+        it valid until prepare() returns."""
+        u = lib().hgt_batch_add_unit_bam(self.handle, locus_index, ctypes.c_void_p(address), n_bytes)
+        if u < 0:
+            _lib.check(int(u))
+        self.unit_locus.append(locus_index)
+        return int(u)
+
+    def unit_text(self, u):
+        """After prepare(): the unit's alignment text as it sits in the device arena (rendered on the GPU for a BAM unit)."""
+        n = ctypes.c_size_t(0)
+        _lib.check(lib().hgt_batch_unit_text(self.handle, u, None, ctypes.byref(n)))
+        buf = np.empty(max(n.value, 1), np.uint8)
+        _lib.check(lib().hgt_batch_unit_text(self.handle, u, buf.ctypes.data_as(ctypes.c_void_p), ctypes.byref(n)))
+        return buf[:n.value].tobytes()
+
     def _call(self, rc):
         if rc == _lib.HGT_ERR_AMBIGUITY:
             raise SystemExit("Error: %s" % _lib.last_error())
@@ -578,9 +603,11 @@ def typing_from_alignments(base_fname, locus_tables, locus_list, alignments, sim
     locus_tables  {gene: LocusTables}
     locus_list    as typing() receives it: gene names, or in simulation mode the lists of truth alleles
                   (gene = names[0].split('*')[0], core:380-383)
-    alignments    {gene: alignment lines in `samtools view <bam> <backbone> | sort -k1,1 -s` order (core:458-468)}
+    alignments    {gene: alignment lines in `samtools view <bam> <backbone> | sort -k1,1 -s` order (core:458-468), or a
+                  sam_intake.BamUnit of split_bam, rendered into those lines on the GPU}
     Returns (report body text starting at the aligner line, test_passed dict of the simulation mode)."""
     from . import report
+    from .sam_intake import BamUnit
     assert index_type == "graph", "the linear-index branch (core:1597-1648) stays on the reference path"
     genes, truths = [], []
     for entry in locus_list:
@@ -599,7 +626,10 @@ def typing_from_alignments(base_fname, locus_tables, locus_list, alignments, sim
                   remove_low_abundance_alleles, device=device)
     try:
         for g in genes:
-            batch.add_unit(uniq.index(g), alignments[g])
+            if isinstance(alignments[g], BamUnit):
+                batch.add_unit_bam(uniq.index(g), alignments[g])
+            else:
+                batch.add_unit(uniq.index(g), alignments[g])
         batch.run()
         text = [report.aligner_line(aligner, index_type)]
         test_passed = {}
@@ -696,7 +726,8 @@ def typing(simulation, full_path_base_fname, locus_list, genotype_genome, partia
         return _reference.typing(*[a[k] for k in _TYPING_PARAMS])
     ref_common = _reference.typing_common  # the module the reference's typing() calls align_reads through (core:358)
     from . import sam_intake
-    # HGT_NATIVE_INTAKE=1: SAM text is read and split natively (SURVEY.md 8f-3) instead of through samtools pipes
+    # HGT_NATIVE_INTAKE=1: a SAM or BAM alignment file is read and split natively (SURVEY.md 8f-3) instead of through
+    # samtools pipes (CRAM and BGZF that is not BAM stay with samtools)
     native = os.environ.get("HGT_NATIVE_INTAKE", "") not in ("", "0")
     base_fname = full_path_base_fname.split("/")[-1]
     report_base = "%s/%s-%s." % (out_dir, output_base, base_fname)
@@ -716,7 +747,7 @@ def typing(simulation, full_path_base_fname, locus_list, genotype_genome, partia
         for aligner, index_type in aligners:
             remove_alignment_file = False
             aln = alignment_fname
-            native_text = None
+            native_text = native_bam = None
             if aln == "":
                 if native:  # HISAT2's SAM stream straight into the native intake: no samtools view -bS / sort / index
                     native_text = sam_intake.align_to_sam(simulation, full_path_base_fname + "." + index_type, base_fname,
@@ -727,7 +758,11 @@ def typing(simulation, full_path_base_fname, locus_list, genotype_genome, partia
                     ref_common.align_reads(aligner, simulation, full_path_base_fname + "." + index_type, index_type, base_fname,
                                            read_fname, fastq, threads, aln, verbose)
             elif native:
-                native_text = sam_intake.read_alignment_text(aln)  # None for BAM: falls through to samtools
+                kind, data = sam_intake.read_alignment(aln, threads)
+                if kind == "bam":
+                    native_bam = data
+                elif kind == "sam":
+                    native_text = data
             genes_here = []
             for entry in locus_list:
                 gene = entry[0].split("*")[0] if simulation else entry
@@ -743,6 +778,10 @@ def typing(simulation, full_path_base_fname, locus_list, genotype_genome, partia
             if native_text is not None:
                 # native intake (sam_intake.py): one pass over the SAM text instead of `samtools view | sort -k1,1 -s` per locus
                 by_ref = sam_intake.split_sam(native_text, [refGenes[g] for g in genes_here], threads)
+                alignments = {g: by_ref[refGenes[g]] for g in genes_here}
+            elif native_bam is not None:
+                # BAM: the host splits the records, the GPU renders them into alignment text (packed units)
+                by_ref = sam_intake.split_bam(native_bam, [refGenes[g] for g in genes_here], threads)
                 alignments = {g: by_ref[refGenes[g]] for g in genes_here}
             else:
                 alignments = {}

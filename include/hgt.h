@@ -57,7 +57,8 @@ int hgt_sm_count(const hgt_ctx *ctx);
  * events on the launching stream.  stage_ms / stage_launches [8]: [0] line index + record parse + pileup, [1]
  * haplotype->allele-set (compat), [2] per-pair class + de-duplication, [3] Gene_counts, [4] first-level EM, [5]
  * projection, [6] second-level EM, [7] run heads + mate de-dup + walk + ambiguity pass + pair jobs.
- * h2d/d2h_bytes count every host<->device copy the library issued since the last reset. */
+ * h2d/d2h_bytes count every host<->device copy the library issued since the last reset (a BAM unit counts its blob
+ * bytes, not the text rendered from it). */
 void hgt_profile_enable(hgt_ctx *ctx, int on);
 void hgt_profile_reset(hgt_ctx *ctx);
 void hgt_profile_read(const hgt_ctx *ctx, double *stage_ms, int64_t *stage_launches, int64_t *h2d_bytes,
@@ -290,7 +291,8 @@ int hgt_typing_em(hgt_ctx *ctx, const hgt_typing *t, int32_t table, const uint64
 /* ---- batches of (sample, locus) units ----------------------------------------------------------------------
  * The production shape of the path: the reference types one (sample, locus) at a time inside Pool workers
  * (hisatgenotype:613-665, core:370); here any number of units over any number of loci go through the GPU
- * together.  prepare = the alignment text goes to the device as it is (one arena, one line count);
+ * together.  prepare = the alignment text goes to the device as it is (one arena, one line count; BAM units go as
+ * packed records and are rendered into their arena slices on the device, hgt_batch_add_unit_bam);
  * execute = GPU only: line index, record parse + filters, pileup, mate de-dup, CIGAR x MD x Zs walk with error
  * correction, ambiguity expansion, pair jobs, haplotype->allele-set, per-pair class, class de-duplication, Gene_counts
  * and the first-level EM (exon table on the hla path, Gene table otherwise) for every unit; the host only reads back
@@ -308,6 +310,16 @@ int64_t hgt_batch_add_unit(hgt_batch *b, int32_t locus_index, const char *sam_te
 /* n units in one call; returns the index of the first one (the others follow) or a negative status */
 int64_t hgt_batch_add_units(hgt_batch *b, int64_t n, const int32_t *locus_index, const char *const *sam_text,
                             const size_t *n_bytes);
+/* A unit given as a packed BAM unit (hgt_bam_split_write_records) instead of text: prepare copies the blob to the device
+ * and renders its records there into the unit's slice of the text arena, byte for byte what hgt_bam_split_write_text
+ * gives; everything after that is the text path.  The blob's header, name table and offset table are checked here
+ * (HGT_ERR_ARG when an offset leaves the blob); blob must be 8-byte aligned and stay valid until prepare returns.
+ * Page-locked blobs are copied directly, pageable ones staged like text.  BAM and text units mix in one batch; a batch
+ * without BAM units does exactly what it did before. */
+int64_t hgt_batch_add_unit_bam(hgt_batch *b, int32_t locus_index, const void *blob, size_t n_bytes);
+/* After prepare: the unit's slice of the device text arena (the rendered text of a BAM unit, the caller's text of a text
+ * unit).  dst NULL: *n_bytes = its length; else *n_bytes (capacity in, length out) must hold it. */
+int hgt_batch_unit_text(const hgt_batch *b, int64_t unit, char *dst, size_t *n_bytes);
 /* Read-sharded locus (several processes hold disjoint reads of the same (sample, locus), SURVEY.md 8e): error
  * correction depends on the pileup of ALL reads (common:1124-1134), so prepare calls the hook once, after the raw
  * base counts of this process are on the device and before nt_set is derived; the hook sums dev_counts
@@ -381,6 +393,26 @@ int hgt_sam_split_create_opts(const char *sam_text, size_t n_bytes, int32_t n_re
 int hgt_sam_split_sizes(const hgt_sam_split *s, size_t *bytes_per_ref, int64_t *lines_per_ref);
 int hgt_sam_split_write(const hgt_sam_split *s, int32_t ref, char *dst);
 void hgt_sam_split_free(hgt_sam_split *s);
+
+/* ---- native BAM intake (host split, device render) ------------------------------------------------------------
+ * The same replacement for a BAM file.  bam = the DECOMPRESSED BAM stream (magic "BAM\1", header, records; BGZF is
+ * inflated by the caller, e.g. sam_intake.read_bgzf).  Every record is validated completely: a block_size that disagrees
+ * with l_read_name / n_cigar_op / l_seq / the aux bytes, a read name without NUL, an aux tag of unknown type or past the
+ * record end, a refID outside the header give HGT_ERR_PARSE naming the read; float tags (f, d, B:f) and the long-CIGAR
+ * placeholder CG give HGT_ERR_UNSUPPORTED naming the read and the tag.  Records are bucketed by refID into the given
+ * backbones (the SAM split's RNAME rule) and ordered by the same rule as hgt_sam_split_*.  flags: HGT_SPLIT_DROP_QUAL
+ * leaves the QUAL bytes out (the text then carries '*').  `bam` must stay valid until the handle is freed.
+ * A bucket leaves as a packed unit (layout: csrc/bam_dev.cuh) for hgt_batch_add_unit_bam (hgt_bam_split_write_records;
+ * dst 8-byte aligned, e.g. page-locked memory) or as the SAM text `samtools view` prints for its records
+ * (hgt_bam_split_write_text, rendered on the host by the functions the device render runs).  sizes: blob bytes, text
+ * bytes (rendered on demand: pass NULL when not needed) and records per reference; any pointer may be NULL. */
+typedef struct hgt_bam_split hgt_bam_split;
+int hgt_bam_split_create(const void *bam, size_t n_bytes, int32_t n_refs, const char *const *ref_names, int32_t n_threads,
+                         int32_t flags, hgt_bam_split **out);
+int hgt_bam_split_sizes(const hgt_bam_split *s, size_t *blob_bytes, size_t *text_bytes, int64_t *records);
+int hgt_bam_split_write_records(const hgt_bam_split *s, int32_t ref, void *dst);
+int hgt_bam_split_write_text(const hgt_bam_split *s, int32_t ref, char *dst);
+void hgt_bam_split_free(hgt_bam_split *s);
 
 /* Host EMULATION of the record stage with a caller-supplied pileup (no GPU needed; test infrastructure, not on the
  * typing path): the same __host__ __device__ functions the kernels call (csrc/walk_dev.cuh: parse, filters, mate
