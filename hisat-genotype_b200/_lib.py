@@ -96,6 +96,16 @@ def lib():
         L.hgt_bam_split_write_text.argtypes = [c_void_p, c_i32, c_void_p]
         L.hgt_bam_split_free.restype = None
         L.hgt_bam_split_free.argtypes = [c_void_p]
+        L.hgt_bgzf_open.restype = c_int
+        L.hgt_bgzf_open.argtypes = [c_i32, c_void_p, c_void_p, P(c_void_p)]
+        L.hgt_bgzf_sizes.restype = c_int
+        L.hgt_bgzf_sizes.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p]
+        L.hgt_bgzf_inflate.restype = c_int
+        L.hgt_bgzf_inflate.argtypes = [c_void_p, c_void_p, c_void_p]
+        L.hgt_bgzf_inflate_host.restype = c_int
+        L.hgt_bgzf_inflate_host.argtypes = [c_void_p, c_i32, c_void_p]
+        L.hgt_bgzf_free.restype = None
+        L.hgt_bgzf_free.argtypes = [c_void_p]
         L.hgt_batch_add_unit_bam.restype = c_i64
         L.hgt_batch_add_unit_bam.argtypes = [c_void_p, c_i32, c_void_p, c_size_t]
         L.hgt_batch_unit_text.restype = c_int
@@ -184,6 +194,16 @@ class PinnedText:
         addr = self.base.value + self.used
         self.used += (n + 15) & ~15
         return addr, n
+
+    def reset(self):
+        """Hand the whole arena out again; earlier slices are no longer the caller's."""
+        self.used = 0
+
+    def view(self, addr, n):
+        """A writable buffer (memoryview of unsigned bytes) over [addr, addr + n) of the arena; it keeps the arena alive."""
+        arr = (ctypes.c_ubyte * int(n)).from_address(addr)
+        arr._owner = self
+        return memoryview(np.ctypeslib.as_array(arr)) if n else memoryview(b"")
 
     def close(self):
         if self.base is not None and self.base.value:

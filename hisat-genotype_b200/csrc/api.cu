@@ -87,7 +87,7 @@ cudaError_t hgt_small_h2d(void *dst_dev, const void *src_pinned, size_t bytes, c
 }
 
 extern "C" const char *hgt_last_error(void) { return g_err; }
-extern "C" int hgt_abi_version(void) { return 2; }
+extern "C" int hgt_abi_version(void) { return 3; }
 extern "C" int hgt_row_pitch(int n_alleles) {
     int w = (n_alleles + 63) / 64;
     if (w < 2) w = 2;

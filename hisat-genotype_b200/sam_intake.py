@@ -8,6 +8,7 @@ alignment text there (hgt_batch_add_unit_bam)."""
 from __future__ import annotations
 
 import ctypes
+import os
 import struct
 import zlib
 
@@ -121,8 +122,66 @@ def read_bgzf(data, n_threads=0):
         return b"".join(pool.map(lambda c: _inflate_blocks(data, c), chunks))
 
 
+def _bgzf_run(streams, inflate, pinned):
+    """hgt_bgzf_open on the streams (any buffers), then inflate(handle, dst) into page-locked memory (pinned: True for a
+    new arena, or a _lib.PinnedText to take it from) or into ordinary memory (False): one buffer per stream.  Header
+    errors and rejected blocks raise AssertionError (HGT_ERR_PARSE)."""
+    L = _lib.lib()
+    arrs = [np.frombuffer(s, np.uint8) for s in streams]
+    n = len(arrs)
+    ptrs = (ctypes.c_void_p * max(n, 1))(*[a.ctypes.data if a.size else None for a in arrs])
+    sizes = (ctypes.c_size_t * max(n, 1))(*[a.size for a in arrs])
+    h = ctypes.c_void_p()
+    rc = L.hgt_bgzf_open(n, ptrs, sizes, ctypes.byref(h))
+    if rc == _lib.HGT_ERR_PARSE:
+        raise AssertionError(_lib.last_error())
+    _lib.check(rc)
+    try:
+        out_n = (ctypes.c_size_t * max(n, 1))()
+        eof = (ctypes.c_int32 * max(n, 1))()
+        _lib.check(L.hgt_bgzf_sizes(h, out_n, None, eof))
+        for i in range(n):
+            if not eof[i]:
+                import warnings
+                warnings.warn("BGZF input has no EOF marker block; it may be truncated")
+        if pinned:
+            arena = pinned if isinstance(pinned, _lib.PinnedText) else _lib.PinnedText(sum(out_n[:n]) + 16 * n + 16)
+            addrs = [arena.reserve(out_n[i])[0] for i in range(n)]
+            outs = [arena.view(a, out_n[i]) for i, a in enumerate(addrs)]
+        else:
+            outs = [np.empty(out_n[i], np.uint8) for i in range(n)]
+            addrs = [o.ctypes.data for o in outs]
+            outs = [memoryview(o) for o in outs]
+        rc = inflate(h, (ctypes.c_void_p * max(n, 1))(*addrs))
+        if rc == _lib.HGT_ERR_PARSE:
+            raise AssertionError(_lib.last_error())
+        _lib.check(rc)
+        return outs
+    finally:
+        L.hgt_bgzf_free(h)
+
+
+def inflate_bgzf(streams, device=None, pinned=None):
+    """Inflate BGZF streams (a list of buffers, e.g. BAM files) on the GPU in one call: one warp per block, every block's
+    CRC32 and ISIZE checked on the device (hgt_bgzf_inflate).  Returns one buffer per stream, backed by page-locked memory,
+    whose bytes() equal read_bgzf's.  A missing EOF block warns as read_bgzf does; a malformed or corrupt block raises
+    AssertionError naming the stream and byte offset.  A block of ISIZE > 65536 (which no BGZF writer produces) is refused
+    here, and read_bgzf accepts it.  pinned: a _lib.PinnedText to take the output from instead of a new allocation."""
+    L = _lib.lib()
+    ctx = _lib.ctx(device)
+    return _bgzf_run(streams, lambda h, dst: L.hgt_bgzf_inflate(ctx, h, dst), pinned if pinned is not None else True)
+
+
+def inflate_bgzf_host(streams, n_threads=0):
+    """The host emulation of inflate_bgzf (hgt_bgzf_inflate_host: the device decoder's code on host threads) - test
+    infrastructure, not on the typing path; the buffers are in ordinary memory."""
+    L = _lib.lib()
+    return _bgzf_run(streams, lambda h, dst: L.hgt_bgzf_inflate_host(h, int(n_threads), dst), False)
+
+
 def split_bam(bam_bytes, ref_names, n_threads=0, pinned=None, drop_qual=False, text=False):
-    """bam_bytes: a BAM file (BGZF, inflated first by read_bgzf) or its decompressed stream.  ref_names: backbone names.
+    """bam_bytes: a BAM file (BGZF, inflated first by read_bgzf) or its decompressed stream (any buffer, e.g. what
+    inflate_bgzf returns; it is read in place).  ref_names: backbone names.
     Returns {ref_name: BamUnit} (packed records for Batch.add_unit_bam), with text=True {ref_name: bytes} (the SAM text
     `samtools view` prints for the same records, in the same order as split_sam), or with pinned=_lib.PinnedText
     {ref_name: (address, n_bytes)} of either written into it.  Records are bucketed and ordered as split_sam does.
@@ -130,14 +189,14 @@ def split_bam(bam_bytes, ref_names, n_threads=0, pinned=None, drop_qual=False, t
     CG long-CIGAR tag raise HgtError (HGT_ERR_UNSUPPORTED)."""
     if bytes(bam_bytes[:2]) == b"\x1f\x8b":
         bam_bytes = read_bgzf(bam_bytes, n_threads)
-    bam_bytes = bytes(bam_bytes)
+    stream = np.frombuffer(bam_bytes, np.uint8)  # no copy: the split reads the caller's buffer (alive until the handle is freed)
     L = _lib.lib()
     n = len(ref_names)
     enc = [r.encode() for r in ref_names]
     arr = (ctypes.c_char_p * n)(*enc)
     h = ctypes.c_void_p()
-    rc = L.hgt_bam_split_create(bam_bytes, len(bam_bytes), n, arr, int(n_threads), 1 if drop_qual else 0,
-                                ctypes.byref(h))
+    rc = L.hgt_bam_split_create(stream.ctypes.data_as(ctypes.c_void_p), stream.size, n, arr, int(n_threads),
+                                1 if drop_qual else 0, ctypes.byref(h))
     if rc == _lib.HGT_ERR_PARSE:
         raise AssertionError(_lib.last_error())
     _lib.check(rc)
@@ -197,10 +256,26 @@ def align_to_sam(simulation, index_name, base_fname, read_fname, fastq, threads,
     return proc.stdout
 
 
-def read_alignment(path, n_threads=0):
+def read_alignment(path, n_threads=0, device=None):
     """The alignment file as the native intake takes it: ("sam", text), ("bam", decompressed BAM stream), or (None, None)
-    for what stays with samtools, like the reference: CRAM, and BGZF that is not BAM."""
+    for what stays with samtools, like the reference: CRAM, and BGZF that is not BAM.  With a device, a BGZF file is read
+    into page-locked memory and inflated on that GPU (inflate_bgzf); the BAM stream is then a page-locked buffer."""
     with open(path, "rb") as f:
+        head = f.read(4)
+        if device is not None and head[:2] == b"\x1f\x8b" and head[3:4] and head[3] & 4:
+            n = os.fstat(f.fileno()).st_size
+            pinned = _lib.PinnedText(n)
+            data = pinned.view(pinned.reserve(n)[0], n)
+            f.seek(0)
+            got = 0
+            while got < n:
+                k = f.readinto(data[got:])
+                if not k:
+                    break
+                got += k
+            raw = inflate_bgzf([data[:got]], device)[0]
+            return ("bam", raw) if bytes(raw[:4]) == b"BAM\1" else (None, None)
+        f.seek(0)
         data = f.read()
     if data[:4] == b"CRAM":
         return None, None

@@ -758,7 +758,7 @@ def typing(simulation, full_path_base_fname, locus_list, genotype_genome, partia
                     ref_common.align_reads(aligner, simulation, full_path_base_fname + "." + index_type, index_type, base_fname,
                                            read_fname, fastq, threads, aln, verbose)
             elif native:
-                kind, data = sam_intake.read_alignment(aln, threads)
+                kind, data = sam_intake.read_alignment(aln, threads, device=_lib.default_device())  # BGZF inflates on the GPU
                 if kind == "bam":
                     native_bam = data
                 elif kind == "sam":

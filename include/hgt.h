@@ -414,6 +414,30 @@ int hgt_bam_split_write_records(const hgt_bam_split *s, int32_t ref, void *dst);
 int hgt_bam_split_write_text(const hgt_bam_split *s, int32_t ref, char *dst);
 void hgt_bam_split_free(hgt_bam_split *s);
 
+/* ---- BGZF inflate (BAM's compression) on the GPU ----------------------------------------------------------------
+ * Replaces read_bgzf's zlib thread pool (sam_intake.py) for the native BAM intake.  open: host walk of the block headers
+ * of n_streams BGZF streams (the rules of sam_intake._bgzf_blocks: gzip magic, FEXTRA, BC subfield, BSIZE within the
+ * stream) plus ISIZE <= 65536 -> per stream the inflated size (sum of ISIZE), block count, and whether it ends in the EOF
+ * marker block.  A malformed header gives HGT_ERR_PARSE naming the stream and byte offset, with read_bgzf's wording.
+ * ISIZE > 65536 is the one input read_bgzf accepts and this path refuses: the BGZF spec caps a block at 64 KiB, htslib
+ * never writes more, and the cap bounds the output a block can claim.
+ * inflate: compressed bytes to the device, ONE kernel launch per call (bgzf_inflate_kernel: one warp per block, all
+ * blocks of all streams; none when there is no block), CRC32 + ISIZE checked on the device, stream i's bytes into dst[i]
+ * (page-locked dst is written by the copy engine directly), one synchronisation.  A block is accepted exactly when zlib's
+ * raw inflate accepts it with nothing left over and the trailer agrees (read_bgzf's decision).  The first failing block
+ * gives HGT_ERR_PARSE "stream %d: BGZF block at byte %d: <rule>", with zlib's or read_bgzf's wording where the rule is
+ * the same; dst then holds unspecified bytes and the context stays usable.  h2d_bytes grows by the streams' bytes plus
+ * 16 * (blocks + 1) bytes of block offsets, d2h_bytes by the inflated bytes plus an 8-byte status word.
+ * Input must stay valid until the handle is freed. */
+typedef struct hgt_bgzf hgt_bgzf;
+int hgt_bgzf_open(int32_t n_streams, const void *const *data, const size_t *n_bytes, hgt_bgzf **out);
+int hgt_bgzf_sizes(const hgt_bgzf *z, size_t *out_bytes, int64_t *n_blocks, int32_t *has_eof);   /* [n_streams] each */
+int hgt_bgzf_inflate(hgt_ctx *ctx, const hgt_bgzf *z, void *const *dst);
+/* Host EMULATION (test infrastructure, not on the typing path): the same bgzf_dev.cuh functions on host threads
+ * (n_threads <= 0: all cores), the same decisions and messages. */
+int hgt_bgzf_inflate_host(const hgt_bgzf *z, int32_t n_threads, void *const *dst);
+void hgt_bgzf_free(hgt_bgzf *z);
+
 /* Host EMULATION of the record stage with a caller-supplied pileup (no GPU needed; test infrastructure, not on the
  * typing path): the same __host__ __device__ functions the kernels call (csrc/walk_dev.cuh: parse, filters, mate
  * de-dup, walk, error correction, ambiguity expansion, exon clipping, pair jobs) run in plain loops.  Output is the

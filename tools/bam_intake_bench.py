@@ -6,8 +6,13 @@ DRB1, paired-end 2x100 bp, 30x, the seeded synthetic database and reads of bench
   - prepare (copies + BAM render + line count, ending in a synchronise) for text / text without QUAL / BAM blobs / BAM blobs
     without QUAL, all from page-locked memory, with h2d_bytes from hgt_profile_read;
   - execute + finish.
-The calls of every variant must equal the text run's (exit status 1 otherwise).  Prints one JSON line (GPU name and power
-limit included) and writes it to --out when given.
+  - BGZF inflate on the GPU (sam_intake.inflate_bgzf) from page-locked input to page-locked output, ending in a
+    synchronise: the step's files in one call (bgzf_inflate_gpu_ms) and as one call per file, the shape typing() uses
+    (bgzf_inflate_gpu_per_file_ms); the kernel alone from torch.profiler's device records (bgzf_inflate_kernel_ms); the
+    compressed / inflated bytes and the call's h2d / d2h bytes; and split_bam fed from one-file inflate_bgzf calls
+    (split_bam_gpu_inflate_ms, against split_bam_ms).
+The calls of every variant must equal the text run's, and every file's GPU-inflated bytes read_bgzf's (exit status 1
+otherwise).  Prints one JSON line (GPU name and power limit included) and writes it to --out when given.
 
 usage: python tools/bam_intake_bench.py [--samples 128] [--steps 3] [--warmup 1] [--threads 0] [--out FILE]"""
 import argparse
@@ -54,7 +59,7 @@ def main():
     from hisatgenotype_b200 import _lib, synth
     from hisatgenotype_b200 import typing_core as TC
     from hisatgenotype_b200.locus import LocusTables
-    from hisatgenotype_b200.sam_intake import read_bgzf, split_bam, split_sam
+    from hisatgenotype_b200.sam_intake import inflate_bgzf, read_bgzf, split_bam, split_sam
 
     threads = args.threads or os.cpu_count() or 1
     info = gpu_info()
@@ -142,6 +147,55 @@ def main():
             fn()
             ts.append((time.perf_counter() - t) * 1e3)
         res[name] = {"mean": round(float(np.mean(ts)), 2), "min": round(float(np.min(ts)), 2)}
+    # BGZF inflate on the GPU: page-locked input, output into one reused page-locked arena
+    inflated = [read_bgzf(b, threads) for b in bams]
+    fin = _lib.PinnedText(sum(len(b) + 16 for b in bams) + 16)
+    bams_pinned = [fin.view(*fin.add(b)) for b in bams]
+    fout = _lib.PinnedText(sum(len(x) + 16 for x in inflated) + 16)
+
+    def gpu_one_call():
+        fout.reset()
+        return inflate_bgzf(bams_pinned, pinned=fout)
+
+    def gpu_per_file():
+        fout.reset()
+        return [inflate_bgzf([b], pinned=fout)[0] for b in bams_pinned]
+
+    def split_gpu():
+        fout.reset()
+        return [split_bam(inflate_bgzf([b], pinned=fout)[0], refs, threads) for b in bams_pinned]
+
+    inflate_ok = all(bytes(g) == w for g, w in zip(gpu_one_call(), inflated))
+    inflate_ok = inflate_ok and all(bytes(g) == w for g, w in zip(gpu_per_file(), inflated))
+    L.hgt_profile_reset(ctx)
+    gpu_one_call()
+    L.hgt_profile_read(ctx, None, None, ctypes.byref(h2d), ctypes.byref(d2h))
+    res.update({"bgzf_compressed_bytes": sum(len(b) for b in bams), "bgzf_inflated_bytes": sum(len(x) for x in inflated),
+                "bgzf_inflate_call_h2d_bytes": h2d.value, "bgzf_inflate_call_d2h_bytes": d2h.value})
+    for name, fn in (("bgzf_inflate_gpu_ms", gpu_one_call), ("bgzf_inflate_gpu_per_file_ms", gpu_per_file),
+                     ("split_bam_gpu_inflate_ms", split_gpu)):
+        for _ in range(args.warmup):
+            fn()
+        ts = []
+        for _ in range(args.steps):
+            t = time.perf_counter()
+            fn()
+            ts.append((time.perf_counter() - t) * 1e3)
+        res[name] = {"mean": round(float(np.mean(ts)), 2), "min": round(float(np.min(ts)), 2)}
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(args.steps):
+            gpu_one_call()
+    kern = [e for e in prof.key_averages() if "bgzf_inflate_kernel" in e.key]
+    if kern:
+        total_us = getattr(kern[0], "device_time_total", None) or getattr(kern[0], "cuda_time_total", 0)
+        res["bgzf_inflate_kernel_ms"] = round(total_us / 1e3 / max(kern[0].count, 1), 3)
+        res["bgzf_inflate_kernel_launches"] = kern[0].count
+    else:
+        res["bgzf_inflate_kernel_ms"] = None  # the profiler recorded no kernel of that name
+    res["inflate_identical"] = inflate_ok
+    fin.close()
+    fout.close()
     # prepare / execute + finish per variant, the variants alternating inside every step
     ref_calls = None
     ok = True
@@ -174,7 +228,7 @@ def main():
         buf.close()
     for t in tables:
         t.close()
-    sys.exit(0 if ok else 1)
+    sys.exit(0 if ok and inflate_ok else 1)
 
 
 if __name__ == "__main__":
