@@ -108,6 +108,16 @@ def lib():
         L.hgt_bgzf_free.argtypes = [c_void_p]
         L.hgt_batch_add_unit_bam.restype = c_i64
         L.hgt_batch_add_unit_bam.argtypes = [c_void_p, c_i32, c_void_p, c_size_t]
+        L.hgt_bam_dsplit_create.restype = c_int
+        L.hgt_bam_dsplit_create.argtypes = [c_void_p, c_void_p, c_i32, c_void_p, c_i32, P(c_void_p)]
+        L.hgt_bam_dsplit_sizes.restype = c_int
+        L.hgt_bam_dsplit_sizes.argtypes = [c_void_p, c_void_p, c_void_p]
+        L.hgt_bam_dsplit_free.restype = None
+        L.hgt_bam_dsplit_free.argtypes = [c_void_p]
+        L.hgt_batch_add_unit_bam_dsplit.restype = c_i64
+        L.hgt_batch_add_unit_bam_dsplit.argtypes = [c_void_p, c_i32, c_void_p, c_i32, c_i32]
+        L.hgt_bam_index_host.restype = c_int
+        L.hgt_bam_index_host.argtypes = [c_void_p, c_size_t, c_i64, c_i32, c_i64, c_void_p, P(c_i64)]
         L.hgt_batch_unit_text.restype = c_int
         L.hgt_batch_unit_text.argtypes = [c_void_p, c_i64, c_void_p, P(c_size_t)]
         L.hgt_batch_unit_reads.restype = c_int

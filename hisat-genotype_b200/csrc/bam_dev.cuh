@@ -1,5 +1,5 @@
 // BAM records -> SAM text lines, the rules of htslib's sam_format1 (what `samtools view` prints), as __host__ __device__
-// functions: the device render of a batch (typing.cu: bam_text_len_kernel, bam_render_kernel) and the host render of the
+// functions: the device render of a batch (bam_kernels.cuh: bam_text_len_kernel, bam_render_kernel) and the host render of the
 // BAM split (bam_split.cpp: hgt_bam_split_write_text) call the same code, so the host render pins the device's output.
 //
 // Packed unit (hgt_bam_split_write_records, hgt_batch_add_unit_bam), little-endian, offsets from the blob's first byte:
@@ -64,8 +64,10 @@ struct BamRec {
     bool has_qual;  // QUAL bytes are present and not 0xff-marked as absent
 };
 
-// p: 4-byte aligned, extent >= REC_FIXED (bam_unit_check guarantees both)
-HGT_HD void bam_decode(const unsigned char *p, uint64_t extent, bool qual_dropped, BamRec *r) {
+// extent >= REC_FIXED (bam_unit_check guarantees it for a packed unit, the chain rule for a record of a stream).  Every
+// load is bytewise, so p may have any alignment (records inside a decompressed stream are not 4-byte aligned).
+// qual_dropped: the record carries no QUAL bytes; qual_hidden: it carries them and the text leaves them out ('*').
+HGT_HD void bam_decode(const unsigned char *p, uint64_t extent, bool qual_dropped, BamRec *r, bool qual_hidden = false) {
     r->p = p;
     const int64_t bs = (int64_t)ld_i32(p) + 4;
     const uint32_t end = (uint32_t)(bs < (int64_t)REC_FIXED ? REC_FIXED : (uint64_t)bs > extent ? extent : (uint64_t)bs);
@@ -94,7 +96,7 @@ HGT_HD void bam_decode(const unsigned char *p, uint64_t extent, bool qual_droppe
     r->has_qual = false;
     if (!qual_dropped) {
         if (r->l_seq <= end - o) {
-            r->has_qual = r->l_seq > 0 && p[o] != 0xff;
+            r->has_qual = !qual_hidden && r->l_seq > 0 && p[o] != 0xff;
             o += r->l_seq;
         } else {
             o = end;

@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "bam_dev.cuh"
+#include "bam_rec.cuh"
 #include "common.cuh"
 #include "split_order.hpp"
 
@@ -43,94 +44,6 @@ struct RecError {
 };
 
 uint32_t a4(uint64_t x) { return (uint32_t)((x + 3) & ~3ull); }
-
-// Complete check of the record at p (size = block_size + 4 bytes, inside the stream).  Returns HGT_OK, HGT_ERR_PARSE or
-// HGT_ERR_UNSUPPORTED with *why set.
-int check_record(const unsigned char *p, uint32_t size, int32_t n_hdr, std::string *why) {
-    using namespace hgtb;
-    if (size < REC_FIXED) {
-        *why = "block_size shorter than the fixed fields";
-        return HGT_ERR_PARSE;
-    }
-    const uint32_t l_name = p[12], n_cigar = ld_u16(p + 16);
-    const int32_t l_seq = ld_i32(p + 20), ref = ld_i32(p + 4), next_ref = ld_i32(p + 24);
-    if (l_name < 1 || REC_FIXED + l_name > size || p[REC_FIXED + l_name - 1] != 0) {
-        *why = "read name is not NUL-terminated inside the record";
-        return HGT_ERR_PARSE;
-    }
-    if (l_seq < 0) {
-        *why = "negative l_seq";
-        return HGT_ERR_PARSE;
-    }
-    const uint64_t aux = (uint64_t)REC_FIXED + l_name + 4ull * n_cigar + ((uint64_t)l_seq + 1) / 2 + (uint64_t)l_seq;
-    if (aux > size) {
-        *why = "block_size inconsistent with l_read_name, n_cigar_op and l_seq";
-        return HGT_ERR_PARSE;
-    }
-    if (ref < -1 || ref >= n_hdr || next_ref < -1 || next_ref >= n_hdr) {
-        *why = "refID or next_refID outside the reference list";
-        return HGT_ERR_PARSE;
-    }
-    for (uint32_t k = 0; k < n_cigar; k++)
-        if ((ld_u32(p + REC_FIXED + l_name + 4 * k) & 15) > 8) {
-            *why = "unknown CIGAR operation";
-            return HGT_ERR_PARSE;
-        }
-    uint64_t o = aux;
-    while (o < size) {
-        if (o + 3 > size) {
-            *why = "aux tag runs past the record end";
-            return HGT_ERR_PARSE;
-        }
-        const unsigned char *t = p + o;
-        const std::string tag((const char *)t, 2);
-        if (tag == "CG") {
-            *why = "tag CG (long CIGAR placeholder) is not supported";
-            return HGT_ERR_UNSUPPORTED;
-        }
-        const unsigned char ty = t[2];
-        uint64_t n = 0;
-        if (ty == 'f' || ty == 'd') {
-            *why = "tag " + tag + " of float type is not supported";
-            return HGT_ERR_UNSUPPORTED;
-        } else if (ty == 'Z' || ty == 'H') {
-            const void *z = memchr(t + 3, 0, size - o - 3);
-            if (!z) {
-                *why = "aux tag " + tag + " runs past the record end";
-                return HGT_ERR_PARSE;
-            }
-            n = 3 + (uint64_t)((const unsigned char *)z - (t + 3)) + 1;
-        } else if (ty == 'B') {
-            if (o + 8 > size) {
-                *why = "aux tag " + tag + " runs past the record end";
-                return HGT_ERR_PARSE;
-            }
-            if (t[3] == 'f') {
-                *why = "tag " + tag + " (B array of floats) is not supported";
-                return HGT_ERR_UNSUPPORTED;
-            }
-            const uint32_t w = t[3] == 'A' ? 0 : aux_int_size(t[3]);
-            if (!w) {
-                *why = "aux tag " + tag + " has an unknown B subtype";
-                return HGT_ERR_PARSE;
-            }
-            n = 8 + (uint64_t)ld_u32(t + 4) * w;
-        } else {
-            const uint32_t w = aux_int_size(ty);
-            if (!w) {
-                *why = "aux tag " + tag + " has an unknown type";
-                return HGT_ERR_PARSE;
-            }
-            n = 3 + w;
-        }
-        if (o + n > size) {
-            *why = "aux tag " + tag + " runs past the record end";
-            return HGT_ERR_PARSE;
-        }
-        o += n;
-    }
-    return HGT_OK;
-}
 
 void pack(const hgt_bam_split *s, size_t r, unsigned char *dst) {
     using namespace hgtb;
@@ -217,41 +130,25 @@ extern "C" int hgt_bam_split_create(const void *bam, size_t n_bytes, int32_t n_r
     *out = nullptr;
     n_threads = hgt_split::default_threads(n_threads);
     const unsigned char *b = static_cast<const unsigned char *>(bam);
-    // header: magic, l_text, text, n_ref, (l_name, name, l_ref) * n_ref
-    if (n_bytes < 12 || memcmp(b, "BAM\1", 4) != 0) {
-        hgt_set_error("hgt_bam_split_create: not a BAM stream (bad magic)");
+    uint64_t o = 0;
+    std::vector<std::string> hdr_names;
+    const int hrc = bam_parse_header(b, n_bytes, &o, &hdr_names);
+    if (hrc != HDR_OK) {
+        hgt_set_error("hgt_bam_split_create: %s", bam_header_why(hrc));
         return HGT_ERR_PARSE;
     }
-    const int32_t l_text = ld_i32(b + 4);
-    if (l_text < 0 || 8ull + (uint64_t)l_text + 4 > n_bytes) {
-        hgt_set_error("hgt_bam_split_create: truncated BAM header");
-        return HGT_ERR_PARSE;
-    }
-    uint64_t o = 8 + (uint64_t)l_text;
-    const int32_t n_hdr = ld_i32(b + o);
-    o += 4;
-    if (n_hdr < 0) {
-        hgt_set_error("hgt_bam_split_create: negative reference count in the BAM header");
-        return HGT_ERR_PARSE;
-    }
+    const int32_t n_hdr = (int32_t)hdr_names.size();
     hgt_bam_split *s = new hgt_bam_split();
     s->bam = b;
     s->drop_qual = (flags & HGT_SPLIT_DROP_QUAL) != 0;
     for (int32_t r = 0; r < n_refs; r++) s->ref_names.emplace_back(ref_names[r]);
     std::unordered_map<std::string, int> ref_index;
     for (int r = 0; r < n_refs; r++) ref_index[ref_names[r]] = r;
+    s->hdr_names = std::move(hdr_names);
     std::vector<int> ref_of_hdr;
-    for (int32_t k = 0; k < n_hdr; k++) {
-        const int32_t l_name = o + 4 <= n_bytes ? ld_i32(b + o) : -1;
-        if (l_name < 1 || o + 4 + (uint64_t)l_name + 4 > n_bytes || b[o + 4 + (uint64_t)l_name - 1] != 0) {
-            delete s;
-            hgt_set_error("hgt_bam_split_create: truncated or malformed reference list in the BAM header");
-            return HGT_ERR_PARSE;
-        }
-        s->hdr_names.emplace_back((const char *)b + o + 4, (size_t)l_name - 1);
-        auto it = ref_index.find(s->hdr_names.back());
+    for (const std::string &nm : s->hdr_names) {
+        auto it = ref_index.find(nm);
         ref_of_hdr.push_back(it == ref_index.end() ? -1 : it->second);
-        o += 4 + (uint64_t)l_name + 4;
     }
     // record boundaries: one sequential pass over the block_size chain
     std::vector<uint64_t> rec_at;
@@ -278,13 +175,12 @@ extern "C" int hgt_bam_split_create(const void *bam, size_t n_bytes, int32_t n_r
         for (size_t i = i0; i < i1; i++) {
             const unsigned char *p = b + rec_at[i];
             const uint32_t size = (uint32_t)ld_i32(p) + 4;
-            std::string why;
-            const int rc = check_record(p, size, n_hdr, &why);
-            if (rc != HGT_OK) {
+            unsigned char tag[2] = {0, 0};
+            const int rule = bam_check_record(p, size, n_hdr, tag);
+            if (rule != RULE_OK) {
                 err[k].index = i;
-                err[k].code = rc;
-                const size_t ln = p[12] && REC_FIXED + p[12] <= size ? strnlen((const char *)p + REC_FIXED, p[12]) : 0;
-                err[k].msg = "read '" + std::string((const char *)p + REC_FIXED, ln) + "': " + why;
+                err[k].code = rule_unsupported(rule) ? HGT_ERR_UNSUPPORTED : HGT_ERR_PARSE;
+                err[k].msg = bam_record_message(p, size, rule, tag);
                 return;
             }
             const int32_t ref = ld_i32(p + 4);

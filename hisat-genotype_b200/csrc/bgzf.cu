@@ -8,6 +8,7 @@
 #include <vector>
 
 #include "bgzf_dev.cuh"
+#include "bgzf_host.h"
 #include "common.cuh"
 
 namespace {
@@ -42,28 +43,13 @@ uint32_t le32(const uint8_t *p) { return p[0] | (uint32_t)p[1] << 8 | (uint32_t)
 
 }  // namespace
 
-struct hgt_bgzf {
-    int32_t n_streams = 0;
-    std::vector<const uint8_t *> data;
-    std::vector<size_t> n_bytes;
-    std::vector<int32_t> has_eof;
-    // blocks of all streams in order; in_off / out_off [n_blocks + 1]: block b = input [in_off[b], in_off[b+1]) of the
-    // streams laid end to end, output [out_off[b], out_off[b+1])
-    std::vector<uint64_t> in_off, out_off;
-    std::vector<int64_t> stream_blk;    // [n_streams + 1] first block of each stream
-    std::vector<uint64_t> stream_in, stream_out;  // [n_streams + 1]
-    int64_t n_blocks() const { return (int64_t)in_off.size() - 1; }
-    int32_t stream_of(int64_t b) const {
-        return (int32_t)(std::upper_bound(stream_blk.begin(), stream_blk.end(), b) - stream_blk.begin() - 1);
-    }
-};
 
 // Failure word of a block: (block << 32) | status << 24 | bytes written.  The smallest one is the first failing block.
 static __host__ __device__ uint64_t fail_word(int64_t b, uint32_t st, uint32_t n_out) {
     return (uint64_t)b << 32 | (uint64_t)st << 24 | (n_out & 0xffffffu);
 }
 
-static int report_failure(const hgt_bgzf *z, uint64_t w) {
+int bgzf_report_failure(const hgt_bgzf *z, uint64_t w) {
     const int64_t b = (int64_t)(w >> 32);
     const uint32_t st = (uint32_t)(w >> 24) & 0xff, n_out = (uint32_t)w & 0xffffff;
     const int32_t s = z->stream_of(b);
@@ -226,6 +212,41 @@ __global__ void __launch_bounds__(WARPS * 32) bgzf_inflate_kernel(const uint8_t 
     if (st != hgtz::OK && lane == 0) atomicMin(fail, (unsigned long long)fail_word(b, st, n_out));
 }
 
+BgzfLayout bgzf_layout(const hgt_bgzf *z) {
+    BgzfLayout L;
+    const size_t in_bytes = z->stream_in.back(), out_bytes = z->stream_out.back();
+    L.desc_bytes = 2 * (size_t)(z->n_blocks() + 1) * sizeof(uint64_t);
+    L.o_out = (in_bytes + 15) & ~(size_t)15;
+    L.o_desc = (L.o_out + out_bytes + 15) & ~(size_t)15;
+    L.o_fail = L.o_desc + L.desc_bytes;
+    L.bytes = L.o_fail + 8;
+    return L;
+}
+
+int bgzf_launch(hgt_ctx *ctx, const hgt_bgzf *z, const BgzfLayout &L, uint8_t *d, const uint8_t *h_desc) {
+    cudaStream_t st = ctx->stream;
+    const int64_t nb = z->n_blocks();
+    for (int32_t s = 0; s < z->n_streams; s++)
+        if (z->n_bytes[s])
+            HGT_CUDA(cudaMemcpyAsync(d + z->stream_in[s], z->data[s], z->n_bytes[s], cudaMemcpyHostToDevice, st));
+    HGT_CUDA(cudaMemcpyAsync(d + L.o_desc, h_desc, L.desc_bytes, cudaMemcpyHostToDevice, st));
+    HGT_CUDA(cudaMemsetAsync(d + L.o_fail, 0xff, 8, st));
+    ctx->h2d_bytes += (int64_t)(z->stream_in.back() + L.desc_bytes);
+    if (nb == 0) return HGT_OK;
+    const uint64_t *d_in_off = reinterpret_cast<const uint64_t *>(d + L.o_desc);
+    bgzf_inflate_kernel<<<(unsigned)((nb + WARPS - 1) / WARPS), WARPS * 32, 0, st>>>(
+        d, d_in_off, d_in_off + nb + 1, nb, d + L.o_out, reinterpret_cast<unsigned long long *>(d + L.o_fail));
+    HGT_CUDA(cudaGetLastError());
+    ctx->launches++;
+    return HGT_OK;
+}
+
+void bgzf_descriptors(const hgt_bgzf *z, uint8_t *h) {
+    const int64_t nb = z->n_blocks();
+    memcpy(h, z->in_off.data(), (nb + 1) * sizeof(uint64_t));
+    memcpy(h + (nb + 1) * sizeof(uint64_t), z->out_off.data(), (nb + 1) * sizeof(uint64_t));
+}
+
 extern "C" int hgt_bgzf_inflate(hgt_ctx *ctx, const hgt_bgzf *z, void *const *dst) {
     if (!ctx || !z || (z->n_streams > 0 && !dst)) {
         hgt_set_error("hgt_bgzf_inflate: bad arguments");
@@ -240,41 +261,27 @@ extern "C" int hgt_bgzf_inflate(hgt_ctx *ctx, const hgt_bgzf *z, void *const *ds
     if (nb == 0) return HGT_OK;
     HGT_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const size_t in_bytes = z->stream_in.back(), out_bytes = z->stream_out.back();
-    const size_t desc_bytes = 2 * (size_t)(nb + 1) * sizeof(uint64_t);
     // device: input | output | descriptors | failure word; page-locked: descriptors | failure word
-    const size_t o_out = (in_bytes + 15) & ~(size_t)15, o_desc = (o_out + out_bytes + 15) & ~(size_t)15,
-                 o_fail = o_desc + desc_bytes, dev_bytes = o_fail + 8;
+    const BgzfLayout L = bgzf_layout(z);
     void *dev = nullptr, *pin = nullptr;
     size_t dev_cap = 0, pin_cap = 0;
-    HGT_CHECK(ctx->pool.get(false, dev_bytes, &dev, &dev_cap));
-    int rc = ctx->pool.get(true, desc_bytes + 8, &pin, &pin_cap);
+    HGT_CHECK(ctx->pool.get(false, L.bytes, &dev, &dev_cap));
+    int rc = ctx->pool.get(true, L.desc_bytes + 8, &pin, &pin_cap);
     if (rc != HGT_OK) {
         ctx->pool.put(false, dev, dev_cap);
         return rc;
     }
     uint8_t *d = static_cast<uint8_t *>(dev), *h = static_cast<uint8_t *>(pin);
-    memcpy(h, z->in_off.data(), (nb + 1) * sizeof(uint64_t));
-    memcpy(h + (nb + 1) * sizeof(uint64_t), z->out_off.data(), (nb + 1) * sizeof(uint64_t));
-    uint64_t *h_fail = reinterpret_cast<uint64_t *>(h + desc_bytes);
+    bgzf_descriptors(z, h);
+    uint64_t *h_fail = reinterpret_cast<uint64_t *>(h + L.desc_bytes);
     auto run = [&]() -> int {
-        for (int32_t s = 0; s < z->n_streams; s++)
-            if (z->n_bytes[s])
-                HGT_CUDA(cudaMemcpyAsync(d + z->stream_in[s], z->data[s], z->n_bytes[s], cudaMemcpyHostToDevice, st));
-        HGT_CUDA(cudaMemcpyAsync(d + o_desc, h, desc_bytes, cudaMemcpyHostToDevice, st));
-        HGT_CUDA(cudaMemsetAsync(d + o_fail, 0xff, 8, st));
-        ctx->h2d_bytes += (int64_t)(in_bytes + desc_bytes);
-        const uint64_t *d_in_off = reinterpret_cast<const uint64_t *>(d + o_desc);
-        bgzf_inflate_kernel<<<(unsigned)((nb + WARPS - 1) / WARPS), WARPS * 32, 0, st>>>(
-            d, d_in_off, d_in_off + nb + 1, nb, d + o_out, reinterpret_cast<unsigned long long *>(d + o_fail));
-        HGT_CUDA(cudaGetLastError());
-        ctx->launches++;
+        HGT_CHECK(bgzf_launch(ctx, z, L, d, h));
         for (int32_t s = 0; s < z->n_streams; s++) {
             const size_t n = z->stream_out[s + 1] - z->stream_out[s];
-            if (n) HGT_CUDA(cudaMemcpyAsync(dst[s], d + o_out + z->stream_out[s], n, cudaMemcpyDeviceToHost, st));
+            if (n) HGT_CUDA(cudaMemcpyAsync(dst[s], d + L.o_out + z->stream_out[s], n, cudaMemcpyDeviceToHost, st));
         }
-        HGT_CUDA(cudaMemcpyAsync(h_fail, d + o_fail, 8, cudaMemcpyDeviceToHost, st));
-        ctx->d2h_bytes += (int64_t)(out_bytes + 8);
+        HGT_CUDA(cudaMemcpyAsync(h_fail, d + L.o_fail, 8, cudaMemcpyDeviceToHost, st));
+        ctx->d2h_bytes += (int64_t)(z->stream_out.back() + 8);
         HGT_CUDA(cudaStreamSynchronize(st));
         return HGT_OK;
     };
@@ -283,7 +290,7 @@ extern "C" int hgt_bgzf_inflate(hgt_ctx *ctx, const hgt_bgzf *z, void *const *ds
     ctx->pool.put(false, dev, dev_cap);
     ctx->pool.put(true, pin, pin_cap);
     if (rc != HGT_OK) return rc;
-    return w == ~0ull ? HGT_OK : report_failure(z, w);
+    return w == ~0ull ? HGT_OK : bgzf_report_failure(z, w);
 }
 
 // ---- host emulation -------------------------------------------------------------------------------------------------
@@ -338,5 +345,5 @@ extern "C" int hgt_bgzf_inflate_host(const hgt_bgzf *z, int32_t n_threads, void 
     worker();
     for (auto &t : pool) t.join();
     const uint64_t w = fail.load();
-    return w == ~0ull ? HGT_OK : report_failure(z, w);
+    return w == ~0ull ? HGT_OK : bgzf_report_failure(z, w);
 }

@@ -49,6 +49,11 @@ void hgt_set_error(const char *fmt, ...);
 // the stream has passed this point (the rule of cudaMemcpyAsync).
 cudaError_t hgt_small_h2d(void *dst_dev, const void *src_pinned, size_t bytes, cudaStream_t st);
 
+// Exclusive scan of n int64 values into out[0..n] (out[n] = total; in == out allowed) on stream st, three launches.
+// partial: device scratch of hgt_dev_scan_partials(n) int64 values.
+int64_t hgt_dev_scan_partials(int64_t n);
+int hgt_dev_scan(hgt_ctx *ctx, cudaStream_t st, const int64_t *in, int64_t n, int64_t *out, int64_t *partial);
+
 // Raises the dynamic shared-memory limit of `kernel` on the current device to at least `bytes`; never lowers it.  The
 // limit is a property of the kernel for the whole process, and batches on other host threads (one context each,
 // typing_core.BatchPipeline) launch the same kernels with their own sizes: a thread that set the exact size of its own

@@ -36,6 +36,8 @@
 #include "walk_dev.cuh"
 #include "reads.cuh"
 #include "bam_dev.cuh"
+#include "bam_dsplit.h"
+#include "bam_kernels.cuh"
 
 using namespace hgt;
 
@@ -1485,6 +1487,8 @@ struct UnitHost {
     size_t n_bytes = 0;             // text bytes (a BAM unit: its rendered text, known after the length pass of prepare)
     const void *blob = nullptr;     // BAM unit: packed records (bam_dev.cuh), rendered into the arena by prepare
     size_t blob_bytes = 0;
+    const hgt_bam_dsplit *ds = nullptr;  // device-split unit: a bucket in HBM (n_bytes known), rendered by prepare
+    hgtk::DsplitUnitDev dsu{};
     int64_t n_records = 0;
     int local = 0;  // index inside its locus batch
     int arena = 0;  // index in arena order (loci-major, add order inside a locus)
@@ -1506,6 +1510,8 @@ struct ReadsDev {
     PinBuf h_units, h_small, h_stage, h_loci, h_jobs_desc;
     DevBuf d_blob, d_blen, d_bunits;  // BAM units: blob arena, per-record text offsets, unit descriptors (prepare only)
     PinBuf h_bstage, h_bunits;
+    DevBuf d_dunits;  // device-split units: descriptors (prepare only)
+    PinBuf h_dunits;
     size_t o_uoff = 0, o_uline0 = 0, o_upos0 = 0, o_ulocus = 0, o_ulocal = 0, o_lu0 = 0, units_bytes = 0;
     size_t s_reads = 0, s_pairs = 0, s_totals = 0, small_bytes = 0;  // offsets inside the small result block
     void release() {
@@ -1517,8 +1523,8 @@ struct ReadsDev {
         release_bam();
     }
     void release_bam() {
-        d_blob.release(); d_blen.release(); d_bunits.release();
-        h_bstage.release(); h_bunits.release();
+        d_blob.release(); d_blen.release(); d_bunits.release(); d_dunits.release();
+        h_bstage.release(); h_bunits.release(); h_dunits.release();
     }
 };
 
@@ -1662,20 +1668,25 @@ static int tune_env(const char *name, int dflt) {  // grid-size experiments with
     return v > 0 ? v : dflt;
 }
 
-// exclusive scan of n int64 values into out[0..n] (out[n] = total); in == out allowed
-static int dev_scan(hgt_ctx *ctx, cudaStream_t st, const int64_t *in, int64_t n, int64_t *out, DevBuf *partial) {
+int64_t hgt_dev_scan_partials(int64_t n) { return (n + hgtk::SCAN_TILE - 1) / hgtk::SCAN_TILE + 1; }
+
+int hgt_dev_scan(hgt_ctx *ctx, cudaStream_t st, const int64_t *in, int64_t n, int64_t *out, int64_t *partial) {
     if (n <= 0) {
         HGT_CUDA(cudaMemsetAsync(out, 0, 8, st));
         return HGT_OK;
     }
     const int64_t n_part = (n + hgtk::SCAN_TILE - 1) / hgtk::SCAN_TILE;
-    HGT_CHECK(partial->alloc((size_t)(n_part + 1) * 8));
-    hgtk::scan_partials_kernel<<<(unsigned)n_part, hgtk::SCAN_THREADS, 0, st>>>(in, n, partial->as<int64_t>());
-    hgtk::scan_single_kernel<<<1, 1024, 0, st>>>(partial->as<int64_t>(), n_part);
-    hgtk::scan_apply_kernel<<<(unsigned)n_part, hgtk::SCAN_THREADS, 0, st>>>(in, n, partial->as<int64_t>(), n_part, out);
+    hgtk::scan_partials_kernel<<<(unsigned)n_part, hgtk::SCAN_THREADS, 0, st>>>(in, n, partial);
+    hgtk::scan_single_kernel<<<1, 1024, 0, st>>>(partial, n_part);
+    hgtk::scan_apply_kernel<<<(unsigned)n_part, hgtk::SCAN_THREADS, 0, st>>>(in, n, partial, n_part, out);
     ctx->launches += 3;
     HGT_CUDA(cudaGetLastError());
     return HGT_OK;
+}
+
+static int dev_scan(hgt_ctx *ctx, cudaStream_t st, const int64_t *in, int64_t n, int64_t *out, DevBuf *partial) {
+    if (n > 0) HGT_CHECK(partial->alloc((size_t)hgt_dev_scan_partials(n) * 8));
+    return hgt_dev_scan(ctx, st, in, n, out, partial->as<int64_t>());
 }
 
 static bool is_pinned_host(const void *p) {
@@ -1687,104 +1698,14 @@ static bool is_pinned_host(const void *p) {
     return at.type == cudaMemoryTypeHost;
 }
 
-// ---- BAM units: packed records (bam_dev.cuh) -> text in the arena ---------------------------------------------------------
+
 namespace hgtk {
-
-constexpr int BAM_THREADS = 256;
-
-struct BamUnitDev {  // one BAM unit of a batch: blob in the blob arena, first record (batch-wide), slice of the text arena
-    int64_t blob_off, rec0, text_off, pad;
-};
-
-// unit of batch-wide record g: the last unit whose first record is <= g (units without records are skipped that way)
-__device__ __forceinline__ int bam_unit_of(const BamUnitDev *__restrict__ u, int nb, int64_t g) {
-    int lo = 0, hi = nb - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (u[mid].rec0 <= g) lo = mid;
-        else hi = mid - 1;
-    }
-    return lo;
-}
-
-__device__ __forceinline__ void bam_view(const unsigned char *__restrict__ blobs, const BamUnitDev &U, int64_t i, hgtb::BamRec *r,
-                                         hgtb::BamNames *nm) {
-    using namespace hgtb;
-    const unsigned char *blob = blobs + U.blob_off;
-    const BamUnitHeader h = *reinterpret_cast<const BamUnitHeader *>(blob);
-    nm->off = reinterpret_cast<const uint32_t *>(blob + unit_name_off_at());
-    nm->bytes = blob + unit_names_at(h.n_names);
-    nm->n = h.n_names;
-    const uint64_t *ro = reinterpret_cast<const uint64_t *>(blob + unit_rec_off_at(h.n_names, h.names_bytes));
-    const uint64_t a = ro[i], e = ro[i + 1];
-    bam_decode(blob + a, e - a, (h.flags & UNIT_DROP_QUAL) != 0, r);
-}
-
-// text length of every record (one thread per record)
-__global__ void __launch_bounds__(BAM_THREADS) bam_text_len_kernel(const unsigned char *__restrict__ blobs,
-                                                                   const BamUnitDev *__restrict__ u, int nb, int64_t n_rec,
-                                                                   int64_t *__restrict__ len) {
-    const int64_t g = (int64_t)blockIdx.x * BAM_THREADS + threadIdx.x;
-    if (g >= n_rec) return;
-    const int k = bam_unit_of(u, nb, g);
-    hgtb::BamRec r;
-    hgtb::BamNames nm;
-    bam_view(blobs, u[k], g - u[k].rec0, &r, &nm);
-    len[g] = hgtb::bam_line_len(r, nm);
-}
-
 // text offset of every unit's first record (k = 0 .. nb; u[nb].rec0 = n_rec): the per-unit sizes the host lays out with
 __global__ void bam_unit_text_kernel(const int64_t *__restrict__ off, const BamUnitDev *__restrict__ u, int nb,
                                      int64_t *__restrict__ out) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k <= nb) out[k] = off[u[k].rec0];
 }
-
-// one warp per record: QNAME, SEQ and QUAL lane-parallel, the other columns and the tags by lane 0 (bam_dev.cuh)
-__global__ void __launch_bounds__(BAM_THREADS) bam_render_kernel(const unsigned char *__restrict__ blobs,
-                                                                 const BamUnitDev *__restrict__ u, int nb, int64_t n_rec,
-                                                                 const int64_t *__restrict__ off, char *__restrict__ text) {
-    const int64_t g = ((int64_t)blockIdx.x * BAM_THREADS + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (g >= n_rec) return;
-    const int k = bam_unit_of(u, nb, g);
-    hgtb::BamRec r;
-    hgtb::BamNames nm;
-    bam_view(blobs, u[k], g - u[k].rec0, &r, &nm);
-    char *dst = text + u[k].text_off + (off[g] - off[u[k].rec0]);
-    const uint32_t qn = hgtb::qname_len(r);
-    for (uint32_t i = lane; i < qn; i += 32) dst[i] = (char)r.p[hgtb::REC_FIXED + i];
-    dst += qn;
-    int64_t hl = 0;
-    if (lane == 0) {
-        hgtb::WriteSink w{dst};
-        hgtb::bam_head(r, nm, w);
-        hl = w.o - dst;
-    }
-    dst += __shfl_sync(0xffffffffu, hl, 0);
-    if (r.l_seq == 0) {
-        if (lane == 0) dst[0] = '*';
-        dst += 1;
-    } else {
-        for (uint32_t i = lane; i < r.l_seq; i += 32) dst[i] = hgtb::seq_base(r, i);
-        dst += r.l_seq;
-    }
-    if (lane == 0) dst[0] = '\t';
-    dst += 1;
-    if (!r.has_qual) {
-        if (lane == 0) dst[0] = '*';
-        dst += 1;
-    } else {
-        for (uint32_t i = lane; i < r.l_seq; i += 32) dst[i] = (char)(r.p[r.o_qual + i] + 33);
-        dst += r.l_seq;
-    }
-    if (lane == 0) {
-        hgtb::WriteSink w{dst};
-        hgtb::bam_tags(r, w);
-        *w.o = '\n';
-    }
-}
-
 }  // namespace hgtk
 
 // Length pass of the BAM units (prepare, only when the batch holds one): blobs to the device, text length per record,
@@ -1833,7 +1754,7 @@ static int bam_units_measure(hgt_batch *b, std::vector<int> &bam_arena, int64_t 
     HGT_CHECK(rd.d_blen.alloc((size_t)(R + 1) * 8));
     if (R > 0) {
         hgtk::bam_text_len_kernel<<<(unsigned)((R + hgtk::BAM_THREADS - 1) / hgtk::BAM_THREADS), hgtk::BAM_THREADS, 0, st>>>(
-            db, rd.d_bunits.as<hgtk::BamUnitDev>(), nb, R, rd.d_blen.as<int64_t>());
+            hgtk::BlobSrc{db, rd.d_bunits.as<hgtk::BamUnitDev>(), nb, nullptr}, R, rd.d_blen.as<int64_t>());
         ctx->launches++;
         HGT_CUDA(cudaGetLastError());
     }
@@ -1862,9 +1783,10 @@ static int bam_units_fill(hgt_batch *b, const std::vector<int> &bam_arena, int64
     std::vector<size_t> stage_off(nu + 1, 0);
     for (size_t a = 0; a < nu; a++) {
         const UnitHost &U = b->units[rd.unit_of_arena[a]];
-        const bool staged = !U.blob && U.n_bytes && !is_pinned_host(U.sam);
+        const bool text = !U.blob && !U.ds && U.n_bytes;
+        const bool staged = text && !is_pinned_host(U.sam);
         stage_off[a + 1] = stage_off[a] + (staged ? a16(U.n_bytes) : 0);
-        if (!U.blob && U.n_bytes && !staged) {
+        if (text && !staged) {
             HGT_CUDA(cudaMemcpyAsync(dt + rd.unit_off[a], U.sam, U.n_bytes, cudaMemcpyHostToDevice, st));
             ctx->h2d_bytes += (int64_t)U.n_bytes;
         }
@@ -1893,7 +1815,40 @@ static int bam_units_fill(hgt_batch *b, const std::vector<int> &bam_arena, int64
     ctx->h2d_bytes += (int64_t)desc;
     const int64_t warps_per_cta = hgtk::BAM_THREADS / 32;
     hgtk::bam_render_kernel<<<(unsigned)((R + warps_per_cta - 1) / warps_per_cta), hgtk::BAM_THREADS, 0, st>>>(
-        rd.d_blob.as<unsigned char>(), rd.d_bunits.as<hgtk::BamUnitDev>(), nb, R, rd.d_blen.as<int64_t>(), dt);
+        hgtk::BlobSrc{rd.d_blob.as<unsigned char>(), rd.d_bunits.as<hgtk::BamUnitDev>(), nb, rd.d_blen.as<int64_t>()}, R, dt);
+    ctx->launches++;
+    HGT_CUDA(cudaGetLastError());
+    return HGT_OK;
+}
+
+// Device-split units: every bucket rendered into its arena slice straight from the split's device memory (one launch; the
+// sizes were known when the units were added, so there is no length pass and no synchronisation).
+static int dsplit_units_render(hgt_batch *b) {
+    hgt_ctx *ctx = b->ctx;
+    cudaStream_t st = ctx->stream;
+    ReadsDev &rd = b->rd;
+    std::vector<hgtk::DsplitUnitDev> du;
+    int64_t R = 0;
+    for (size_t a = 0; a < b->units.size(); a++) {
+        const UnitHost &U = b->units[rd.unit_of_arena[a]];
+        if (!U.ds) continue;
+        hgtk::DsplitUnitDev d = U.dsu;
+        d.rec0 = R;
+        d.text_off = rd.unit_off[a];
+        du.push_back(d);
+        R += U.n_records;
+    }
+    if (R == 0) return HGT_OK;
+    const int nd = (int)du.size();
+    const size_t bytes = du.size() * sizeof(hgtk::DsplitUnitDev);
+    HGT_CHECK(rd.h_dunits.alloc(bytes));
+    HGT_CHECK(rd.d_dunits.alloc(bytes));
+    memcpy(rd.h_dunits.p, du.data(), bytes);
+    HGT_CUDA(cudaMemcpyAsync(rd.d_dunits.p, rd.h_dunits.p, bytes, cudaMemcpyHostToDevice, st));
+    ctx->h2d_bytes += (int64_t)bytes;
+    const int64_t warps_per_cta = hgtk::BAM_THREADS / 32;
+    hgtk::bam_render_kernel<<<(unsigned)((R + warps_per_cta - 1) / warps_per_cta), hgtk::BAM_THREADS, 0, st>>>(
+        hgtk::DsplitSrc{rd.d_dunits.as<hgtk::DsplitUnitDev>(), nd}, R, rd.d_text.as<char>());
     ctx->launches++;
     HGT_CUDA(cudaGetLastError());
     return HGT_OK;
@@ -1950,15 +1905,17 @@ static int batch_prepare(hgt_batch *b) {
         HGT_CHECK(rd.d_text.alloc((size_t)rd.text_bytes));
         char *dt = rd.d_text.as<char>();
         bool all_pinned = true;
-        for (const UnitHost &U : b->units) all_pinned &= U.blob || U.n_bytes == 0 || is_pinned_host(U.sam);
+        for (const UnitHost &U : b->units) all_pinned &= U.blob || U.ds || U.n_bytes == 0 || is_pinned_host(U.sam);
         if (!bam_arena.empty()) {  // text units copied, BAM units rendered (h2d_bytes: the bytes actually copied)
             HGT_CHECK(bam_units_fill(b, bam_arena, n_bam_rec));
         } else if (all_pinned) {  // page-locked input: the DMA engine reads the caller's buffers directly
             ctx->h2d_bytes += rd.text_bytes;
+            for (size_t a = 0; a < nu; a++)  // device-split units are rendered, not copied
+                if (b->units[rd.unit_of_arena[a]].ds) ctx->h2d_bytes -= rd.unit_off[a + 1] - rd.unit_off[a];
             HGT_CUDA(cudaMemsetAsync(dt, '\n', (size_t)rd.text_bytes, st));
             for (size_t a = 0; a < nu; a++) {
                 const UnitHost &U = b->units[rd.unit_of_arena[a]];
-                if (U.n_bytes) HGT_CUDA(cudaMemcpyAsync(dt + rd.unit_off[a], U.sam, U.n_bytes, cudaMemcpyHostToDevice, st));
+                if (U.n_bytes && !U.ds) HGT_CUDA(cudaMemcpyAsync(dt + rd.unit_off[a], U.sam, U.n_bytes, cudaMemcpyHostToDevice, st));
             }
         } else {  // pageable input: host threads assemble the arena image in page-locked memory, one copy
             ctx->h2d_bytes += rd.text_bytes;
@@ -1966,11 +1923,13 @@ static int batch_prepare(hgt_batch *b) {
             char *hs = rd.h_stage.as<char>();
             parallel_units(batch_threads(b->params), nu, [&](size_t a) {
                 const UnitHost &U = b->units[rd.unit_of_arena[a]];
-                if (U.n_bytes) memcpy(hs + rd.unit_off[a], U.sam, U.n_bytes);
-                memset(hs + rd.unit_off[a] + U.n_bytes, '\n', (size_t)(rd.unit_off[a + 1] - rd.unit_off[a]) - U.n_bytes);
+                const size_t n = U.ds ? 0 : U.n_bytes;  // a device-split unit is rendered over its slice below
+                if (n) memcpy(hs + rd.unit_off[a], U.sam, n);
+                memset(hs + rd.unit_off[a] + n, '\n', (size_t)(rd.unit_off[a + 1] - rd.unit_off[a]) - n);
             });
             HGT_CUDA(cudaMemcpyAsync(dt, hs, (size_t)rd.text_bytes, cudaMemcpyHostToDevice, st));
         }
+        HGT_CHECK(dsplit_units_render(b));
     }
     {
         HostTimer ht(ctx, 1);
@@ -2919,6 +2878,28 @@ extern "C" int64_t hgt_batch_add_unit_bam(hgt_batch *b, int32_t locus_index, con
     u.blob = blob;
     u.blob_bytes = n_bytes;
     u.n_records = h.n_records;
+    b->units.push_back(std::move(u));
+    return (int64_t)b->units.size() - 1;
+}
+
+extern "C" int64_t hgt_batch_add_unit_bam_dsplit(hgt_batch *b, int32_t locus_index, const hgt_bam_dsplit *s, int32_t stream,
+                                                 int32_t ref) {
+    if (!b || locus_index < 0 || locus_index >= (int)b->loci.size() || b->prepared || !s) {
+        hgt_set_error("hgt_batch_add_unit_bam_dsplit: bad argument");
+        return HGT_ERR_ARG;
+    }
+    UnitHost u;
+    int device = -1;
+    if (bam_dsplit_unit(s, stream, ref, &u.dsu, &u.n_records, &u.n_bytes, &device) != HGT_OK) {
+        hgt_set_error("hgt_batch_add_unit_bam_dsplit: stream %d / reference %d outside the split", stream, ref);
+        return HGT_ERR_ARG;
+    }
+    if (device != b->ctx->device) {
+        hgt_set_error("hgt_batch_add_unit_bam_dsplit: the split is on device %d, the batch on device %d", device, b->ctx->device);
+        return HGT_ERR_ARG;
+    }
+    u.locus = locus_index;
+    u.ds = s;
     b->units.push_back(std::move(u));
     return (int64_t)b->units.size() - 1;
 }

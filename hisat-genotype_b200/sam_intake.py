@@ -224,6 +224,105 @@ def split_bam(bam_bytes, ref_names, n_threads=0, pinned=None, drop_qual=False, t
         L.hgt_bam_split_free(h)
 
 
+class DeviceBamUnit:
+    """Bucket `ref` of stream `stream` of a DeviceBamSplit: what Batch.add_unit_bam_dsplit / typing_from_alignments take in
+    place of alignment text.  Its records stay in device memory; prepare() renders them there."""
+
+    def __init__(self, split, stream, ref):
+        self.split, self.stream, self.ref = split, stream, ref
+
+
+class DeviceBamSplit:
+    """The device split of BGZF-compressed BAM files (hgt_bam_dsplit_*): for every (file, backbone) the records of that
+    bucket, in split_bam's order, resident in HBM.  A context manager; close() frees the device memory, after every batch
+    that uses a unit of it is prepared."""
+
+    def __init__(self, handle, n_streams, ref_names):
+        self.handle, self.n_streams, self.ref_names = handle, n_streams, list(ref_names)
+
+    def sizes(self):
+        """(records, text_bytes): numpy int64 arrays [n_streams][n_refs]."""
+        n = self.n_streams * len(self.ref_names)
+        rec = np.zeros(n, np.int64)
+        txt = np.zeros(n, np.uint64)
+        _lib.check(_lib.lib().hgt_bam_dsplit_sizes(self.handle, rec.ctypes.data, txt.ctypes.data))
+        shape = (self.n_streams, len(self.ref_names))
+        return rec.reshape(shape), txt.astype(np.int64).reshape(shape)
+
+    def unit(self, stream, ref):
+        """ref: a backbone name or its index."""
+        r = self.ref_names.index(ref) if isinstance(ref, str) else int(ref)
+        assert 0 <= stream < self.n_streams and 0 <= r < len(self.ref_names)
+        return DeviceBamUnit(self, int(stream), r)
+
+    def close(self):
+        if self.handle:
+            _lib.lib().hgt_bam_dsplit_free(self.handle)
+            self.handle = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        self.close()
+
+
+def split_bam_device(files, ref_names, device=None, drop_qual=False):
+    """BGZF-compressed BAM files (a list of buffers) split by backbone on the GPU in one call: inflate, record index,
+    complete check of every record, bucketing and name order on the device (hgt_bam_dsplit_create); only the compressed
+    bytes and small tables cross PCIe.  Returns a DeviceBamSplit whose unit(stream, ref) renders into what
+    split_bam(files[stream], ref_names, text=True)[ref] holds.  A missing EOF block warns as read_bgzf does; malformed
+    input raises AssertionError, float tags and the CG long-CIGAR tag raise HgtError (HGT_ERR_UNSUPPORTED), each
+    naming the stream."""
+    L = _lib.lib()
+    ctx = _lib.ctx(device)
+    arrs = [np.frombuffer(f, np.uint8) for f in files]
+    n = len(arrs)
+    ptrs = (ctypes.c_void_p * max(n, 1))(*[a.ctypes.data if a.size else None for a in arrs])
+    sizes = (ctypes.c_size_t * max(n, 1))(*[a.size for a in arrs])
+    z = ctypes.c_void_p()
+    rc = L.hgt_bgzf_open(n, ptrs, sizes, ctypes.byref(z))
+    if rc == _lib.HGT_ERR_PARSE:
+        raise AssertionError(_lib.last_error())
+    _lib.check(rc)
+    try:
+        eof = (ctypes.c_int32 * max(n, 1))()
+        _lib.check(L.hgt_bgzf_sizes(z, None, None, eof))
+        for i in range(n):
+            if not eof[i]:
+                import warnings
+                warnings.warn("BGZF input has no EOF marker block; it may be truncated")
+        enc = [r.encode() for r in ref_names]
+        arr = (ctypes.c_char_p * len(enc))(*enc)
+        h = ctypes.c_void_p()
+        rc = L.hgt_bam_dsplit_create(ctx, z, len(enc), arr, 1 if drop_qual else 0, ctypes.byref(h))
+        if rc == _lib.HGT_ERR_PARSE:
+            raise AssertionError(_lib.last_error())
+        _lib.check(rc)
+        return DeviceBamSplit(h, n, ref_names)
+    finally:
+        L.hgt_bgzf_free(z)
+
+
+def bam_index_host(bam_stream, chunk_bytes, n_threads=0):
+    """The host emulation of the device split's record index (hgt_bam_index_host) over one decompressed BAM stream:
+    numpy uint64 offsets of every record.  A broken block_size chain raises AssertionError.  Test infrastructure."""
+    L = _lib.lib()
+    a = np.frombuffer(bam_stream, np.uint8)
+    cap = a.size // 36 + 1
+    out = np.zeros(cap, np.uint64)
+    n = ctypes.c_int64(0)
+    rc = L.hgt_bam_index_host(a.ctypes.data if a.size else None, a.size, int(chunk_bytes), int(n_threads), cap,
+                              out.ctypes.data, ctypes.byref(n))
+    if rc == _lib.HGT_ERR_PARSE:
+        raise AssertionError(_lib.last_error())
+    _lib.check(rc)
+    return out[:n.value]
+
+
 def hisat2_command(simulation, index_name, base_fname, read_fname, fastq, threads):
     """The command line of the reference's align_reads() for aligner == "hisat2" on a graph index
     (hisatgenotype_typing_common.py:995-1024), without the samtools stages behind it."""

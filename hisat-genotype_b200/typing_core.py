@@ -215,6 +215,16 @@ class Batch:
         self.unit_locus.append(locus_index)
         return int(u)
 
+    def add_unit_bam_dsplit(self, locus_index, unit):
+        """A sam_intake.DeviceBamUnit: prepare() renders the bucket into alignment text straight from the split's device
+        memory.  The split must stay open until prepare() returns."""
+        u = lib().hgt_batch_add_unit_bam_dsplit(self.handle, locus_index, unit.split.handle, unit.stream, unit.ref)
+        if u < 0:
+            _lib.check(int(u))
+        self._texts.append(unit.split)  # kept alive until prepare()
+        self.unit_locus.append(locus_index)
+        return int(u)
+
     def unit_text(self, u):
         """After prepare(): the unit's alignment text as it sits in the device arena (rendered on the GPU for a BAM unit)."""
         n = ctypes.c_size_t(0)
@@ -604,10 +614,11 @@ def typing_from_alignments(base_fname, locus_tables, locus_list, alignments, sim
     locus_list    as typing() receives it: gene names, or in simulation mode the lists of truth alleles
                   (gene = names[0].split('*')[0], core:380-383)
     alignments    {gene: alignment lines in `samtools view <bam> <backbone> | sort -k1,1 -s` order (core:458-468), or a
-                  sam_intake.BamUnit of split_bam, rendered into those lines on the GPU}
+                  sam_intake.BamUnit of split_bam or a sam_intake.DeviceBamUnit of split_bam_device, rendered into those
+                  lines on the GPU}
     Returns (report body text starting at the aligner line, test_passed dict of the simulation mode)."""
     from . import report
-    from .sam_intake import BamUnit
+    from .sam_intake import BamUnit, DeviceBamUnit
     assert index_type == "graph", "the linear-index branch (core:1597-1648) stays on the reference path"
     genes, truths = [], []
     for entry in locus_list:
@@ -628,6 +639,8 @@ def typing_from_alignments(base_fname, locus_tables, locus_list, alignments, sim
         for g in genes:
             if isinstance(alignments[g], BamUnit):
                 batch.add_unit_bam(uniq.index(g), alignments[g])
+            elif isinstance(alignments[g], DeviceBamUnit):
+                batch.add_unit_bam_dsplit(uniq.index(g), alignments[g])
             else:
                 batch.add_unit(uniq.index(g), alignments[g])
         batch.run()

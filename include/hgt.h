@@ -438,6 +438,46 @@ int hgt_bgzf_inflate(hgt_ctx *ctx, const hgt_bgzf *z, void *const *dst);
 int hgt_bgzf_inflate_host(const hgt_bgzf *z, int32_t n_threads, void *const *dst);
 void hgt_bgzf_free(hgt_bgzf *z);
 
+/* ---- device split of BGZF-compressed BAM files -------------------------------------------------------------------
+ * The host split's work (hgt_bam_split_*) on the GPU, from the inflated streams kept in HBM: for every (stream, backbone)
+ * the records of that bucket, in the host split's order, resident in device memory; a batch unit renders one bucket into
+ * the text arena (hgt_batch_add_unit_bam_dsplit), byte for byte what hgt_bam_split_write_text gives for the same stream.
+ * The inflated bytes never come back to the host.
+ * create: z from hgt_bgzf_open (its header walk, sizes and messages are reused; has_eof is the caller's to check);
+ * ref_names: the backbones (the host split's rule for repeated names); flags: HGT_SPLIT_DROP_QUAL.  One call does the
+ * inflate, the header walk, the record index, the complete check of every record, the bucketing and ordering, and the text
+ * sizes on the device (csrc/bam_dsplit.cu).  Synchronisations: three, plus one when a stream's header is longer than the
+ * 64 KB read-back window, plus one when a record fails its check.
+ * Errors, in this precedence: a failing BGZF block (hgt_bgzf_inflate's message); else the lowest stream with an error,
+ * and within it the host split's order: header, block_size chain, first bad record.  The message is the host split's
+ * without its function name, after "stream <i>: ".  HGT_ERR_PARSE, or HGT_ERR_UNSUPPORTED for float tags and CG.  After
+ * an error the context and other handles stay usable.
+ * Limits: 1 .. 2^31 - 1 (streams x backbones) buckets, at most 2^31 - 1 records per call; read names are at most 254
+ * bytes (BAM's l_read_name).
+ * Counters (S streams, B blocks, R = n_refs, K = S x R, n_hdr(s) and names(s) = reference count and name bytes of the
+ * header of stream s, a8 = rounded up to 8):
+ *   h2d_bytes grows by the compressed bytes + 16 (B + 1) + 8 (S + 1) + 48 (S + 1) + sum over s of
+ *     a8(8 n_hdr(s) + 4 + names(s)) + 4 K;
+ *   d2h_bytes by 56 S + 16 (K + 2) + sum over s of min(inflated(s), 65536), plus the walked bytes of a header longer
+ *     than the window and, when a record fails, 312.
+ * The handle holds the inflated streams and lives on ctx's device; free it after every batch that uses it is prepared. */
+typedef struct hgt_bam_dsplit hgt_bam_dsplit;
+int hgt_bam_dsplit_create(hgt_ctx *ctx, const hgt_bgzf *z, int32_t n_refs, const char *const *ref_names, int32_t flags,
+                          hgt_bam_dsplit **out);
+/* records and text bytes of every bucket, [n_streams][n_refs] each; any pointer may be NULL */
+int hgt_bam_dsplit_sizes(const hgt_bam_dsplit *s, int64_t *records, size_t *text_bytes);
+void hgt_bam_dsplit_free(hgt_bam_dsplit *s);
+/* A unit whose text is bucket `ref` of stream `stream`, rendered by prepare from the handle's device memory (no copy, no
+ * length pass: the size is known).  s must live until prepare returns and belong to the batch's device. */
+int64_t hgt_batch_add_unit_bam_dsplit(hgt_batch *b, int32_t locus_index, const hgt_bam_dsplit *s, int32_t stream,
+                                      int32_t ref);
+/* Host EMULATION of the device split's record index (test infrastructure): the same chunk guess, walk, fix-up passes and
+ * resolve on host threads over one decompressed BAM stream, with chunks of chunk_bytes.  Writes the first `cap` record
+ * offsets (bytes of the stream) and *n_records; a broken block_size chain gives HGT_ERR_PARSE with the host split's
+ * message. */
+int hgt_bam_index_host(const void *bam, size_t n_bytes, int64_t chunk_bytes, int32_t n_threads, int64_t cap,
+                       uint64_t *offsets, int64_t *n_records);
+
 /* Host EMULATION of the record stage with a caller-supplied pileup (no GPU needed; test infrastructure, not on the
  * typing path): the same __host__ __device__ functions the kernels call (csrc/walk_dev.cuh: parse, filters, mate
  * de-dup, walk, error correction, ambiguity expansion, exon clipping, pair jobs) run in plain loops.  Output is the

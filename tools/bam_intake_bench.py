@@ -11,6 +11,9 @@ DRB1, paired-end 2x100 bp, 30x, the seeded synthetic database and reads of bench
     (bgzf_inflate_gpu_per_file_ms); the kernel alone from torch.profiler's device records (bgzf_inflate_kernel_ms); the
     compressed / inflated bytes and the call's h2d / d2h bytes; and split_bam fed from one-file inflate_bgzf calls
     (split_bam_gpu_inflate_ms, against split_bam_ms).
+  - the device split (sam_intake.split_bam_device: inflate, record index, checks, bucketing and order on the GPU) of the
+    step's files in one call from page-locked input, ending in its synchronisation (split_bam_device_ms), with the call's
+    h2d / d2h bytes; and a bam_device variant of prepare / execute + finish whose units render from that split's HBM.
 The calls of every variant must equal the text run's, and every file's GPU-inflated bytes read_bgzf's (exit status 1
 otherwise).  Prints one JSON line (GPU name and power limit included) and writes it to --out when given.
 
@@ -59,7 +62,7 @@ def main():
     from hisatgenotype_b200 import _lib, synth
     from hisatgenotype_b200 import typing_core as TC
     from hisatgenotype_b200.locus import LocusTables
-    from hisatgenotype_b200.sam_intake import inflate_bgzf, read_bgzf, split_bam, split_sam
+    from hisatgenotype_b200.sam_intake import inflate_bgzf, read_bgzf, split_bam, split_bam_device, split_sam
 
     threads = args.threads or os.cpu_count() or 1
     info = gpu_info()
@@ -99,8 +102,13 @@ def main():
         pinned[v] = (buf, [[(li,) + buf.add(p[r]) for li, r in enumerate(refs)] for p in parts])
 
     def one_batch(v):
-        kind = variants[v][0]
         b = TC.Batch(tables, params, True)
+        if v == "bam_device":
+            for s in range(args.samples):
+                for li in range(len(refs)):
+                    b.add_unit_bam_dsplit(li, dsplit.unit(s, li))
+            return b
+        kind = variants[v][0]
         for sample in pinned[v][1]:
             for li, addr, n in sample:
                 if kind == "sam":
@@ -194,14 +202,32 @@ def main():
     else:
         res["bgzf_inflate_kernel_ms"] = None  # the profiler recorded no kernel of that name
     res["inflate_identical"] = inflate_ok
+    # the device split: one call over the step's files, page-locked compressed input
+    def dsplit_call():
+        return split_bam_device(bams_pinned, refs)
+
+    L.hgt_profile_reset(ctx)
+    dsplit = dsplit_call()
+    L.hgt_profile_read(ctx, None, None, ctypes.byref(h2d), ctypes.byref(d2h))
+    res.update({"split_bam_device_h2d_bytes": h2d.value, "split_bam_device_d2h_bytes": d2h.value})
+    for _ in range(args.warmup):
+        dsplit_call().close()
+    ts = []
+    for _ in range(args.steps):
+        t = time.perf_counter()
+        sp = dsplit_call()
+        ts.append((time.perf_counter() - t) * 1e3)
+        sp.close()
+    res["split_bam_device_ms"] = {"mean": round(float(np.mean(ts)), 2), "min": round(float(np.min(ts)), 2)}
     fin.close()
     fout.close()
     # prepare / execute + finish per variant, the variants alternating inside every step
     ref_calls = None
     ok = True
-    acc = {v: {"prepare_ms": [], "execute_finish_ms": [], "h2d_bytes": [], "launches": 0} for v in variants}
+    run_variants = list(variants) + ["bam_device"]
+    acc = {v: {"prepare_ms": [], "execute_finish_ms": [], "h2d_bytes": [], "launches": 0} for v in run_variants}
     for step in range(args.warmup + args.steps):
-        for v in variants:
+        for v in run_variants:
             t_prep, t_exec, hb, calls, acc[v]["launches"] = run_step(v)
             if v == "text":
                 ref_calls = calls
@@ -212,7 +238,7 @@ def main():
                 acc[v]["execute_finish_ms"].append(t_exec * 1e3)
                 acc[v]["h2d_bytes"].append(hb)
     for v, a in acc.items():
-        res["variants"][v] = {"input_bytes": int(sum(n for s in pinned[v][1] for _, _, n in s)),
+        res["variants"][v] = {"input_bytes": int(sum(n for s in pinned[v][1] for _, _, n in s)) if v in pinned else 0,
                               "prepare_ms": {"mean": round(float(np.mean(a["prepare_ms"])), 2),
                                              "min": round(float(np.min(a["prepare_ms"])), 2)},
                               "execute_finish_ms": {"mean": round(float(np.mean(a["execute_finish_ms"])), 2),
@@ -224,6 +250,7 @@ def main():
     if args.out:
         with open(args.out, "w") as f:
             f.write(line + "\n")
+    dsplit.close()
     for buf, _ in pinned.values():
         buf.close()
     for t in tables:
