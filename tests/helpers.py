@@ -87,7 +87,7 @@ def tables_from_jobs(loc, walk, hla):
 
 
 def synthetic_case(seed, A, L=2500, n_pairs=1000, base="hla", del_frac=0.1, alphabet="ACGT", n_groups=12, core_vars=60,
-                   pool_private=300, err_rate=0.004, paired=True):
+                   pool_private=300, err_rate=0.004, paired=True, read_len=100, frag_len=350):
     """Database + reads from hisatgenotype_b200.synth (sizes the reference-captured goldens do not reach): returns
     (LocusTables/OracleLocus constructor args, alignment lines, truth alleles)."""
     from hisatgenotype_b200 import synth
@@ -101,7 +101,8 @@ def synthetic_case(seed, A, L=2500, n_pairs=1000, base="hla", del_frac=0.1, alph
     rng = np.random.default_rng(seed)
     names = sorted(n for n in loc.alleles if loc.alleles[n])
     truth = [names[i] for i in rng.choice(len(names), 2, replace=False)]
-    sam = synth.simulate_sam(loc, truth, n_pairs=n_pairs, rng=rng, err_rate=err_rate, paired=paired)
+    sam = synth.simulate_sam(loc, truth, n_pairs=n_pairs, rng=rng, err_rate=err_rate, paired=paired, read_len=read_len,
+                             frag_len=frag_len)
     return args, sam, truth
 
 
