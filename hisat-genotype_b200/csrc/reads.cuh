@@ -238,7 +238,6 @@ __device__ __forceinline__ const char *stage_lines(Stage &s, const ReadsView &R,
 }
 
 // ---- pileup (common:1100-1121) straight from the CIGAR text: warp per line, lanes over the bases of each M / D op ------------
-// one line of the pileup by one warp; `line` may point into the shared-memory image of the CTA's lines
 __device__ __forceinline__ void pileup_line(const ReadsView &R, int64_t r, const char *line, uint32_t *__restrict__ counts_all, int lane) {
     const RecFields f = R.rec[r];
     const char *cig = line + f.cig_off, *seq = line + f.seq_off;
@@ -278,7 +277,7 @@ __global__ void __launch_bounds__(256) pileup_text_kernel(ReadsView R, uint32_t 
         if (R.st[r] & ST_PU) pileup_line(R, r, R.text + R.line_off[r], counts_all, lane);
 }
 
-__global__ void __launch_bounds__(STAGE_LINES) parse_kernel(ReadsView R, WalkParams P, int smem_bytes, uint32_t *__restrict__ counts_all) {
+__global__ void __launch_bounds__(STAGE_LINES) parse_kernel(ReadsView R, WalkParams P, int smem_bytes) {
     extern __shared__ __align__(128) char s_text[];
     __shared__ uint64_t mbar;
     Stage sg;
@@ -289,14 +288,6 @@ __global__ void __launch_bounds__(STAGE_LINES) parse_kernel(ReadsView R, WalkPar
         const char *base = stage_lines(sg, R, i0, i1);
         const int64_t i = i0 + threadIdx.x;
         if (i < i1) parse_line(R, P, base, i);
-        if (counts_all) {
-            // pileup of the same lines while their image is in shared memory (one pass over the text less): warp per line;
-            // the record fields written by the CTA's other threads are visible after the barrier
-            __syncthreads();
-            const int lane = threadIdx.x & 31;
-            for (int64_t r = i0 + (threadIdx.x >> 5); r < i1; r += STAGE_LINES / 32)
-                if (R.st[r] & ST_PU) pileup_line(R, r, base + R.line_off[r], counts_all, lane);
-        }
     }
 }
 __global__ void __launch_bounds__(256) head_kernel(ReadsView R) {
@@ -446,20 +437,18 @@ __device__ __forceinline__ EcMask warp_ec_masks(const ReadsView &R, const WalkPa
     return mine;
 }
 
-__global__ void __launch_bounds__(STAGE_LINES) walk_kernel(ReadsView R, WalkParams P, int smem_bytes) {
-    extern __shared__ __align__(128) char s_text[];
-    __shared__ uint64_t mbar;
+// The walk reads its lines from the arena, not from a staged image like parse_kernel: with the ambiguity work split off
+// into two list passes, L1-cached global loads measured faster for it (DESIGN.md 7).  Compiled for 6 CTAs per SM
+// (80 registers): without the bound ptxas picks 72 registers and more spill loads, and the walk measured 1 % slower.
+__global__ void __launch_bounds__(STAGE_LINES, 6) walk_kernel(ReadsView R, WalkParams P) {
     __shared__ __align__(16) EcParams s_ecp[STAGE_LINES];
-    Stage sg;
-    stage_init(sg, &mbar, s_text, smem_bytes);
     const int64_t n_blk = (R.n_lines + STAGE_LINES - 1) / STAGE_LINES;
     for (int64_t blk = blockIdx.x; blk < n_blk; blk += gridDim.x) {
         const int64_t i0 = blk * STAGE_LINES, i1 = min(i0 + (int64_t)STAGE_LINES, R.n_lines);
-        const char *base = stage_lines(sg, R, i0, i1);
         const int64_t i = i0 + threadIdx.x;
         const bool cand = i < i1 && (R.st[i] & ST_CAND);
-        const EcMask M = warp_ec_masks(R, P, base, i, cand, s_ecp + (threadIdx.x & ~31));
-        if (cand) walk_record<0>(R, P, base, i, -1, M);
+        const EcMask M = warp_ec_masks(R, P, R.text, i, cand, s_ecp + (threadIdx.x & ~31));
+        if (cand) walk_record<0>(R, P, R.text, i, -1, M);
     }
 }
 // ---- list passes by position ---------------------------------------------------------------------------------------------------
@@ -524,24 +513,25 @@ __global__ void __launch_bounds__(256) list_scatter_kernel(ReadsView R, const in
     }
 }
 
-// second pass: records with an Alts anchor in reach (amb_list, filled by walk_kernel; its length stays on the device)
-__global__ void __launch_bounds__(128) walk_amb_kernel(ReadsView R, WalkParams P) {
+// second pass: records with an Alts anchor in reach (amb_list, filled by walk_kernel; its length stays on the device),
+// `list` = amb_list in backbone order
+__global__ void __launch_bounds__(128) walk_amb_kernel(ReadsView R, WalkParams P, const int32_t *__restrict__ list) {
     __shared__ __align__(16) EcParams s_ecp[128];
     const int n = *R.n_amb, n_round = (n + 31) & ~31;  // whole warps: the lanes compute the masks together
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_round; k += gridDim.x * blockDim.x) {
         const bool on = k < n;
-        const int64_t i = on ? (R.list_sorted ? R.list_sorted[k] : R.amb_list[k]) : 0;
+        const int64_t i = on ? list[k] : 0;
         const EcMask M = warp_ec_masks(R, P, R.text, i, on, s_ecp + (threadIdx.x & ~31));
         if (on) walk_record<1>(R, P, R.text, i, -1, M);
     }
 }
-// third pass: records with several haplotypes
-__global__ void __launch_bounds__(128) walk_slow_kernel(ReadsView R, WalkParams P, int n_slow) {
+// third pass: records with several haplotypes, `list` = slow_list in backbone order
+__global__ void __launch_bounds__(128) walk_slow_kernel(ReadsView R, WalkParams P, const int32_t *__restrict__ list, int n_slow) {
     __shared__ __align__(16) EcParams s_ecp[128];
     const int n_round = (n_slow + 31) & ~31;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_round; k += gridDim.x * blockDim.x) {
         const bool on = k < n_slow;
-        const int64_t i = on ? (R.list_sorted ? R.list_sorted[k] : R.slow_list[k]) : 0;
+        const int64_t i = on ? list[k] : 0;
         const EcMask M = warp_ec_masks(R, P, R.text, i, on, s_ecp + (threadIdx.x & ~31));
         if (on) walk_record<2>(R, P, R.text, i, k, M);
     }

@@ -583,8 +583,7 @@ __device__ __forceinline__ unsigned del_rows_left_of(const LocusDev &loc, int d0
     return __ballot_sync(0xffffffffu, q);
 }
 
-// Set algebra of one haplotype.  ROW(k) yields its k-th sorted variant row (k < k1): a pointer read in compat_kernel,
-// registers for the first two rows in job_class_kernel.
+// Set algebra of one haplotype.  ROW(k) yields its k-th sorted variant row (k < k1).
 template <int WPL, class RowFn>
 __device__ __forceinline__ void hap_allele_set_core(const LocusDev &loc, int left, const HapBounds &hb, RowFn ROW, int k1,
                                                     const uint64_t *__restrict__ mask, int lane, uint64_t (&set)[WPL]) {
@@ -647,7 +646,7 @@ __device__ __forceinline__ void hap_allele_set(const LocusDev &loc, int left, in
     hap_allele_set_core<WPL>(loc, left, hb, [rw](int k) { return rw[k]; }, k1, mask, lane, set);
 }
 
-// warp per haplotype -> hapbits (two-kernel form of stage (a), the default)
+// warp per haplotype -> hapbits (read by class_kernel)
 template <int WPL>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32)
     compat_kernel(LocusDev loc, const int32_t *__restrict__ hap_table, const int32_t *__restrict__ hap_left,
@@ -695,7 +694,7 @@ __device__ __forceinline__ uint64_t mix64(uint64_t x) {
     return x;
 }
 
-// Insert in two halves so that a caller can keep the first CAS in flight behind other work (job_class_kernel).
+// Insert in two halves: the CAS on the home slot, then the probe that resolves it (pool_insert runs both back to back).
 struct PoolProbe {
     unsigned long long tag, prev;  // prev: what lane 0's CAS found in the first slot
     uint32_t slot;
@@ -915,284 +914,6 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, (WPL <= 4 && P <= 3) ? 5 :
         }
         pool_insert<WPL>(pool, wp, ut, best, 1ull, job_pair[job], lane);
     }
-}
-
-// Fused stage (a): warp per job computes the allele set of each of the job's haplotypes in registers (hap_allele_set) and
-// feeds it straight into the bit-plane counter, so the sets never travel through HBM (add_count + add_stat in one pass).
-template <int WPL, int P>
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32)
-    pair_class_kernel(LocusDev loc, const int64_t *__restrict__ job_off, const int32_t *__restrict__ job_ut,
-                      const int32_t *__restrict__ job_pair, const int32_t *__restrict__ job_list, int64_t n_jobs,
-                      const int32_t *__restrict__ hap_left, const int32_t *__restrict__ hap_right,
-                      const int64_t *__restrict__ row_off, const int32_t *__restrict__ rows, ClassPool pool,
-                      const int32_t *__restrict__ n_jobs_dev) {
-    const int lane = threadIdx.x & 31;
-    const int wp = loc.wp;
-    const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    if (n_jobs_dev) n_jobs = min(n_jobs, (int64_t)*n_jobs_dev);  // list written by job_class_kernel
-    for (int64_t q = warp0; q < n_jobs; q += nwarps) {
-        const int job = job_list[q];
-        const int64_t h0 = job_off[job], h1 = job_off[job + 1];
-        const int ut = job_ut[job];
-        const uint64_t *mask = loc.mask + (size_t)(ut & 3) * wp + lane;
-        uint64_t plane[P][WPL], best[WPL];
-#pragma unroll
-        for (int p = 0; p < P; p++)
-#pragma unroll
-            for (int i = 0; i < WPL; i++) plane[p][i] = 0ull;
-        for (int64_t h = h0; h < h1; h++) {
-            uint64_t set[WPL];
-            hap_allele_set<WPL>(loc, hap_left[h], hap_right[h], rows + row_off[h], (int)(row_off[h + 1] - row_off[h]), mask,
-                                lane, set);
-#pragma unroll
-            for (int i = 0; i < WPL; i++) {
-                uint64_t carry = set[i];
-#pragma unroll
-                for (int p = 0; p < P; p++) {
-                    const uint64_t t = plane[p][i] & carry;
-                    plane[p][i] ^= carry;
-                    carry = t;
-                }
-            }
-        }
-#pragma unroll
-        for (int i = 0; i < WPL; i++) best[i] = lane + 32 * i < wp ? mask[32 * i] : 0ull;
-#pragma unroll
-        for (int p = P - 1; p >= 0; p--) {
-            uint64_t any = 0;
-#pragma unroll
-            for (int i = 0; i < WPL; i++) any |= best[i] & plane[p][i];
-            if (__any_sync(0xffffffffu, any != 0ull)) {
-#pragma unroll
-                for (int i = 0; i < WPL; i++) best[i] &= plane[p][i];
-            }
-        }
-        pool_insert<WPL>(pool, wp, ut, best, 1ull, job_pair[job], lane);
-    }
-}
-
-// Stage (a) in ONE pass for the common job - zero, one or two haplotypes per (pair, table); on a 2x100 bp run that is
-// 90-99 % of the jobs (Gene table: one haplotype per mate; exon tables: mostly none).  The class is then plain set
-// algebra - none: the table mask; one: its set; two: A and B when that is not empty, else A or B; the mask when all of
-// it is empty (add_stat's max_count rule, core:1196-1209) - so no per-allele counter is needed, the sets never leave
-// the registers and nothing but NEW class rows is written to HBM.  Both kernels of the two-kernel form were bound by
-// their chain of dependent L2 round trips (job -> offsets -> haplotype -> rows -> table rows | job -> set -> CAS -> slot
-// -> row compare), so the chain is cut, not just the bytes:
-//   * a warp takes 32 consecutive jobs; lane i fetches ALL scalars of job i (job, offsets, table, pair, region, and per
-//     haplotype: ends, position bounds, first two variant rows) - a handful of dependent loads per 32 jobs instead of per
-//     job - and the jobs are then replayed one at a time from shuffles;
-//   * jobs without a haplotype all insert the table mask: the lanes of a block that share (unit, table) insert once;
-//   * the CAS of job j's insert stays in flight while job j + 1 reads its table rows (pool_probe_issue / _resolve), and a
-//     hit resolves from the CAS result alone (tagged slot words).
-// Jobs with three or more haplotypes are queued for pair_class_kernel (bit-plane counter).
-struct HapMeta {  // lane-resident scalars of one haplotype
-    int left, lo, hi, pk, r0, rw0, rw1;  // pk = rows (6 bits) | deletions ending inside << 6 (6 bits) | first of them << 12
-};
-__device__ __forceinline__ bool hap_meta_load(const LocusDev &loc, const int32_t *__restrict__ hap_left,
-                                              const int32_t *__restrict__ hap_right, const int64_t *__restrict__ row_off,
-                                              const int32_t *__restrict__ rows, int64_t h, HapMeta &m) {
-    m.left = hap_left[h];
-    const HapBounds hb = hap_bounds(loc, m.left, hap_right[h]);
-    const int64_t r0 = row_off[h];
-    const int k1 = (int)(row_off[h + 1] - r0);
-    m.lo = hb.lo;
-    m.hi = hb.hi;
-    m.r0 = (int)r0;
-    m.rw0 = k1 > 0 ? rows[r0] : 0;
-    m.rw1 = k1 > 1 ? rows[r0 + 1] : 0;
-    const int nd = hb.dhi - hb.dlo;
-    m.pk = k1 | (nd << 6) | (hb.dlo << 12);
-    return k1 < 64 && nd < 64 && hb.dlo < (1 << 19);
-}
-// Set algebra of one haplotype with the table-row loads batched.  hap_allele_set_core waits for every row before it
-// knows the next address (one L2 round trip per row, 3k + 2 rows per haplotype); here the warp first walks the
-// haplotype's scalars - uniform integer work - and leaves the e-th row to fetch with lane e (row id in the sparse table,
-// sign bit = "AND it", else "OR it into the negatives"), then fetches the rows B at a time: B x WPL independent loads per
-// round trip.  More than 32 rows (never seen) takes hap_allele_set_core.
-template <int WPL, int B>
-__device__ __forceinline__ void hap_meta_set(const LocusDev &loc, const int32_t *__restrict__ rows, const HapMeta &m, int j,
-                                             const uint64_t *__restrict__ mask, int lane, uint64_t (&set)[WPL]) {
-    const int left = __shfl_sync(0xffffffffu, m.left, j);
-    const int pk = __shfl_sync(0xffffffffu, m.pk, j);
-    const int lo = __shfl_sync(0xffffffffu, m.lo, j), hi = __shfl_sync(0xffffffffu, m.hi, j);
-    const int dlo = pk >> 12, dhi = dlo + ((pk >> 6) & 63), k1 = pk & 63;
-    const int a0 = __shfl_sync(0xffffffffu, m.rw0, j), a1 = __shfl_sync(0xffffffffu, m.rw1, j);
-    const int32_t *rw = rows + __shfl_sync(0xffffffffu, m.r0, j);
-    auto ROW = [=](int k) { return k == 0 ? a0 : (k == 1 ? a1 : rw[k]); };
-    const int wp = loc.wp;
-    const int V1 = max(loc.V, 1);
-    int mine = 0, n = 0;  // entry of this lane: (level * V + row) | AND flag in the sign bit
-    bool fits = true;
-    for (int d0 = dlo; d0 < dhi; d0 += 32) {  // deletions that start left of the haplotype and end inside it
-        int row = 0;
-        const unsigned qm = del_rows_left_of(loc, d0, dhi, left, ROW, k1, lane, row);
-        const int cnt = __popc(qm);
-        if (cnt) {
-            if (n + cnt > 32) {
-                fits = false;
-                break;
-            }
-            const int v = __shfl_sync(0xffffffffu, row, __fns(qm, 0, lane - n + 1) & 31);
-            if (lane >= n && lane < n + cnt) mine = v;
-            n += cnt;
-        }
-    }
-    if (!fits || n + 3 * k1 + 2 > 32) {
-        HapBounds hb = {lo, hi, dlo, dhi};
-        hap_allele_set_core<WPL>(loc, left, hb, ROW, k1, mask, lane, set);
-        return;
-    }
-    int prev = lo;
-    for (int k = 0; k <= k1; k++) {
-        int endr = hi;
-        if (k < k1) {
-            endr = ROW(k);
-            if (n == lane) mine = endr | (int)0x80000000;
-            n++;
-            if (endr < lo) continue;
-            if (endr > hi) endr = hi;
-        }
-        if (endr > prev && prev < hi) {
-            const int lv = 31 - __clz(endr - prev);
-            if (n == lane) mine = lv * V1 + prev;
-            if (n + 1 == lane) mine = lv * V1 + endr - (1 << lv);
-            n += 2;
-        }
-        prev = max(prev, endr + 1);
-    }
-    uint64_t neg[WPL];
-#pragma unroll
-    for (int i = 0; i < WPL; i++) {
-        set[i] = lane + 32 * i < wp ? mask[32 * i] : 0ull;
-        neg[i] = 0ull;
-    }
-    const uint64_t *st = loc.st + lane;
-    for (int e0 = 0; e0 < n; e0 += B) {
-        uint64_t v[B][WPL];
-        int ent[B];
-#pragma unroll
-        for (int b = 0; b < B; b++) {
-            ent[b] = __shfl_sync(0xffffffffu, mine, (e0 + b) & 31);
-            const uint64_t *row = st + (size_t)(ent[b] & 0x7fffffff) * wp;
-            const bool on = e0 + b < n;
-#pragma unroll
-            for (int i = 0; i < WPL; i++) v[b][i] = (on && lane + 32 * i < wp) ? row[32 * i] : 0ull;
-        }
-#pragma unroll
-        for (int b = 0; b < B; b++) {
-            if (e0 + b < n) {
-                if (ent[b] < 0) {
-#pragma unroll
-                    for (int i = 0; i < WPL; i++) set[i] &= v[b][i];
-                } else {
-#pragma unroll
-                    for (int i = 0; i < WPL; i++) neg[i] |= v[b][i];
-                }
-            }
-        }
-    }
-#pragma unroll
-    for (int i = 0; i < WPL; i++) set[i] &= ~neg[i];
-}
-
-template <int WPL, int MINB>
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, WPL <= 4 ? MINB : 2)
-    job_class_kernel(LocusDev loc, const int64_t *__restrict__ job_off, const int32_t *__restrict__ job_ut,
-                     const int32_t *__restrict__ job_pair, const int32_t *__restrict__ job_list, int64_t n_jobs,
-                     const int32_t *__restrict__ hap_left, const int32_t *__restrict__ hap_right,
-                     const int64_t *__restrict__ row_off, const int32_t *__restrict__ rows, ClassPool pool,
-                     int32_t *__restrict__ multi_n, int32_t *__restrict__ multi_list) {
-    const int lane = threadIdx.x & 31;
-    const int wp = loc.wp;
-    const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
-    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    const int64_t nblk = (n_jobs + 31) >> 5;
-    bool pending = false;
-    PoolProbe pp;
-    uint64_t pbest[WPL];
-    int p_ut = 0, p_pair = 0, p_base = 0, p_limit = 0, p_add = 0;
-    for (int64_t blk = warp0; blk < nblk; blk += nwarps) {
-        const int64_t q = (blk << 5) + lane;
-        int job = 0, nh = -1, ut = 0, pair = 0, base = 0, limit = 0, add = 1;
-        HapMeta m0 = {0, 0, 0, 0, 0, 0, 0}, m1 = m0;
-        if (q < n_jobs) {
-            job = job_list[q];
-            const int64_t h0 = job_off[job];
-            nh = (int)(job_off[job + 1] - h0);
-            ut = job_ut[job];
-            pair = job_pair[job];
-            base = (int)pool.ut_base[ut];
-            limit = (int)pool.ut_base[ut + 1];
-            bool ok = true;
-            if (nh == 1 || nh == 2) ok = hap_meta_load(loc, hap_left, hap_right, row_off, rows, h0, m0);
-            if (nh == 2) ok &= hap_meta_load(loc, hap_left, hap_right, row_off, rows, h0 + 1, m1);
-            if (!ok) nh = 99;  // (scalars beyond the packed form: take the general kernel)
-        }
-        {  // jobs with several haplotypes go to the bit-plane kernel
-            const unsigned multi = __ballot_sync(0xffffffffu, nh > 2);
-            if (multi) {
-                int at = 0;
-                if (lane == 0) at = atomicAdd(multi_n, __popc(multi));
-                at = __shfl_sync(0xffffffffu, at, 0);
-                if (nh > 2) multi_list[at + __popc(multi & ((1u << lane) - 1u))] = job;
-            }
-        }
-        {  // jobs without a haplotype: one insert per (unit, table) of the block, by the first of its lanes (smallest pair)
-            const unsigned none = __ballot_sync(0xffffffffu, nh == 0);
-            if (nh == 0) {
-                const unsigned grp = __match_any_sync(none, ut);
-                add = __popc(grp);
-                if ((__ffs((int)grp) - 1) != lane) nh = -1;
-            }
-        }
-        unsigned todo = __ballot_sync(0xffffffffu, nh >= 0 && nh <= 2);
-        while (todo) {
-            const int j = __ffs((int)todo) - 1;
-            todo &= todo - 1;
-            const int nh_j = __shfl_sync(0xffffffffu, nh, j);
-            const int ut_j = __shfl_sync(0xffffffffu, ut, j);
-            const uint64_t *mask = loc.mask + (size_t)(ut_j & 3) * wp + lane;
-            uint64_t set[WPL];
-            bool empty = true;
-            if (nh_j >= 1) {
-                hap_meta_set<WPL, (MINB <= 2 ? 4 : 2)>(loc, rows, m0, j, mask, lane, set);
-                uint64_t any = 0;
-                if (nh_j == 2) {
-                    uint64_t other[WPL], any2 = 0;
-                    hap_meta_set<WPL, (MINB <= 2 ? 4 : 2)>(loc, rows, m1, j, mask, lane, other);
-#pragma unroll
-                    for (int i = 0; i < WPL; i++) {
-                        any2 |= set[i] & other[i];
-                        any |= set[i] | other[i];
-                    }
-                    const bool both = __any_sync(0xffffffffu, any2 != 0ull);
-#pragma unroll
-                    for (int i = 0; i < WPL; i++) set[i] = both ? (set[i] & other[i]) : (set[i] | other[i]);
-                } else {
-#pragma unroll
-                    for (int i = 0; i < WPL; i++) any |= set[i];
-                }
-                empty = !__any_sync(0xffffffffu, any != 0ull);
-            }
-            if (empty) {  // max_count == 0: every allele of the table (core:1203-1209)
-#pragma unroll
-                for (int i = 0; i < WPL; i++) set[i] = lane + 32 * i < wp ? mask[32 * i] : 0ull;
-            }
-            if (pending)
-                pool_probe_resolve<WPL>(pool, wp, p_ut, p_base, p_limit, pbest, (unsigned long long)p_add, p_pair, lane, pp);
-            pool_probe_issue<WPL>(pool, wp, ut_j, set, lane, pp);
-#pragma unroll
-            for (int i = 0; i < WPL; i++) pbest[i] = set[i];
-            p_ut = ut_j;
-            p_pair = __shfl_sync(0xffffffffu, pair, j);
-            p_base = __shfl_sync(0xffffffffu, base, j);
-            p_limit = __shfl_sync(0xffffffffu, limit, j);
-            p_add = __shfl_sync(0xffffffffu, add, j);
-            pending = true;
-        }
-    }
-    if (pending) pool_probe_resolve<WPL>(pool, wp, p_ut, p_base, p_limit, pbest, (unsigned long long)p_add, p_pair, lane, pp);
 }
 
 // Projection of the Gene table onto a kept allele set (core:1753-1766): every class of table src_ut is ANDed with
@@ -1536,7 +1257,7 @@ struct LocusBatch {
     // job_list (<= 7 haplotypes first, then the rest) | hap_left | hap_right | hap_table | rows
     struct JobArena {
         size_t o_job_off = 0, o_row_off = 0, o_ut_base = 0, o_job_ut = 0, o_job_pair = 0, o_job_list = 0, o_hl = 0, o_hr = 0,
-               o_ht = 0, o_rows = 0, o_multi = 0, bytes = 0;
+               o_ht = 0, o_rows = 0, bytes = 0;
     } ja;
     int64_t n_jobs = 0, n_small = 0, n_big = 0, n_haps = 0, n_rows = 0, max_job_haps = 0;
     std::vector<int64_t> ut_base;  // [n_units*4 + 1]
@@ -1647,20 +1368,6 @@ static int batch_threads(const hgt_params &p) {
 
 // ---- stage 1: text to the device, line count ----------------------------------------------------------------------------------
 static inline size_t a16(size_t x) { return (x + 15) & ~(size_t)15; }
-
-// Stage (a) forms.  Default: two kernels (compat_kernel -> hapbits in HBM -> class_kernel).  HGT_STAGE_A=job selects
-// job_class_kernel (0 / 1 / 2 haplotypes per job, sets stay in registers) + pair_class_kernel for the rest: a fifth of the
-// DRAM traffic, but measured SLOWER on B200 (3.6 vs 2.6 ms per 128-sample step) - every form is bound by warp
-// instructions and L2 round trips per haplotype, not by HBM bytes (DESIGN.md 4).  HGT_STAGE_A=fused = the bit-plane kernel
-// for every job.  All three give identical tables (tests/test_gpu_wide.py).
-enum { STAGE_A_JOB = 0, STAGE_A_SPLIT = 1, STAGE_A_FUSED = 2 };
-static int stage_a_mode() {
-    const char *e = getenv("HGT_STAGE_A");  // (read on every call: the tests switch it between batches)
-    if (e && !strcmp(e, "job")) return STAGE_A_JOB;
-    if (e && !strcmp(e, "fused")) return STAGE_A_FUSED;
-    return STAGE_A_SPLIT;
-}
-static bool stage_a_split() { return stage_a_mode() == STAGE_A_SPLIT; }
 
 static int tune_env(const char *name, int dflt) {  // grid-size experiments without a rebuild
     const char *e = getenv(name);
@@ -2069,7 +1776,6 @@ static hgtd::ReadsView reads_view(hgt_batch *b) {
     R.n_amb = reinterpret_cast<int32_t *>(sm + 16);
     R.n_heads = reinterpret_cast<int32_t *>(sm + 20);
     R.head_list = R.slow_list + std::max<size_t>(N, 1);
-    R.list_sorted = nullptr;
     R.pair_cnt = R.amb_list + 4 * std::max<size_t>(N, 1) + hgtk::SORT_BUCKETS;
     R.max_job_haps = reinterpret_cast<int32_t *>(sm + 12);
     R.unit_reads = reinterpret_cast<unsigned long long *>(sm + rd.s_reads);
@@ -2134,7 +1840,7 @@ static int reads_execute(hgt_batch *b, cudaStream_t st) {
     HGT_CUDA(cudaMemsetAsync(rd.d_cnt.p, 0, (size_t)std::max<int64_t>(rd.POS, 1) * 24, st));
     // ---- line index, records, pileup --------------------------------------------------------------------------------------
     b->timer.begin(ctx, st, 0);
-    int launches = 0;
+    int launches = 4;  // index_lines, unit_lines, parse, pileup_text (pileup_flags below)
     ctx->launches += 5;
     hgtk::index_lines_kernel<<<(unsigned)rd.n_chunks, hgtk::LINE_THREADS, 0, st>>>(rd.d_text.as<char>(), rd.text_bytes,
                                                                                rd.d_chunk.as<int64_t>(), rd.d_line_off.as<int64_t>());
@@ -2144,26 +1850,13 @@ static int reads_execute(hgt_batch *b, cudaStream_t st) {
     int stage_bytes = (int)std::min<int64_t>(
         160 << 10, std::max<int64_t>(16 << 10, (rd.text_bytes / std::max<int64_t>(N, 1) * 147 + 1023) / 1024 * 1024 + 1024));
     if (stage_kb_env > 0) stage_bytes = stage_kb_env << 10;
-    // the walk reads its lines straight from global memory: after the three-pass split the TMA-staged image measured
-    // slower for it (5.97 vs 4.69 ms of walk per step); HGT_WALK_STAGE=1 brings it back for A/B runs
-    static const int walk_stage_off = !getenv("HGT_WALK_STAGE") && !getenv("HGT_WALK_STAGE_ON");
     HGT_CUDA(hgt_smem_at_least((const void *)hgtk::parse_kernel, stage_bytes));
-    HGT_CUDA(hgt_smem_at_least((const void *)hgtk::walk_kernel, stage_bytes));
     const int stage_grid = (int)std::max<int64_t>(1, std::min<int64_t>((N + hgtk::STAGE_LINES - 1) / hgtk::STAGE_LINES,
                                                                      (int64_t)ctx->sm_count * stage_ctas));
-    // The pileup is its own pass (warp per line, 8 CTAs of 256 threads per SM).  HGT_PILEUP_FUSED=1 runs it inside the parse
-    // kernel on the shared-memory image of the lines - one pass over the text less (-0.5 GB of DRAM traffic per step), but
-    // SLOWER: the staged kernel holds 16 warps per SM and the histogram atomics need more in flight (records 1.65 vs 1.39 ms).
-    static const bool pileup_split = getenv("HGT_PILEUP_FUSED") == nullptr;
-    hgtk::parse_kernel<<<stage_grid, hgtk::STAGE_LINES, stage_bytes, st>>>(R, P, stage_bytes,
-                                                                            pileup_split ? nullptr : rd.d_cnt.as<uint32_t>());
-    if (pileup_split) {
-        hgtk::pileup_text_kernel<<<line_grid(ctx, N * 32, 256, 8), 256, 0, st>>>(R, rd.d_cnt.as<uint32_t>());
-        ctx->launches++;
-        launches++;
-    }
-    launches += 3;
-    ctx->launches -= 1;
+    hgtk::parse_kernel<<<stage_grid, hgtk::STAGE_LINES, stage_bytes, st>>>(R, P, stage_bytes);
+    // the pileup is its own pass (warp per line, 8 CTAs of 256 threads per SM): the histogram atomics need more warps in
+    // flight than the staged parse kernel holds
+    hgtk::pileup_text_kernel<<<line_grid(ctx, N * 32, 256, 8), 256, 0, st>>>(R, rd.d_cnt.as<uint32_t>());
     HGT_CUDA(cudaGetLastError());
     if (b->pileup_hook) {  // read-sharded locus: the caller sums the raw counts over ranks (SURVEY.md 8e)
         HGT_CUDA(cudaStreamSynchronize(st));
@@ -2192,23 +1885,15 @@ static int reads_execute(hgt_batch *b, cudaStream_t st) {
     b->timer.begin(ctx, st, 7);
     hgtk::head_kernel<<<line_grid(ctx, N, 256, 8), 256, 0, st>>>(R);
     hgtk::candidate_kernel<<<line_grid(ctx, N, 256, 8), 256, 0, st>>>(R);
-    if (walk_stage_off)
-        hgtk::walk_kernel<<<line_grid(ctx, N, 128, 16), hgtk::STAGE_LINES, 0, st>>>(R, P, 0);
-    else
-        hgtk::walk_kernel<<<stage_grid, hgtk::STAGE_LINES, stage_bytes, st>>>(R, P, stage_bytes);
-    static const bool list_sort = !getenv("HGT_LIST_SORT_OFF");
+    hgtk::walk_kernel<<<line_grid(ctx, N, 128, 16), hgtk::STAGE_LINES, 0, st>>>(R, P);
+    // second pass in backbone order (its length is read on the device)
     int32_t *sorted = rd.d_slow_list.as<int32_t>() + 3 * std::max<size_t>(N, 1), *buckets = sorted + std::max<size_t>(N, 1);
-    launches = 4;
-    if (list_sort) {  // second pass in backbone order (its length is read on the device)
-        HGT_CUDA(cudaMemsetAsync(buckets, 0, (size_t)hgtk::SORT_BUCKETS * 4, st));
-        hgtk::list_hist_kernel<<<line_grid(ctx, N / 8 + 1, 256, 4), 256, 0, st>>>(R, R.amb_list, R.n_amb, buckets);
-        hgtk::list_scan_kernel<<<1, 1024, 0, st>>>(buckets);
-        hgtk::list_scatter_kernel<<<line_grid(ctx, N / 8 + 1, 256, 4), 256, 0, st>>>(R, R.amb_list, R.n_amb, buckets, sorted);
-        R.list_sorted = sorted;
-        launches += 3;
-    }
-    hgtk::walk_amb_kernel<<<line_grid(ctx, N, 128, 16), 128, 0, st>>>(R, P);  // its length is read on the device
-    R.list_sorted = nullptr;
+    HGT_CUDA(cudaMemsetAsync(buckets, 0, (size_t)hgtk::SORT_BUCKETS * 4, st));
+    hgtk::list_hist_kernel<<<line_grid(ctx, N / 8 + 1, 256, 4), 256, 0, st>>>(R, R.amb_list, R.n_amb, buckets);
+    hgtk::list_scan_kernel<<<1, 1024, 0, st>>>(buckets);
+    hgtk::list_scatter_kernel<<<line_grid(ctx, N / 8 + 1, 256, 4), 256, 0, st>>>(R, R.amb_list, R.n_amb, buckets, sorted);
+    hgtk::walk_amb_kernel<<<line_grid(ctx, N, 128, 16), 128, 0, st>>>(R, P, sorted);
+    launches = 7;  // head, candidate, walk, the three list-sort kernels, walk_amb
     ctx->launches += launches;
     HGT_CUDA(cudaGetLastError());
     HGT_CUDA(d2h(rd.h_small.p, rd.d_small.p, 16, st));
@@ -2221,19 +1906,13 @@ static int reads_execute(hgt_batch *b, cudaStream_t st) {
     if (rd.n_slow > 0) {
         HGT_CHECK(rd.d_slow.alloc((size_t)rd.n_slow * sizeof(hgtd::SlowRec)));
         R = reads_view(b);
-        if (list_sort) {
-            HGT_CUDA(cudaMemsetAsync(buckets, 0, (size_t)hgtk::SORT_BUCKETS * 4, st));
-            hgtk::list_hist_kernel<<<line_grid(ctx, rd.n_slow, 256, 4), 256, 0, st>>>(R, R.slow_list, R.n_slow, buckets);
-            hgtk::list_scan_kernel<<<1, 1024, 0, st>>>(buckets);
-            hgtk::list_scatter_kernel<<<line_grid(ctx, rd.n_slow, 256, 4), 256, 0, st>>>(R, R.slow_list, R.n_slow, buckets, sorted);
-            R.list_sorted = sorted;
-            launches += 3;
-            ctx->launches += 3;
-        }
-        hgtk::walk_slow_kernel<<<line_grid(ctx, rd.n_slow, 128, 16), 128, 0, st>>>(R, P, rd.n_slow);
-        R.list_sorted = nullptr;
-        launches++;
-        ctx->launches++;
+        HGT_CUDA(cudaMemsetAsync(buckets, 0, (size_t)hgtk::SORT_BUCKETS * 4, st));
+        hgtk::list_hist_kernel<<<line_grid(ctx, rd.n_slow, 256, 4), 256, 0, st>>>(R, R.slow_list, R.n_slow, buckets);
+        hgtk::list_scan_kernel<<<1, 1024, 0, st>>>(buckets);
+        hgtk::list_scatter_kernel<<<line_grid(ctx, rd.n_slow, 256, 4), 256, 0, st>>>(R, R.slow_list, R.n_slow, buckets, sorted);
+        hgtk::walk_slow_kernel<<<line_grid(ctx, rd.n_slow, 128, 16), 128, 0, st>>>(R, P, sorted, rd.n_slow);
+        launches += 4;
+        ctx->launches += 4;
     }
     HGT_CUDA(cudaMemsetAsync(rd.d_scan.p, 0, (size_t)(N + 1) * 8 * 5, st));
     hgtk::pair_count_kernel<<<line_grid(ctx, N, 128, 16), 128, 0, st>>>(R);
@@ -2303,8 +1982,7 @@ static int reads_execute(hgt_batch *b, cudaStream_t st) {
         ja.o_hr = a16(ja.o_hl + (size_t)H * 4);
         ja.o_ht = a16(ja.o_hr + (size_t)H * 4);
         ja.o_rows = a16(ja.o_ht + (size_t)H * 4);
-        ja.o_multi = a16(ja.o_rows + (size_t)RW * 4);  // [0] = length, [4..] = jobs with >= 2 haplotypes (job_class_kernel)
-        ja.bytes = a16(ja.o_multi + (size_t)(J + 4) * 4);
+        ja.bytes = a16(ja.o_rows + (size_t)RW * 4);
         HGT_CHECK(lb.d_jobs.alloc(ja.bytes));
         HGT_CHECK(lb.h_jobs.alloc((n_units * 4 + 1) * 8));
         memcpy(lb.h_jobs.p, lb.ut_base.data(), (n_units * 4 + 1) * 8);
@@ -2340,7 +2018,7 @@ static int batch_alloc_tables(hgt_batch *b, cudaStream_t st) {
             const size_t n_units = lb.units.size();
             lb.cap = 64;
             while ((int64_t)lb.cap < 2 * std::max<int64_t>(lb.n_rows_pool, 1)) lb.cap <<= 1;
-            if (stage_a_split()) HGT_CHECK(lb.d_hapbits.alloc((size_t)std::max<int64_t>(lb.n_haps, 1) * wp * 8));
+            HGT_CHECK(lb.d_hapbits.alloc((size_t)std::max<int64_t>(lb.n_haps, 1) * wp * 8));
             HGT_CHECK(lb.d_keys.alloc((size_t)lb.cap * 8));
             const size_t pr = (size_t)std::max<int64_t>(lb.n_rows_pool, 1);
             HGT_CHECK(lb.d_bits.alloc(pr * wp * 8));
@@ -2507,51 +2185,6 @@ static void launch_stage_a(hgt_batch *b, cudaStream_t st, LocusBatch &lb) {
     const LocusDev ld = locus_dev(loc);
     const int wp = loc->wp;
     const int64_t H = lb.n_haps;
-    const int mode = stage_a_mode();
-    if (mode != STAGE_A_SPLIT) {
-        const ClassPool pool = lb.pool();
-        const int64_t ns = lb.n_small, nb = lb.n_big;
-        int n_launch = 0;
-        b->timer.begin(ctx, st, 2);
-        const int32_t *small_list = lb.dj<int32_t>(lb.ja.o_job_list), *small_n = nullptr;
-        if (ns > 0 && mode == STAGE_A_JOB) {
-            static const int job_per_sm = tune_env("HGT_JOB_CTAS_PER_SM", 16);
-            int32_t *multi = lb.dj<int32_t>(lb.ja.o_multi);
-            cudaMemsetAsync(multi, 0, 16, st);
-            const int64_t blocks = (ns + 31) / 32;
-            const int ctas = (int)std::min<int64_t>((blocks + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (int64_t)ctx->sm_count * job_per_sm);
-            static const int minb = tune_env("HGT_JOB_MINB", 3);  // resident CTAs per SM the kernel is compiled for (64 / 80 / 128 registers)
-            auto kern = minb == 3 ? job_class_kernel<WPL, 3> : (minb == 2 ? job_class_kernel<WPL, 2> : job_class_kernel<WPL, 4>);
-            kern<<<ctas, WARPS_PER_CTA * 32, 0, st>>>(
-                ld, lb.dj<int64_t>(lb.ja.o_job_off), lb.dj<int32_t>(lb.ja.o_job_ut), lb.dj<int32_t>(lb.ja.o_job_pair), small_list, ns,
-                lb.dj<int32_t>(lb.ja.o_hl), lb.dj<int32_t>(lb.ja.o_hr), lb.dj<int64_t>(lb.ja.o_row_off), lb.dj<int32_t>(lb.ja.o_rows),
-                pool, multi, multi + 4);
-            small_list = multi + 4;
-            small_n = multi;
-            n_launch++;
-        }
-        if (ns > 0) {
-            // (job form: the list length is on the device; 2-3 % of the jobs, so a small grid)
-            const int64_t est = small_n ? std::max<int64_t>(ns / 8, 1) : ns;
-            const int ctas = (int)std::min<int64_t>((est + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (int64_t)ctx->sm_count * 8);
-            pair_class_kernel<WPL, 3><<<ctas, WARPS_PER_CTA * 32, 0, st>>>(
-                ld, lb.dj<int64_t>(lb.ja.o_job_off), lb.dj<int32_t>(lb.ja.o_job_ut), lb.dj<int32_t>(lb.ja.o_job_pair), small_list, ns,
-                lb.dj<int32_t>(lb.ja.o_hl), lb.dj<int32_t>(lb.ja.o_hr), lb.dj<int64_t>(lb.ja.o_row_off), lb.dj<int32_t>(lb.ja.o_rows),
-                pool, small_n);
-            n_launch++;
-        }
-        if (nb > 0) {
-            const int ctas = (int)std::min<int64_t>((nb + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (int64_t)ctx->sm_count * 8);
-            pair_class_kernel<WPL, 8><<<ctas, WARPS_PER_CTA * 32, 0, st>>>(
-                ld, lb.dj<int64_t>(lb.ja.o_job_off), lb.dj<int32_t>(lb.ja.o_job_ut), lb.dj<int32_t>(lb.ja.o_job_pair),
-                lb.dj<int32_t>(lb.ja.o_job_list) + ns, nb, lb.dj<int32_t>(lb.ja.o_hl), lb.dj<int32_t>(lb.ja.o_hr),
-                lb.dj<int64_t>(lb.ja.o_row_off), lb.dj<int32_t>(lb.ja.o_rows), pool, nullptr);
-            n_launch++;
-        }
-        ctx->launches += n_launch;
-        b->timer.end(n_launch);
-        return;
-    }
     b->timer.begin(ctx, st, 1);
     if (H > 0) {
         const int ctas = (int)std::min<int64_t>((H + WARPS_PER_CTA - 1) / WARPS_PER_CTA, (int64_t)ctx->sm_count * compat_per_sm);

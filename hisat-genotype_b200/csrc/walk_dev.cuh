@@ -189,7 +189,6 @@ struct ReadsView {
     int32_t *h_ids;            // [n_lines][MAXI]
     SlowRec *slow;
     int32_t *amb_list, *slow_list;  // lines queued for the second pass (an Alts anchor in reach) / the third (several haplotypes)
-    const int32_t *list_sorted;     // the list of the running pass ordered by position (reads.cuh list_*_kernel); null = as queued
     int32_t *n_amb, *n_slow;
     int32_t *head_list, *n_heads;   // run heads (any order): the pair stage runs one thread per run
     // units

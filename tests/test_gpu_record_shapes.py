@@ -138,10 +138,10 @@ def test_staging_long_block_in_short_batch():
     t.close()
 
 
-@pytest.mark.parametrize("env", ["HGT_STAGE_KB=16", "HGT_WALK_STAGE=1"])
+@pytest.mark.parametrize("env", ["HGT_STAGE_KB=16"])
 def test_stage_switches(env):
-    """The length, probe and staging cases with a 16 KB stage (every block of 128 lines overflows it) and with the
-    staged walk kernel.  Both switches are read once per process, hence the child interpreter."""
+    """The length, probe and staging cases with a 16 KB stage (every block of 128 lines overflows it).  The switch is
+    read once per process, hence the child interpreter."""
     k, v = env.split("=")
     r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(ROOT, "tests", "test_gpu_record_shapes.py"), "-x", "-q",
                         "-m", "gpu", "-k", "test_lengths or test_mask_probes or test_staging_long",
@@ -177,16 +177,11 @@ def test_capacity_past_limit_refused(kind):
     t.close()
 
 
-@pytest.mark.parametrize("form", [None, "job", "fused"])
-def test_job_split_7_and_8(form, monkeypatch):
-    """Exon-table jobs of exactly 7 haplotypes (3 bit planes) and exactly 8 (8 bit planes), winning counts 7 and 8, under
-    every stage (a) form; plus the pair of 255 haplotypes (the largest count) of the capacity case."""
+def test_job_split_7_and_8():
+    """Exon-table jobs of exactly 7 haplotypes (3 bit planes) and exactly 8 (8 bit planes), winning counts 7 and 8; plus
+    the pair of 255 haplotypes (the largest count) of the capacity case."""
     from hisatgenotype_b200 import typing_core as TC
     from hisatgenotype_b200.locus import LocusTables
-    if form:
-        monkeypatch.setenv("HGT_STAGE_A", form)
-    else:
-        monkeypatch.delenv("HGT_STAGE_A", raising=False)
     loc, lines, n8 = F.job_split_case()
     args = F.locus_args(loc)
     ol, ref, hts = oracle_run(args, lines, {})
