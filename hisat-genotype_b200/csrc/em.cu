@@ -1535,68 +1535,6 @@ __global__ void __launch_bounds__(EM_THREADS, 1) em_kernel(const EmArgs *__restr
     }
 }
 
-// ---- partial sweeps for a read-sharded locus (SURVEY.md 8e) ---------------------------------------------------------
-// The class rows of one locus are spread over several GPUs; one next_prob() is then: every rank runs em_part_kernel +
-// em_part_reduce_kernel over ITS rows with the global probability vector, the per-allele sums are all-reduced (NCCL),
-// and every rank finishes the step identically (hisat-genotype_b200/em_dist.py).
-template <int NA>
-__global__ void __launch_bounds__(EM_THREADS, 1) em_part_kernel(EmArgs a, int mode, const double *__restrict__ pin) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int tid = threadIdx.x;
-    Smem sm;
-    sm.mbar = reinterpret_cast<uint64_t *>(smem_raw);
-    sm.red = reinterpret_cast<double *>(smem_raw + 16);
-    sm.lv = nullptr; sm.cnt = nullptr; sm.cm64 = nullptr; sm.c64 = nullptr;
-    sm.row_off = nullptr; sm.col_off = nullptr; sm.r_ent = nullptr; sm.c_ent = nullptr; sm.dense_g = nullptr;
-    sm.mult = nullptr;
-    const int Apad = a.wp * 64;
-    sm.p = sm.red + 40;
-    sm.w = sm.p + p_slots(Apad);
-    sm.slab = reinterpret_cast<uint64_t *>(sm.w + a.slab_rows);
-    sm.valid = reinterpret_cast<uint8_t *>(sm.slab + (size_t)a.slab_rows * a.wp);
-    if (tid == 0) {
-        mbar_init(sm.mbar, 1);
-        fence_barrier_init();
-    }
-    __syncthreads();
-    const int G = gridDim.x, g = blockIdx.x;
-    const int per = (a.C + G - 1) / G;
-    const int row_lo = min(a.C, g * per), row_hi = min(a.C, row_lo + per);
-    bool loaded = false;
-    uint32_t parity = 0;
-    double acc[NA];
-    int32_t fk[NA];
-    uint32_t hit = 0;
-    Trace tr;
-    tr.on = false; tr.t = 0; tr.ns0 = 0;
-    em_accumulate<NA>(a, sm, mode, pin, nullptr, row_lo, row_hi, false, loaded, parity, acc, fk, hit, tr);
-#pragma unroll
-    for (int i = 0; i < NA; i++) {
-        const int al = tid + i * EM_THREADS;
-        if (al < a.A) {
-            a.part_acc[(size_t)g * Apad + al] = acc[i];
-            a.part_aux[(size_t)g * Apad + al] = (mode == MODE_FIRSTK) ? fk[i] : (int32_t)((hit >> i) & 1u);
-        }
-    }
-}
-
-__global__ void em_part_reduce_kernel(int G, int A, int Apad, int mode, const double *__restrict__ part_acc,
-                                      const int32_t *__restrict__ part_aux, double *__restrict__ acc_out,
-                                      int32_t *__restrict__ aux_out, double *__restrict__ hit_out) {
-    const int al = blockIdx.x * blockDim.x + threadIdx.x;
-    if (al >= A) return;
-    double s = 0.0;
-    int32_t x = (mode == MODE_FIRSTK) ? FK_NONE : 0;
-    for (int g = 0; g < G; g++) {  // fixed order: reproducible
-        s += part_acc[(size_t)g * Apad + al];
-        const int32_t y = part_aux[(size_t)g * Apad + al];
-        x = (mode == MODE_FIRSTK) ? min(x, y) : (x | y);
-    }
-    if (acc_out) acc_out[al] = s;
-    if (aux_out) aux_out[al] = x;
-    if (hit_out) hit_out[al] = (double)x;  // modes 0, 1: the flag as a summable number (one all-reduce for both)
-}
-
 struct EmPlan {
     int na;
     int slab_rows;
@@ -2094,247 +2032,6 @@ extern "C" int hgt_em_batch(hgt_ctx *ctx, int32_t n_problems, const uint64_t *cl
         if (iters) iters[i] = is[(size_t)i * 3];
         if (status) status[i] = is[(size_t)i * 3 + 1];
     }
-    return HGT_OK;
-}
-
-extern "C" size_t hgt_em_partial_workspace_bytes(const hgt_ctx *ctx, int32_t n_alleles) {
-    const size_t Apad = (size_t)hgt_row_pitch(n_alleles) * 64;
-    const int G = ctx ? ctx->sm_count : 148;
-    return align_up((size_t)G * Apad * 8, 256) + align_up((size_t)G * Apad * 4, 256);
-}
-
-static int em_partial_impl(hgt_ctx *ctx, void *stream, const uint64_t *class_bits, const double *class_count_f64,
-                           const uint64_t *class_count_u64, const int32_t *class_key, int32_t key_offset,
-                           int32_t n_classes, int32_t n_alleles, int32_t wp, const double *p_in, int32_t mode,
-                           double *acc_out, int32_t *aux_out, double *hit_out, void *workspace);
-
-extern "C" int hgt_em_partial_dev(hgt_ctx *ctx, void *stream, const uint64_t *class_bits, const double *class_count_f64,
-                                  const uint64_t *class_count_u64, const int32_t *class_key, int32_t key_offset,
-                                  int32_t n_classes, int32_t n_alleles, int32_t wp, const double *p_in, int32_t mode,
-                                  double *acc_out, int32_t *aux_out, void *workspace) {
-    return em_partial_impl(ctx, stream, class_bits, class_count_f64, class_count_u64, class_key, key_offset, n_classes,
-                           n_alleles, wp, p_in, mode, acc_out, aux_out, nullptr, workspace);
-}
-
-static int em_partial_impl(hgt_ctx *ctx, void *stream, const uint64_t *class_bits, const double *class_count_f64,
-                           const uint64_t *class_count_u64, const int32_t *class_key, int32_t key_offset,
-                           int32_t n_classes, int32_t n_alleles, int32_t wp, const double *p_in, int32_t mode,
-                           double *acc_out, int32_t *aux_out, double *hit_out, void *workspace) {
-    if (!ctx || (!acc_out && !aux_out) || !workspace || (!class_count_f64 && !class_count_u64 && n_classes > 0) ||
-        (mode != MODE_INIT && !p_in) || mode < 0 || mode > 2 || (n_classes > 0 && !class_bits)) {
-        hgt_set_error("hgt_em_partial_dev: bad argument");
-        return HGT_ERR_ARG;
-    }
-    if (wp != hgt_row_pitch(n_alleles) || n_alleles < 1 || n_classes < 0) {
-        hgt_set_error("hgt_em_partial_dev: need n_alleles >= 1 and wp == hgt_row_pitch(n_alleles)");
-        return HGT_ERR_ARG;
-    }
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const size_t Apad = (size_t)wp * 64;
-    int G = ctx->sm_count;
-    if (G > n_classes) G = n_classes < 1 ? 1 : n_classes;
-    EmPlan plan;
-    HGT_CHECK(em_plan(ctx, (n_classes + G - 1) / G, n_alleles, wp, &plan));
-    EmArgs a;
-    memset(&a, 0, sizeof(a));
-    a.bits = class_bits; a.cnt = class_count_f64; a.cnt_u64 = reinterpret_cast<const unsigned long long *>(class_count_u64);
-    a.class_first = class_key; a.key_offset = key_offset;
-    a.C = n_classes; a.A = n_alleles; a.wp = wp; a.slab_rows = plan.slab_rows;
-    unsigned char *w = static_cast<unsigned char *>(workspace);
-    a.part_acc = reinterpret_cast<double *>(w);
-    a.part_aux = reinterpret_cast<int32_t *>(w + align_up((size_t)ctx->sm_count * Apad * 8, 256));
-    void (*kern)(EmArgs, int, const double *) = nullptr;
-    switch (plan.na) {
-        case 1: kern = em_part_kernel<1>; break;
-        case 2: kern = em_part_kernel<2>; break;
-        case 4: kern = em_part_kernel<4>; break;
-        case 8: kern = em_part_kernel<8>; break;
-        default: kern = em_part_kernel<16>; break;
-    }
-    HGT_CUDA(hgt_smem_at_least((const void *)kern, plan.smem));
-    kern<<<G, EM_THREADS, plan.smem, st>>>(a, mode, p_in);
-    HGT_CUDA(cudaGetLastError());
-    em_part_reduce_kernel<<<(n_alleles + 255) / 256, 256, 0, st>>>(G, n_alleles, (int)Apad, mode, a.part_acc, a.part_aux,
-                                                                   acc_out, aux_out, hit_out);
-    HGT_CUDA(cudaGetLastError());
-    ctx->launches += 2;
-    return HGT_OK;
-}
-
-
-// ---- read-sharded locus: the O(A) vector half of the loop on the device ---------------------------------------------
-// State block (device, caller-allocated, hgt_em_shard_state_bytes): doubles vec[6][A] (0 p0, 1 p1, 2 p2, 3 p3, 4 p1', 5
-// last input), red[2A] (all-reduce buffer: sums | hit counts), scal[8] (0 sum r^2, 1 sum v^2, 2 key error, 3 division by
-// zero, 4 diff, 5 third sweep used, 6 keys left, 7 -), then int32 fk[A], then bytes live[5][A] (0 l0, 1 l1, 2 l2, 3 l1', 4
-// last).  Every vector op is ONE single-CTA kernel (A <= 16 k), so an iteration of the reference loop (common:1351-1400)
-// is 3 x (sweep, all-reduce, finish) + squarem + advance and ONE host read of scal.
-struct ShardState {
-    double *vec, *red, *scal;
-    int32_t *fk;
-    uint8_t *live;
-};
-__host__ __device__ inline ShardState shard_state(void *base, int A) {
-    ShardState s;
-    unsigned char *b = static_cast<unsigned char *>(base);
-    s.vec = reinterpret_cast<double *>(b);
-    s.red = s.vec + 6 * (size_t)A;
-    s.scal = s.red + 2 * (size_t)A;
-    s.fk = reinterpret_cast<int32_t *>(s.scal + 8);
-    s.live = reinterpret_cast<uint8_t *>(s.fk + (((size_t)A + 1) & ~(size_t)1));
-    return s;
-}
-enum { SHARD_FINISH = 0, SHARD_SQUAREM = 1, SHARD_ADVANCE = 2, SHARD_FINAL = 3 };
-
-__device__ void shard_prune(int A, double *p, uint8_t *live, double *red) {  // select_alleles (common:1338-1346)
-    double mx = -1.0;
-    for (int al = threadIdx.x; al < A; al += EM_THREADS)
-        if (live[al]) mx = fmax(mx, p[al]);
-    mx = block_max(mx, red);
-    if (mx < 0.0) return;
-    const double thr = mx / 10.0;
-    for (int al = threadIdx.x; al < A; al += EM_THREADS)
-        if (live[al] && !(p[al] >= thr)) {
-            live[al] = 0;
-            p[al] = 0.0;
-        }
-    __syncthreads();
-}
-
-__global__ void __launch_bounds__(EM_THREADS, 1)
-    em_shard_vec_kernel(int op, int A, void *state, const double *__restrict__ len, int src, int dst, int it, int remove_low) {
-    __shared__ double red[40];
-    const ShardState s = shard_state(state, A);
-    const int tid = threadIdx.x;
-    if (op == SHARD_FINISH) {
-        // normalize (common:1285-1297) of q = p * sums over keys = live & hit; src < 0: initial mass (q = sums, keys = hit)
-        const double *pin = src >= 0 ? s.vec + (size_t)(src == 3 ? 3 : src) * A : nullptr;
-        const uint8_t *lin = src < 0 ? nullptr : s.live + (size_t)(src == 3 ? 2 : src) * A;  // p3 is masked by l2
-        double *pout = s.vec + (size_t)dst * A;
-        uint8_t *lout = s.live + (size_t)(dst == 4 ? 3 : dst) * A;
-        double part = 0.0;
-        int any = 0;
-        for (int al = tid; al < A; al += EM_THREADS) {
-            const bool key = s.red[A + al] > 0.0 && (!lin || lin[al]);
-            double q = 0.0;
-            if (key) {
-                q = pin ? pin[al] * s.red[al] : s.red[al];
-                if (len) q = q / len[al];
-                any = 1;
-            }
-            pout[al] = q;
-            lout[al] = key ? 1 : 0;
-            part += q;
-        }
-        const double total = block_sum(part, red);
-        any = block_or(any);
-        if (any && !(total > 0.0) && !(total < 0.0) && tid == 0) s.scal[3] = 1.0;
-        for (int al = tid; al < A; al += EM_THREADS) pout[al] = lout[al] ? pout[al] / total : 0.0;
-    } else if (op == SHARD_SQUAREM) {
-        // common:1361-1383
-        const double *p0 = s.vec, *p1 = s.vec + A, *p2 = s.vec + 2 * (size_t)A;
-        double *p3 = s.vec + 3 * (size_t)A;
-        const uint8_t *l0 = s.live, *l1 = s.live + A, *l2 = s.live + 2 * (size_t)A;
-        double ssr = 0.0, ssv = 0.0;
-        int keyerr = 0;
-        for (int al = tid; al < A; al += EM_THREADS)
-            if (l0[al]) {
-                if (!l1[al] || !l2[al]) keyerr = 1;
-                const double r = p1[al] - p0[al], v = p2[al] - p1[al] - r;
-                ssr += r * r;
-                ssv += v * v;
-            }
-        ssr = block_sum(ssr, red);
-        ssv = block_sum(ssv, red);
-        keyerr = block_or(keyerr);
-        const double g = ssv > 0.0 ? -sqrt(ssr / ssv) : 0.0;
-        for (int al = tid; al < A; al += EM_THREADS) {
-            double x = 0.0;
-            if (l0[al] && l2[al] && ssv > 0.0) {
-                const double r = p1[al] - p0[al], v = p2[al] - p1[al] - r;
-                x = p0[al] - 2 * g * r + g * g * v;
-                x = x > 0.0 ? x : 0.0;
-            }
-            p3[al] = x;
-        }
-        if (tid == 0) {
-            s.scal[0] = ssr; s.scal[1] = ssv;
-            if (keyerr) s.scal[2] = 1.0;
-            s.scal[5] = ssv > 0.0 ? 1.0 : 0.0;
-        }
-    } else if (op == SHARD_ADVANCE) {
-        // prob_diff (common:1272-1279), Gene_prob = Gene_prob_next, select_alleles from iteration 10 on
-        const bool use3 = s.scal[5] != 0.0;
-        double *p0 = s.vec, *lastp = s.vec + 5 * (size_t)A;
-        const double *pn = s.vec + (size_t)(use3 ? 4 : 1) * A, *p3 = s.vec + 3 * (size_t)A;
-        uint8_t *l0 = s.live, *lastl = s.live + 4 * (size_t)A;
-        const uint8_t *ln = s.live + (size_t)(use3 ? 3 : 1) * A, *l2 = s.live + 2 * (size_t)A;
-        double d = 0.0;
-        for (int al = tid; al < A; al += EM_THREADS) {
-            const double a0 = p0[al], an = pn[al];
-            const uint8_t k0 = l0[al], kn = ln[al];
-            if (k0) d += kn ? fabs(a0 - an) : a0;
-            lastp[al] = use3 ? (l2[al] ? p3[al] : 0.0) : (k0 ? a0 : 0.0);
-            lastl[al] = use3 ? l2[al] : k0;
-            p0[al] = an;
-            l0[al] = kn;
-        }
-        d = block_sum(d, red);
-        if (it >= 10 && remove_low) shard_prune(A, p0, l0, red);
-        if (tid == 0) s.scal[4] = d;
-    } else {  // SHARD_FINAL: last select_alleles + normalize (common:1402-1407); prob -> vec[1], keys stay in live[0]
-        double *p0 = s.vec, *prob = s.vec + A;
-        uint8_t *l0 = s.live;
-        if (remove_low) shard_prune(A, p0, l0, red);
-        double part = 0.0;
-        int any = 0;
-        for (int al = tid; al < A; al += EM_THREADS)
-            if (l0[al]) {
-                part += len ? p0[al] / len[al] : p0[al];
-                any = 1;
-            }
-        const double total = block_sum(part, red);
-        any = block_or(any);
-        if (any && !(total > 0.0) && !(total < 0.0) && tid == 0) s.scal[3] = 1.0;
-        for (int al = tid; al < A; al += EM_THREADS)
-            prob[al] = l0[al] ? (len ? p0[al] / len[al] / total : p0[al] / total) : 0.0;
-        if (tid == 0) s.scal[6] = any ? 1.0 : 0.0;
-    }
-}
-
-extern "C" size_t hgt_em_shard_state_bytes(int32_t n_alleles) {
-    const size_t A = (size_t)(n_alleles < 1 ? 1 : n_alleles);
-    return align_up((8 * A + 8) * 8 + ((A + 1) & ~(size_t)1) * 4 + 5 * A, 256);
-}
-
-extern "C" int hgt_em_shard_sweep_dev(hgt_ctx *ctx, void *stream, const uint64_t *class_bits, const double *class_count_f64,
-                                      const uint64_t *class_count_u64, const int32_t *class_key, int32_t key_offset,
-                                      int32_t n_classes, int32_t n_alleles, int32_t wp, int32_t mode, int32_t src,
-                                      void *state, void *workspace) {
-    if (!state || src > 5) {
-        hgt_set_error("hgt_em_shard_sweep_dev: bad argument");
-        return HGT_ERR_ARG;
-    }
-    const ShardState s = shard_state(state, n_alleles);
-    const double *pin = (mode == MODE_INIT || src < 0) ? nullptr : s.vec + (size_t)src * n_alleles;
-    if (mode == MODE_FIRSTK)
-        return em_partial_impl(ctx, stream, class_bits, class_count_f64, class_count_u64, class_key, key_offset, n_classes,
-                               n_alleles, wp, pin, mode, nullptr, s.fk, nullptr, workspace);
-    return em_partial_impl(ctx, stream, class_bits, class_count_f64, class_count_u64, class_key, key_offset, n_classes,
-                           n_alleles, wp, pin, mode, s.red, nullptr, s.red + n_alleles, workspace);
-}
-
-extern "C" int hgt_em_shard_vec_dev(hgt_ctx *ctx, void *stream, int32_t op, int32_t n_alleles, void *state,
-                                    const double *allele_len, int32_t src, int32_t dst, int32_t iteration,
-                                    int32_t remove_low) {
-    if (!ctx || !state || op < SHARD_FINISH || op > SHARD_FINAL || n_alleles < 1 || n_alleles > 16 * EM_THREADS ||
-        (op == SHARD_FINISH && (src > 3 || dst < 0 || dst > 4 || dst == 3))) {
-        hgt_set_error("hgt_em_shard_vec_dev: bad argument");
-        return HGT_ERR_ARG;
-    }
-    em_shard_vec_kernel<<<1, EM_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(op, n_alleles, state, allele_len, src, dst,
-                                                                                 iteration, remove_low);
-    HGT_CUDA(cudaGetLastError());
-    ctx->launches++;
     return HGT_OK;
 }
 

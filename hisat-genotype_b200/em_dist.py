@@ -1,17 +1,15 @@
 """EM abundance for ONE locus whose reads (hence class tables) are sharded over several GPUs (SURVEY.md 8e).
 
-Every rank holds the Gene_cmpt classes of its own reads; classes that occur on several ranks simply appear several
-times, which the EM sums do not mind.  One next_prob() evaluation (reference hisatgenotype_typing_common.py:1311-1336)
-is then
-    local partial sweep over this rank's class rows  (CUDA: hgt_em_partial_dev, csrc/em.cu)
-    all-reduce of the per-allele sums                (torch.distributed: NCCL over NVLink; 8*A bytes, 64 KB at A = 8 k)
-    normalisation / SQUAREM / pruning                (identical on every rank: O(A) vector work)
-and the control flow below is the reference's loop (common:1351-1409) statement by statement, so a world of one
-rank reproduces hgt_em and a world of N ranks differs from it only by the association of the partial sums.
-
-The sweep is a backend object so that the distributed control flow can be exercised without a GPU
-(tests/test_dist_em.py runs it under gloo with a numpy sweep); the product backend is CudaSweep and has no
-fallback.
+Every rank holds the Gene_cmpt classes of its own reads; a class can occur on several ranks.  The pieces, in the order
+Batch.sharded_abundance uses them:
+    pileup_allreduce_hook   sums the raw pileup counts over the ranks before the representative-base sets are derived
+                            (the reference uses the pileup of ALL reads, common:1124-1134)
+    merge_class_tables      gathers every rank's class table (gather_class_tables: NCCL all_gather, once per call) and
+                            keeps the rows this rank owns, duplicates merged (CUDA: hgt_class_merge_dev, csrc/typing.cu),
+                            so that every class lives on exactly one rank
+    single_abundance_peer   the reference loop (common:1282-1410) as ONE cooperative kernel per rank that sums the
+                            per-allele accumulators of every sweep over the ranks through NVLink peer memory
+                            (CUDA: hgt_em_peer_dev, csrc/em.cu; exchange blocks mapped with CUDA IPC by PeerGroup)
 """
 from __future__ import annotations
 
@@ -22,233 +20,7 @@ import torch
 
 from . import _lib
 
-MODE_INIT, MODE_NEXT, MODE_FIRSTK = 0, 1, 2
 FK_NONE = 0x7FFFFFFF
-
-
-class CudaSweep:
-    """Partial sweeps on this rank's device-resident class table (pointers from hgt_batch_unit_table_dev or tensors)."""
-
-    def __init__(self, n_alleles, bits_ptr, n_classes, count_u64_ptr=None, count_f64_ptr=None, key_ptr=None, key_offset=0,
-                 device=None, keep=()):
-        self.A = int(n_alleles)
-        self.wp = _lib.row_pitch(self.A)
-        self.C = int(n_classes)
-        self.bits_ptr, self.cnt_u64, self.cnt_f64, self.key_ptr = bits_ptr, count_u64_ptr, count_f64_ptr, key_ptr
-        self.key_offset = int(key_offset)
-        self.dev_index = _lib.default_device() if device is None else device
-        self.device = torch.device("cuda", self.dev_index)
-        self.ctx = _lib.ctx(self.dev_index)
-        L = _lib.lib()
-        L.hgt_em_partial_workspace_bytes.restype = ctypes.c_size_t
-        L.hgt_em_partial_workspace_bytes.argtypes = [ctypes.c_void_p, ctypes.c_int32]
-        L.hgt_em_partial_dev.restype = ctypes.c_int
-        L.hgt_em_partial_dev.argtypes = [ctypes.c_void_p] * 6 + [ctypes.c_int32] * 4 + [ctypes.c_void_p, ctypes.c_int32,
-                                                                                      ctypes.c_void_p, ctypes.c_void_p,
-                                                                                      ctypes.c_void_p]
-        L.hgt_em_shard_state_bytes.restype = ctypes.c_size_t
-        L.hgt_em_shard_state_bytes.argtypes = [ctypes.c_int32]
-        L.hgt_em_shard_sweep_dev.restype = ctypes.c_int
-        L.hgt_em_shard_sweep_dev.argtypes = [ctypes.c_void_p] * 6 + [ctypes.c_int32] * 6 + [ctypes.c_void_p, ctypes.c_void_p]
-        L.hgt_em_shard_vec_dev.restype = ctypes.c_int
-        L.hgt_em_shard_vec_dev.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p,
-                                           ctypes.c_void_p] + [ctypes.c_int32] * 4
-        self.L = L
-        self.ws = torch.empty(L.hgt_em_partial_workspace_bytes(self.ctx, self.A), dtype=torch.uint8, device=self.device)
-        self._keep = keep  # tensors that own the memory behind the raw pointers
-        # device-resident loop state (csrc/em.cu, "State block"): vec[6][A] | red[2A] | scal[8] | fk[A] | live[5][A]
-        A = self.A
-        self.state = torch.zeros(L.hgt_em_shard_state_bytes(A), dtype=torch.uint8, device=self.device)
-        f64 = self.state[:(8 * A + 8) * 8].view(torch.float64)
-        self.vec = f64[:6 * A].view(6, A)
-        self.red = f64[6 * A:8 * A]
-        self.scal = f64[8 * A:8 * A + 8]
-        o_fk = (8 * A + 8) * 8
-        self.fk = self.state[o_fk:o_fk + 4 * A].view(torch.int32)
-        o_live = o_fk + 4 * ((A + 1) & ~1)
-        self.live = self.state[o_live:o_live + 5 * A].view(5, A)
-
-    @classmethod
-    def from_arrays(cls, class_bits, class_count, n_alleles, class_key=None, key_offset=0, device=None):
-        dev = torch.device("cuda", _lib.default_device() if device is None else device)
-        bits = torch.from_numpy(np.ascontiguousarray(class_bits, np.uint64).view(np.int64)).to(dev)
-        cnt = torch.from_numpy(np.ascontiguousarray(class_count, np.float64)).to(dev)
-        key = None if class_key is None else torch.from_numpy(np.ascontiguousarray(class_key, np.int32)).to(dev)
-        return cls(n_alleles, bits.data_ptr(), len(class_count), None, cnt.data_ptr(), None if key is None else key.data_ptr(),
-                   key_offset, dev.index, keep=(bits, cnt, key))
-
-    def sweep(self, mode, p):
-        acc = torch.empty(self.A, dtype=torch.float64, device=self.device)
-        aux = torch.empty(self.A, dtype=torch.int32, device=self.device)
-        stream = torch.cuda.current_stream(self.device).cuda_stream
-        rc = self.L.hgt_em_partial_dev(self.ctx, stream, self.bits_ptr, self.cnt_f64, self.cnt_u64, self.key_ptr,
-                                       self.key_offset, self.C, self.A, self.wp, None if p is None else p.data_ptr(), mode,
-                                       acc.data_ptr(), aux.data_ptr(), self.ws.data_ptr())
-        _lib.check(rc)
-        return acc, aux
-
-
-    # ---- device-resident loop: sweeps and O(A) vector steps are kernels of libhgt, nothing but the all-reduce is torch
-    def dev_sweep(self, mode, src, stream=None):
-        if stream is None:
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-        _lib.check(self.L.hgt_em_shard_sweep_dev(self.ctx, stream, self.bits_ptr, self.cnt_f64, self.cnt_u64, self.key_ptr,
-                                                 self.key_offset, self.C, self.A, self.wp, mode, src, self.state.data_ptr(),
-                                                 self.ws.data_ptr()))
-
-    def dev_vec(self, op, len_ptr, src=0, dst=0, iteration=0, remove_low=False, stream=None):
-        if stream is None:
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-        _lib.check(self.L.hgt_em_shard_vec_dev(self.ctx, stream, op, self.A, self.state.data_ptr(), len_ptr, src, dst,
-                                               iteration, 1 if remove_low else 0))
-
-
-SHARD_FINISH, SHARD_SQUAREM, SHARD_ADVANCE, SHARD_FINAL = 0, 1, 2, 3
-
-
-def _single_abundance_sharded_dev(backend, allele_len, remove_low, group, max_iter):
-    """The loop of single_abundance_sharded with every vector step on the device (hgt_em_shard_vec_dev): per iteration
-    3 x (partial sweep, all-reduce of red[2A], finish) + squarem + advance, and ONE 64-byte host read (diff, key error,
-    division by zero).  The third next_prob always runs; when sum(v^2) == 0 its result is dropped on the device, which is
-    what the reference's `if` does (common:1371-1383)."""
-    import torch.distributed as dist
-    SUM = dist.ReduceOp.SUM if dist.is_available() else None
-    MIN = dist.ReduceOp.MIN if dist.is_available() else None
-    b = backend
-    ln = None if allele_len is None else torch.as_tensor(np.asarray(allele_len, np.float64), device=b.device)
-    ln_ptr = None if ln is None else ln.data_ptr()
-    b.state.zero_()
-    st = torch.cuda.current_stream(b.device).cuda_stream  # looked up once: every launch of the loop goes to this stream
-
-    def next_prob(src, dst):
-        b.dev_sweep(MODE_NEXT, src, st)
-        _allreduce(b.red, SUM, group)
-        b.dev_vec(SHARD_FINISH, ln_ptr, src, dst, stream=st)
-
-    def check(scal):
-        if scal[3] != 0:
-            raise ZeroDivisionError("float division by zero")
-        if scal[2] != 0:
-            raise KeyError("allele vanished from next_prob output during SQUAREM step")
-
-    b.dev_sweep(MODE_INIT, -1, st)
-    _allreduce(b.red, SUM, group)
-    b.dev_vec(SHARD_FINISH, ln_ptr, -1, 0, stream=st)
-    diff, it = 1.0, 0
-    while diff > 0.0001 and it < max_iter:
-        next_prob(0, 1)
-        next_prob(1, 2)
-        b.dev_vec(SHARD_SQUAREM, ln_ptr, stream=st)
-        next_prob(3, 4)
-        b.dev_vec(SHARD_ADVANCE, ln_ptr, iteration=it, remove_low=remove_low, stream=st)
-        scal = b.scal.tolist()  # the one host synchronisation of the iteration (64 bytes)
-        check(scal)
-        diff = float(scal[4])
-        it += 1
-    b.dev_vec(SHARD_FINAL, ln_ptr, remove_low=remove_low, stream=st)
-    first = torch.full((b.A,), FK_NONE, dtype=torch.int32, device=b.device)
-    if it > 0:
-        b.dev_sweep(MODE_FIRSTK, 5, st)
-        _allreduce(b.fk, MIN, group)
-        first = torch.where(b.live[4] != 0, b.fk, first)
-    check(b.scal.tolist())
-    return b.vec[1].clone(), b.live[0] != 0, first, it
-
-
-def _allreduce(t, op, group):
-    import torch.distributed as dist
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
-        dist.all_reduce(t, op=op, group=group)
-    return t
-
-
-def single_abundance_sharded(backend, allele_len=None, remove_low=False, group=None, max_iter=1000):
-    """Returns (prob[A], in_result[A] bool, first_key[A] int32, iters) as torch tensors on backend.device.
-    Raises KeyError / ZeroDivisionError where the reference does (common:1365-1369, 1285-1297).
-    Per loop iteration: 3 sweeps + 3 all-reduces of 2*A doubles and two host synchronisations (the SQUAREM branch on
-    sum(v^2) > 0 and the convergence test are host decisions, exactly as in the reference's while loop)."""
-    import torch.distributed as dist
-    if isinstance(backend, CudaSweep):
-        return _single_abundance_sharded_dev(backend, allele_len, remove_low, group, max_iter)
-    SUM = dist.ReduceOp.SUM if dist.is_available() else None
-    MIN = dist.ReduceOp.MIN if dist.is_available() else None
-    dev = backend.device
-    A = backend.A
-    ln = None if allele_len is None else torch.as_tensor(np.asarray(allele_len, np.float64), device=dev)
-    zero = torch.zeros(A, dtype=torch.float64, device=dev)
-    bad = torch.zeros((), dtype=torch.bool, device=dev)  # "normalize() would divide by zero", checked once per iteration
-
-    def reduced_sweep(mode, pm):
-        acc, hit = backend.sweep(mode, pm)
-        both = torch.cat([acc, hit.to(torch.float64)])  # one all-reduce: sums and hit counts
-        _allreduce(both, SUM, group)
-        return both[:A], both[A:] > 0
-
-    def finish(q, keys):
-        nonlocal bad
-        if ln is not None:
-            q = q / ln
-        q = torch.where(keys, q, zero)
-        total = q.sum()
-        bad = bad | (keys.any() & (total == 0))
-        return torch.where(keys, q / total, zero), keys
-
-    def next_prob(p, live):
-        pm = torch.where(live, p, zero)
-        acc, hit = reduced_sweep(MODE_NEXT, pm)
-        return finish(pm * acc, live & hit)
-
-    acc, hit = reduced_sweep(MODE_INIT, None)
-    p0, l0 = finish(acc, hit)
-    diff, it = 1.0, 0
-    last = None
-    while diff > 0.0001 and it < max_iter:
-        p1, l1 = next_prob(p0, l0)
-        p2, l2 = next_prob(p1, l1)
-        r = torch.where(l0, p1 - p0, zero)
-        v = torch.where(l0, p2 - p1 - r, zero)
-        scal = torch.stack([(r * r).sum(), (v * v).sum(), (l0 & ~(l1 & l2)).any().to(torch.float64),
-                            bad.to(torch.float64)]).cpu()  # host sync 1
-        if scal[3] != 0:
-            raise ZeroDivisionError("float division by zero")
-        if scal[2] != 0:
-            raise KeyError("allele vanished from next_prob output during SQUAREM step")
-        ssr, ssv = float(scal[0]), float(scal[1])
-        if ssv > 0.0:
-            g = -np.sqrt(ssr / ssv)
-            p3 = torch.where(l0, torch.clamp(p0 - 2 * g * r + g * g * v, min=0.0), zero)
-            p1, l1 = next_prob(p3, l2)
-            last = (p3, l2)
-        else:
-            last = (p0, l0)
-        d = torch.where(l0, torch.where(l1, (p0 - p1).abs(), p0), zero).sum()
-        p0, l0 = p1, l1
-        if it >= 10 and remove_low:
-            p0, l0 = _prune(p0, l0, zero)
-        diff = float(d)  # host sync 2
-        it += 1
-    if remove_low:
-        p0, l0 = _prune(p0, l0, zero)
-    q = p0 / ln if ln is not None else p0
-    q = torch.where(l0, q, zero)
-    total = q.sum()
-    if bool(bad) or (bool(l0.any()) and float(total) == 0.0):
-        raise ZeroDivisionError("float division by zero")
-    prob = torch.where(l0, q / total, zero)
-    first = torch.full((A,), FK_NONE, dtype=torch.int32, device=dev)
-    if last is not None:
-        pm = torch.where(last[1], last[0], zero)
-        _, fk = backend.sweep(MODE_FIRSTK, pm)
-        _allreduce(fk, MIN, group)
-        first = torch.where(last[1], fk, first)
-    return prob, l0, first, it
-
-
-def _prune(p, live, zero):
-    """select_alleles (common:1338-1346): keep p >= max/10 among the keys; no keys -> nothing to do."""
-    mx = torch.where(live, p, torch.full_like(p, -1.0)).max()
-    keep = live & (p >= mx / 10.0)
-    return torch.where(keep, p, zero), keep
 
 
 class _DevAlias:
@@ -425,14 +197,10 @@ def pileup_allreduce_hook(group=None):
     (the reference derives nt_set from the pileup of ALL reads, common:1124-1134)."""
     import torch.distributed as dist
 
-    class _Alias:
-        def __init__(self, ptr, n):
-            self.__cuda_array_interface__ = {"data": (ptr, False), "shape": (n,), "typestr": "<i4", "version": 2}
-
     @ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p)
     def hook(_arg, dev_counts, n_u32, _stream):
         try:
-            t = torch.as_tensor(_Alias(dev_counts, int(n_u32)), device="cuda")
+            t = _alias(dev_counts, n_u32, "<i4", torch.device("cuda"))
             dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)  # int32 wrap-around == uint32 sum
             torch.cuda.synchronize()
             return 0

@@ -367,10 +367,9 @@ class Batch:
     def sharded_abundance(self, u, table=TABLE_GENE, lengths=None, remove_low=False, group=None, max_n=None):
         """single_abundance over the union of every rank's classes of unit u (read-sharded locus, SURVEY.md 8e).
         Returns (ranked [[allele, prob]] (the first max_n entries when given), iterations); identical on every rank.
-        Default path: the ranks' tables are merged so that every class lives on exactly one rank
-        (em_dist.merge_class_tables), then ONE cooperative kernel per rank runs the whole loop and sums the per-allele
-        accumulators through NVLink peer memory (em_dist.single_abundance_peer).  HGT_SHARD_EM=nccl selects the earlier
-        host-driven loop (partial sweep + NCCL all-reduce per next_prob on the unmerged tables)."""
+        The ranks' tables are merged so that every class lives on exactly one rank (em_dist.merge_class_tables), then ONE
+        cooperative kernel per rank runs the whole loop and sums the per-allele accumulators through NVLink peer memory
+        (em_dist.single_abundance_peer)."""
         import torch
         import torch.distributed as dist
         from . import em_dist
@@ -388,29 +387,22 @@ class Batch:
             dist.all_gather(every, mine, group=group)
             offset = int(sum(int(x) for x in every[:dist.get_rank(group)]))
         ln = None if not lengths else np.asarray([lengths[x] for x in t.names], np.float64)
-        peer = os.environ.get("HGT_SHARD_EM", "peer") != "nccl"
-        if peer:
-            keep = ()
-            if multi:
-                m_bits, m_cnt, m_first, n = em_dist.merge_class_tables(t.A, t.wp, bits, cnt, first, n, offset, dev_index, group)
-                keep = (m_bits, m_cnt, m_first)
-                bits, cnt, first, offset = m_bits.data_ptr(), m_cnt.data_ptr(), m_first.data_ptr(), 0
-            t1 = time.perf_counter()
-            prob, live, fk, iters = em_dist.single_abundance_peer(t.A, t.wp, bits, cnt, first, offset, n, dev_index, ln,
-                                                                  remove_low, group, keep)
-            self.shard_classes = int(n)
-        else:
-            sweep = em_dist.CudaSweep(t.A, bits, n, count_u64_ptr=cnt, key_ptr=first, key_offset=offset, device=self.device)
-            t1 = time.perf_counter()
-            prob, live, fk, iters = em_dist.single_abundance_sharded(sweep, ln, remove_low, group)
-            self.shard_classes = int(n)
+        keep = ()
+        if multi:
+            m_bits, m_cnt, m_first, n = em_dist.merge_class_tables(t.A, t.wp, bits, cnt, first, n, offset, dev_index, group)
+            keep = (m_bits, m_cnt, m_first)
+            bits, cnt, first, offset = m_bits.data_ptr(), m_cnt.data_ptr(), m_first.data_ptr(), 0
+        t1 = time.perf_counter()
+        prob, live, fk, iters = em_dist.single_abundance_peer(t.A, t.wp, bits, cnt, first, offset, n, dev_index, ln,
+                                                              remove_low, group, keep)
+        self.shard_classes = int(n)
         prob, live, fk = prob.cpu().numpy(), live.cpu().numpy().astype(np.uint8), fk.cpu().numpy()
         t2 = time.perf_counter()
         ranked = rank_result(t.names, prob, live, fk, max_n)
         t3 = time.perf_counter()
         # wall-clock split of the call, read by bench.py: set-up (offsets, table merge), EM loop incl. the final copy, ranking
         self.shard_ms = {"setup": (t1 - t0) * 1e3, "em_loop": (t2 - t1) * 1e3, "rank": (t3 - t2) * 1e3,
-                         "em": "peer" if peer else "nccl", "classes": self.shard_classes}
+                         "em": "peer", "classes": self.shard_classes}
         return ranked, iters
 
     def unit_calls(self, u, max_n=None):

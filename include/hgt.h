@@ -135,40 +135,6 @@ typedef struct {
 int hgt_em_form(const hgt_ctx *ctx, int32_t n_classes, int32_t n_alleles, int32_t wp, int32_t has_lengths, int32_t n_ctas,
                 int32_t a_live_max, int32_t n_problems, hgt_em_form_info *out);
 
-/* Read-sharded locus (SURVEY.md 8e): ONE partial sweep of next_prob() over the class rows that live on this device.
- * mode 0: initial mass (common:1299-1309; p_in unused), 1: next_prob E/M sums (common:1311-1331), 2: smallest class
- * key per allele (dict insertion order of the output, common:1324-1331).  p_in[n_alleles] holds the GLOBAL current
- * probabilities with 0 for alleles that are not keys.  acc_out[a] = sum over local classes k with s_k > 0 that hold a
- * of n_k / s_k (n_k / |class| in mode 0); aux_out[a] = 1 if any such class exists (modes 0, 1) or the smallest
- * class_key + key_offset (mode 2; class_key NULL = class index).  The caller all-reduces acc_out (sum) and aux_out
- * (max / min) over the ranks and finishes the step (hisat-genotype_b200/em_dist.py).  Exactly one of the two count
- * arrays is non-NULL.  Device pointers, no synchronisation. */
-size_t hgt_em_partial_workspace_bytes(const hgt_ctx *ctx, int32_t n_alleles);
-int hgt_em_partial_dev(hgt_ctx *ctx, void *stream, const uint64_t *class_bits, const double *class_count_f64,
-                       const uint64_t *class_count_u64, const int32_t *class_key, int32_t key_offset, int32_t n_classes,
-                       int32_t n_alleles, int32_t wp, const double *p_in, int32_t mode, double *acc_out, int32_t *aux_out,
-                       void *workspace);
-
-/* Read-sharded locus, device-resident loop: the O(A) vector half of the reference loop (common:1351-1409) as kernels, so
- * that one iteration costs 3 x (sweep, all-reduce, finish) + squarem + advance and one 64-byte host read.
- * `state` (device, hgt_em_shard_state_bytes(n_alleles), zeroed by the caller before the loop) holds, in this order,
- *   double vec[6][A]  0 Gene_prob, 1 next, 2 next2, 3 extrapolated, 4 next of extrapolated, 5 input of the last next_prob
- *   double red[2A]    the buffer the caller all-reduces (sum): per-allele sums | hit counts of the sweep
- *   double scal[8]    0 sum r^2, 1 sum v^2, 2 KeyError, 3 ZeroDivisionError, 4 prob_diff, 5 third sweep used, 6 keys left
- *   int32 fk[A]       (A rounded up to even) smallest class key of the mode-2 sweep, all-reduced with min
- *   uint8 live[5][A]  key flags of vec 0, 1, 2, 4 and 5
- * hgt_em_shard_sweep_dev = hgt_em_partial_dev with p_in = vec[src] (src < 0 or mode 0: none), results into red (modes 0, 1)
- * or fk (mode 2).  hgt_em_shard_vec_dev op 0 FINISH: vec[dst] = normalize(vec[src] * sums) over keys = live(src) & hit
- * (src < 0: initial mass; src 3 is masked by the keys of vec 2), 1 SQUAREM (common:1361-1383; vec[3], scal 0, 1, 2, 5),
- * 2 ADVANCE (prob_diff into scal[4], Gene_prob = next, select_alleles when iteration >= 10 and remove_low), 3 FINAL
- * (select_alleles + normalize: prob into vec[1], keys in live[0]).  Device pointers, no synchronisation. */
-size_t hgt_em_shard_state_bytes(int32_t n_alleles);
-int hgt_em_shard_sweep_dev(hgt_ctx *ctx, void *stream, const uint64_t *class_bits, const double *class_count_f64,
-                           const uint64_t *class_count_u64, const int32_t *class_key, int32_t key_offset, int32_t n_classes,
-                           int32_t n_alleles, int32_t wp, int32_t mode, int32_t src, void *state, void *workspace);
-int hgt_em_shard_vec_dev(hgt_ctx *ctx, void *stream, int32_t op, int32_t n_alleles, void *state, const double *allele_len,
-                         int32_t src, int32_t dst, int32_t iteration, int32_t remove_low);
-
 /* Read-sharded locus, the whole loop as ONE cooperative launch per rank (one process per GPU).  The reference has no
  * counterpart: it is single_abundance (common:1282-1410) run on class rows that live on several GPUs.  Every rank owns an
  * exchange block (hgt_em_peer_alloc; its 64-byte CUDA IPC handle is passed to the other ranks by the caller, e.g. with

@@ -1,126 +1,17 @@
-"""Distributed control flow of the read-sharded EM (hisat-genotype_b200/em_dist.py) under gloo, world_size 2, CPU only.
+"""The class-table exchange of the read-sharded EM (hisat-genotype_b200/em_dist.py) under gloo, world_size 2, CPU only.
 
-The CUDA sweep is replaced by a numpy sweep over the same bit-matrix layout (test-side code); everything else —
-the all-reduces, normalisation, SQUAREM, pruning, tie keys — is the product code.  The union of the two shards must
-give the single-process oracle result (oracle/em_oracle.py) on the concatenated class table."""
+gather_class_tables is the all_gather in front of hgt_class_merge_dev; the merge and the peer-memory EM behind it need
+GPUs (tests/test_gpu_em.py, tests/test_gpu_multi.py)."""
 import os
 import socket
 import sys
 
 import numpy as np
-import pytest
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-class NumpySweep:
-    """Same contract as em_dist.CudaSweep.sweep on host arrays (test infrastructure)."""
-
-    def __init__(self, members, counts, keys, n_alleles):
-        self.A = n_alleles
-        self.device = torch.device("cpu")
-        self.members, self.counts, self.keys = members, counts, keys
-
-    def sweep(self, mode, p):
-        acc = np.zeros(self.A)
-        aux = np.full(self.A, 0x7FFFFFFF if mode == 2 else 0, np.int32)
-        pv = None if p is None else p.numpy()
-        for mem, n, key in zip(self.members, self.counts, self.keys):
-            s = float(len(mem)) if mode == 0 else float(pv[mem].sum())
-            if not s > 0.0:
-                continue
-            if mode == 2:
-                aux[mem] = np.minimum(aux[mem], key)
-            else:
-                acc[mem] += n / s
-                aux[mem] = 1
-        return torch.from_numpy(acc), torch.from_numpy(aux)
-
-
-def make_problem(seed, n_alleles=90, n_classes=70):
-    rng = np.random.default_rng(seed)
-    members, counts = [], []
-    for _ in range(n_classes):
-        g0 = int(rng.integers(0, n_alleles // 10)) * 10
-        mem = [g0 + j for j in range(10) if rng.random() < 0.55] or [g0]
-        if rng.random() < 0.1:
-            mem = sorted(set(mem) | set(int(x) for x in rng.integers(0, n_alleles, 25)))
-        members.append(np.asarray(mem))
-        counts.append(int(rng.integers(1, 40)))
-    return members, counts
-
-
-def _worker(rank, world, port, seed, remove_low, use_len, out):
-    sys.path.insert(0, ROOT)
-    import _hgt_path
-    _hgt_path.load()
-    from hisatgenotype_b200 import em_dist
-    os.environ["MASTER_ADDR"] = "127.0.0.1"
-    os.environ["MASTER_PORT"] = str(port)
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    members, counts = make_problem(seed)
-    A = 90
-    lo, hi = (0, len(members) // 2) if rank == 0 else (len(members) // 2, len(members))
-    # the first eight classes live on BOTH ranks with their count split (shards of one locus see the same class from
-    # different read pairs): duplicates across shards must not matter once the counts add up
-    idx = list(range(lo, hi))
-    cnt = [counts[k] for k in idx]
-    dup = list(range(8))
-    if rank == 0:
-        cnt = [c // 2 if k in dup else c for k, c in zip(idx, cnt)]
-    else:
-        idx = dup + idx
-        cnt = [counts[k] - counts[k] // 2 for k in dup] + cnt
-    keep = [j for j, c in enumerate(cnt) if c > 0]
-    sweep = NumpySweep([members[idx[j]] for j in keep], [cnt[j] for j in keep], [idx[j] for j in keep], A)
-    ln = (1000.0 + np.arange(A) % 7) if use_len else None
-    prob, live, fk, iters = em_dist.single_abundance_sharded(sweep, ln, remove_low)
-    if rank == 0:
-        out.put((prob.numpy().copy(), live.numpy().copy(), fk.numpy().copy(), iters))
-    dist.barrier()
-    dist.destroy_process_group()
-
-
-@pytest.mark.parametrize("remove_low,use_len", [(False, False), (True, False), (True, True)])
-def test_sharded_em_matches_oracle_world2(remove_low, use_len):
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import em_oracle
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    seed = 11
-    ctx = mp.get_context("spawn")
-    out = ctx.Queue()
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, seed, remove_low, use_len, out)) for r in range(2)]
-    for p in procs:
-        p.start()
-    prob, live, fk, iters = out.get(timeout=120)
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
-    members, counts = make_problem(seed)
-    names = ["A*%03d" % i for i in range(90)]
-    cmpt = {}
-    for mem, n in zip(members, counts):
-        key = "-".join(names[i] for i in sorted(mem))
-        cmpt[key] = cmpt.get(key, 0) + n
-    lengths = {names[i]: 1000.0 + i % 7 for i in range(90)} if use_len else {}
-    ref, ref_iters = em_oracle.single_abundance(cmpt, remove_low, lengths)
-    assert iters == ref_iters
-    got = sorted(((names[i], float(prob[i])) for i in np.nonzero(live)[0]), key=lambda x: -x[1])
-    assert [a for a, _ in got] == [a for a, _ in sorted(ref, key=lambda x: -x[1])] or \
-        sorted(a for a, _ in got) == sorted(a for a, _ in ref)
-    refd = dict(ref)
-    assert set(refd) == set(a for a, _ in got)
-    for a, p in got:
-        # the contract's tolerance (BASELINE.json north_star: abundances within 1e-6 relative); alleles far below
-        # the report threshold (1 %) sit in the cancellation noise of the SQUAREM extrapolation (p0 - 2gr + g^2 v
-        # with terms ~1e-3) whose last bits depend on the association of the partial sums, so they get an absolute bound
-        assert p == pytest.approx(refd[a], rel=1e-6, abs=1e-9)
 
 
 def _gather_worker(rank, world, port, out):

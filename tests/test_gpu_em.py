@@ -133,54 +133,6 @@ def test_em_batch_matches_single():
         np.testing.assert_array_equal(f, fk[s])
 
 
-class _TwoShards:
-    """Two CudaSweep shards summed in-process: what the NCCL all-reduce does between two ranks."""
-
-    def __init__(self, a, b):
-        self.a, self.b = a, b
-        self.A, self.device = a.A, a.device
-
-    def sweep(self, mode, p):
-        import torch
-        acc0, aux0 = self.a.sweep(mode, p)
-        acc1, aux1 = self.b.sweep(mode, p)
-        return acc0 + acc1, (torch.minimum(aux0, aux1) if mode == 2 else torch.maximum(aux0, aux1))
-
-
-@pytest.mark.parametrize("A,C,groups,remove_low,use_len", [
-    (700, 84, 12, True, False),
-    (2000, 500, 40, False, True),
-    (8192, 6000, 64, True, False),
-])
-def test_sharded_em_partial_sweeps(A, C, groups, remove_low, use_len):
-    """em_dist.single_abundance_sharded on hgt_em_partial_dev sweeps: one shard, and two shards with summed partials,
-    against the single-kernel EM (hgt_em) — same iterations, same ranking, abundances within the contract tolerance."""
-    from hisatgenotype_b200 import _lib, em_dist
-    from hisatgenotype_b200.typing_common import em_arrays, rank_result
-    rng = np.random.default_rng(A + C)
-    cmpt, lengths = random_problem(rng, A, C, groups)
-    names = sorted({a for k in cmpt for a in k.split("-")})
-    index = {n: i for i, n in enumerate(names)}
-    keys = list(cmpt)
-    n = len(names)
-    bits = _lib.pack_bits([[index[a] for a in k.split("-")] for k in keys], n)
-    cnt = np.asarray([cmpt[k] for k in keys], np.int64)
-    ln = np.asarray([lengths[a] for a in names], np.float64) if use_len else None
-    prob, inres, fk, iters = em_arrays(bits, cnt, n, ln, remove_low)
-    ref = rank_result(names, prob, inres, fk)
-    h = len(keys) // 3
-    one = em_dist.CudaSweep.from_arrays(bits, cnt, n)
-    two = _TwoShards(em_dist.CudaSweep.from_arrays(bits[:h], cnt[:h], n, np.arange(h, dtype=np.int32)),
-                     em_dist.CudaSweep.from_arrays(bits[h:], cnt[h:], n, np.arange(len(keys) - h, dtype=np.int32), key_offset=h))
-    for backend in (one, two):
-        p2, live2, fk2, it2 = em_dist.single_abundance_sharded(backend, ln, remove_low)
-        res = rank_result(names, p2.cpu().numpy(), live2.cpu().numpy().astype(np.uint8), fk2.cpu().numpy())
-        assert it2 == iters
-        assert [a for a, _ in res] == [a for a, _ in ref]
-        for (_, x), (_, y) in zip(res, ref):
-            assert x == pytest.approx(y, rel=REL, abs=1e-9)
-
-
 @pytest.mark.parametrize("use_len", [False, True])
 @pytest.mark.parametrize("A,C", [(200, 60), (3000, 400), (8192, 3000)])  # the last one runs on all SMs
 def test_em_identical_columns_tie_exactly(A, C, use_len):
@@ -213,10 +165,18 @@ def test_em_identical_columns_tie_exactly(A, C, use_len):
             np.testing.assert_allclose(prob, first, rtol=1e-6, atol=1e-12)  # the row order only moves the last bits (tiny values: SQUAREM cancellation)
 
 
-@pytest.mark.parametrize("A,C,remove_low,use_len", [(700, 300, True, False), (8192, 6000, True, False), (3000, 900, False, True)])
-def test_peer_kernel_single_rank_equals_hgt_em(A, C, remove_low, use_len):
+@pytest.mark.parametrize("A,C,remove_low,use_len,rel,abs_", [
+    pytest.param(700, 300, True, False, 1e-9, 1e-15, id="700-300-True-False"),
+    pytest.param(8192, 6000, True, False, 1e-9, 1e-15, id="8192-6000-True-False"),
+    pytest.param(3000, 900, False, True, 1e-9, 1e-15, id="3000-900-False-True"),
+    # hgt_em runs this shape and 700 x 300 in its one-CTA form, whose sums associate differently from the peer kernel's
+    # cooperative sweep.  The pruned 700 x 300 still agrees to 1e-9; here (no pruning, lengths) SQUAREM carries the
+    # difference to ~2e-9 relative, so this shape is held to the contract tolerance.
+    pytest.param(2000, 500, False, True, REL, 1e-9, id="2000-500-False-True"),
+])
+def test_peer_kernel_single_rank_equals_hgt_em(A, C, remove_low, use_len, rel, abs_):
     """hgt_em_peer_dev with a world of ONE rank: the exchange step only reads the rank's own block, so the result must
-    equal hgt_em (same loop, same sums) - iterations, keys, order and values.  The two-rank case needs two GPUs
+    equal hgt_em (same loop) - iterations, keys, order and values.  The two-rank case needs two GPUs
     (tests/test_gpu_multi.py)."""
     import torch
     from hisatgenotype_b200 import _lib, em_dist
@@ -242,7 +202,7 @@ def test_peer_kernel_single_rank_equals_hgt_em(A, C, remove_low, use_len):
         want = rank_result(names, prob, inres, fk)
         assert [a for a, _ in got] == [a for a, _ in want]
         for (_, x), (_, y) in zip(got, want):
-            assert x == pytest.approx(y, rel=1e-9, abs=1e-15)
+            assert x == pytest.approx(y, rel=rel, abs=abs_)
 
 
 @pytest.mark.parametrize("A,world", [(300, 2), (7000, 3)])

@@ -1,9 +1,8 @@
 """Read-sharded locus on TWO GPUs (SURVEY.md 8e): every rank types its half of the reads of one unit - pileup counts
 all-reduced before the representative-base sets are derived, class tables merged so that every class lives on one rank,
-EM as one cooperative kernel per rank that sums through NVLink peer memory (and, for comparison, as partial sweeps + NCCL
-all-reduce; em_dist.py) - and the union must equal the unsharded run on one GPU: read / pair totals, the merged class table (by
-allele set), identical ranked alleles on both ranks, abundances within 1e-6.  Needs >= 2 visible GPUs (skipped otherwise;
-run with `gpurun --gpus 2`)."""
+EM as one cooperative kernel per rank that sums through NVLink peer memory (em_dist.py) - and the union must equal the
+unsharded run on one GPU: read / pair totals, the merged class table (by allele set), identical ranked alleles on both ranks,
+abundances within 1e-6.  Needs >= 2 visible GPUs (skipped otherwise)."""
 import os
 import pickle
 import socket
@@ -48,14 +47,9 @@ def _worker(rank, world, port, out_dir):
     ranked_again, iters_again = bt.sharded_abundance(0)  # second launch on the same exchange blocks
     peer_classes = bt.shard_ms["classes"]
     assert bt.shard_ms["em"] == "peer"
-    os.environ["HGT_SHARD_EM"] = "nccl"  # the host-driven loop (partial sweep + NCCL all-reduce per next_prob)
-    ranked_nccl, iters_nccl = bt.sharded_abundance(0)
-    assert bt.shard_ms["em"] == "nccl"
-    del os.environ["HGT_SHARD_EM"]
     s = bt.unit_summary(0)
     res = {"reads": s["num_reads"], "pairs": s["num_pairs"], "cmpt": bt.unit_gene_cmpt(0, TC.TABLE_GENE), "ranked": ranked,
-           "iters": iters, "ranked_again": ranked_again, "iters_again": iters_again, "ranked_nccl": ranked_nccl,
-           "iters_nccl": iters_nccl, "peer_classes": peer_classes}
+           "iters": iters, "ranked_again": ranked_again, "iters_again": iters_again, "peer_classes": peer_classes}
     with open(os.path.join(out_dir, "rank%d.pkl" % rank), "wb") as f:
         pickle.dump(res, f)
     bt.close()
@@ -98,10 +92,6 @@ def test_two_gpu_read_sharded_locus_equals_unsharded(tmp_path):
     assert shards[0]["iters"] == s["em_iters"][0]
     for sh in shards:
         assert sh["ranked_again"] == sh["ranked"] and sh["iters_again"] == sh["iters"]
-        assert sh["iters_nccl"] == sh["iters"]
-        assert [a for a, _ in sh["ranked_nccl"]] == [a for a, _ in whole]
-        for (_, x), (_, y) in zip(sh["ranked_nccl"], whole):
-            assert x == pytest.approx(y, rel=1e-6, abs=1e-12)
     # after the merge every class lives on exactly one rank
     assert shards[0]["peer_classes"] + shards[1]["peer_classes"] == len(merged)
     bt.close()
