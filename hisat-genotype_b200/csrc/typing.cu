@@ -22,6 +22,7 @@
 #include <atomic>
 #include <deque>
 #include <memory>
+#include <mutex>
 #include <numeric>
 #include <thread>
 #include <string>
@@ -38,6 +39,7 @@
 #include "bam_dev.cuh"
 #include "bam_dsplit.h"
 #include "bam_kernels.cuh"
+#include "pair_batch.h"
 
 using namespace hgt;
 
@@ -67,6 +69,27 @@ struct hgt_locus {
     int wt_n_alt[2] = {0, 0};
     unsigned char *d_wt = nullptr;
     hgtd::LocusWalk wt_host, wt_dev;
+    // containment relation of the allele names (hgt_locus_set_names), for the pair model.  Loci are shared by batches on
+    // several host threads (one context each): the relation is replaced as a whole under names_mu, never changed in
+    // place except for its lazily made device copy (also under names_mu), and a pair call holds a reference until it
+    // has synchronised, so a replaced relation's device arrays outlive every kernel that reads them.
+    std::mutex names_mu;
+    std::shared_ptr<struct NameRel> names;
+};
+
+// sub(a) = alleles whose name occurs inside a's name (a included), sup(x) = alleles whose name contains x's; CSR in
+// sorted-name index space.  The device copy is made at the first pair call and freed with the relation.
+struct NameRel {
+    std::vector<int64_t> sub_off, sup_off;
+    std::vector<int32_t> sub_idx, sup_idx;
+    int device = -1;
+    int64_t *d_sub_off = nullptr, *d_sup_off = nullptr;
+    int32_t *d_sub_idx = nullptr, *d_sup_idx = nullptr;
+    ~NameRel() {
+        if (device < 0) return;
+        cudaSetDevice(device);
+        cudaFree(d_sub_off); cudaFree(d_sub_idx); cudaFree(d_sup_off); cudaFree(d_sup_idx);
+    }
 };
 
 struct LocusDev {
@@ -178,6 +201,124 @@ extern "C" void hgt_locus_free(hgt_locus *l) {
         cudaFree(l->d_st); cudaFree(l->d_mask); cudaFree(l->d_allele_len); cudaFree(l->d_wt);
     }
     delete l;
+}
+
+// ---- allele names: the name-containment relation of the pair model --------------------------------------------------------
+// The legacy pair model tests `allele in allele_pair` on the key string "a-b"; names hold no '-', so x matches the pair
+// exactly when x's name is a substring of a's or of b's.  That relation is a property of the locus: every substring of
+// every name is looked up in a hash set of the names, O(A len^2) lookups instead of O(A^2) string tests.
+extern "C" int hgt_locus_set_names(hgt_locus *loc, int32_t n, const char *const *names) {
+    if (!loc || !names || n != loc->A) {
+        hgt_set_error("hgt_locus_set_names: need the locus and its %d allele names", loc ? loc->A : 0);
+        return HGT_ERR_ARG;
+    }
+    std::vector<std::string_view> nm((size_t)n);
+    for (int32_t a = 0; a < n; a++) {
+        if (!names[a] || !names[a][0] || strchr(names[a], '-')) {
+            hgt_set_error("hgt_locus_set_names: name %d is empty or contains '-'", a);
+            return HGT_ERR_ARG;
+        }
+        nm[a] = names[a];
+        if (a > 0 && !(nm[a - 1] < nm[a])) {
+            hgt_set_error("hgt_locus_set_names: names must be distinct and in sorted order (name %d)", a);
+            return HGT_ERR_ARG;
+        }
+    }
+    std::unordered_map<std::string_view, int32_t> index;
+    index.reserve((size_t)n * 2);
+    size_t max_len = 0;
+    for (int32_t a = 0; a < n; a++) {
+        index.emplace(nm[a], a);
+        max_len = std::max(max_len, nm[a].size());
+    }
+    auto rel = std::make_shared<NameRel>();
+    std::vector<int64_t> &sub_off = rel->sub_off, &sup_off = rel->sup_off;
+    std::vector<int32_t> &sub_idx = rel->sub_idx, found;
+    sub_off.assign((size_t)n + 1, 0);
+    sup_off.assign((size_t)n + 1, 0);
+    for (int32_t a = 0; a < n; a++) {
+        const std::string_view s = nm[a];
+        found.clear();
+        for (size_t i = 0; i < s.size(); i++)
+            for (size_t len = 1; i + len <= s.size(); len++) {
+                auto it = index.find(s.substr(i, len));
+                if (it != index.end()) found.push_back(it->second);
+            }
+        std::sort(found.begin(), found.end());
+        found.erase(std::unique(found.begin(), found.end()), found.end());
+        sub_idx.insert(sub_idx.end(), found.begin(), found.end());
+        sub_off[a + 1] = (int64_t)sub_idx.size();
+    }
+    std::vector<int32_t> &sup_idx = rel->sup_idx;
+    sup_idx.resize(sub_idx.size());
+    for (int32_t x : sub_idx) sup_off[x + 1]++;
+    for (int32_t a = 0; a < n; a++) sup_off[a + 1] += sup_off[a];
+    std::vector<int64_t> fill(sup_off.begin(), sup_off.end() - 1);
+    for (int32_t a = 0; a < n; a++)  // a ascending: every sup list comes out ascending
+        for (int64_t s = sub_off[a]; s < sub_off[a + 1]; s++) sup_idx[fill[sub_idx[s]]++] = a;
+    std::shared_ptr<NameRel> old;
+    {
+        std::lock_guard<std::mutex> g(loc->names_mu);
+        old.swap(loc->names);
+        loc->names = std::move(rel);
+    }
+    return HGT_OK;  // (old is released here, or by the last pair call still holding it)
+}
+
+static std::shared_ptr<NameRel> locus_names(const hgt_locus *loc) {
+    std::lock_guard<std::mutex> g(const_cast<hgt_locus *>(loc)->names_mu);
+    return loc->names;
+}
+
+extern "C" int hgt_locus_name_subsets(const hgt_locus *loc, int64_t *off, int32_t *idx, int64_t *n_idx) {
+    const std::shared_ptr<NameRel> rel = loc ? locus_names(loc) : nullptr;
+    if (!rel) {
+        hgt_set_error("hgt_locus_name_subsets: no names set on this locus");
+        return HGT_ERR_ARG;
+    }
+    // one relation for the whole read: another thread may replace it between a size query and this call, so idx comes
+    // with its capacity in *n_idx
+    const int64_t n = (int64_t)rel->sub_idx.size();
+    if (idx && (!n_idx || *n_idx < n)) {
+        if (n_idx) *n_idx = n;
+        hgt_set_error("hgt_locus_name_subsets: idx holds fewer than the %lld entries of the relation", (long long)n);
+        return HGT_ERR_ARG;
+    }
+    if (n_idx) *n_idx = n;
+    if (off) memcpy(off, rel->sub_off.data(), rel->sub_off.size() * sizeof(int64_t));
+    if (idx) memcpy(idx, rel->sub_idx.data(), (size_t)n * sizeof(int32_t));
+    return HGT_OK;
+}
+
+// The locus's current relation with its device copy made (on `device`); the caller keeps the reference until its kernels
+// have finished.  The copy is complete before any thread can see it: it is built and published under names_mu.
+static int locus_names_dev(hgt_locus *l, int device, std::shared_ptr<NameRel> *out) {
+    std::lock_guard<std::mutex> g(l->names_mu);
+    std::shared_ptr<NameRel> rel = l->names;
+    if (!rel) {
+        hgt_set_error("hgt_batch_pairs: no allele names set on a locus of the batch (hgt_locus_set_names)");
+        return HGT_ERR_ARG;
+    }
+    if (!rel->d_sub_off) {
+        void *p[4] = {nullptr, nullptr, nullptr, nullptr};
+        const void *src[4] = {rel->sub_off.data(), rel->sub_idx.data(), rel->sup_off.data(), rel->sup_idx.data()};
+        const size_t n[4] = {rel->sub_off.size() * 8, rel->sub_idx.size() * 4, rel->sup_off.size() * 8, rel->sup_idx.size() * 4};
+        cudaError_t e = cudaSuccess;
+        for (int i = 0; i < 4 && e == cudaSuccess; i++) {
+            e = cudaMalloc(&p[i], std::max<size_t>(n[i], 8));
+            if (e == cudaSuccess && n[i]) e = cudaMemcpy(p[i], src[i], n[i], cudaMemcpyHostToDevice);
+        }
+        if (e != cudaSuccess) {
+            for (void *x : p) cudaFree(x);
+            hgt_set_error("hgt_batch_pairs: device copy of the allele names: %s", cudaGetErrorString(e));
+            return HGT_ERR_CUDA;
+        }
+        rel->device = device;
+        rel->d_sub_off = static_cast<int64_t *>(p[0]); rel->d_sub_idx = static_cast<int32_t *>(p[1]);
+        rel->d_sup_off = static_cast<int64_t *>(p[2]); rel->d_sup_idx = static_cast<int32_t *>(p[3]);
+    }
+    *out = std::move(rel);
+    return HGT_OK;
 }
 
 // ---- tables of the record walk as one blob ----------------------------------------------------------------------------------
@@ -1325,6 +1466,14 @@ struct hgt_batch {
     int remove_low = 1;
     PinBuf h_em_args[2];   // kernel-argument staging of the two EM levels
     DevBuf d_em_args[2];
+    // the last hgt_batch_pairs result, complete, for a repeated call (e.g. with a larger cap) on the same tables and names
+    struct {
+        bool valid = false;
+        int32_t table = -1;
+        int64_t max_pairs = -1;
+        std::vector<std::shared_ptr<NameRel>> names;  // per locus of the batch (held: their device copies stay valid)
+        PairResult r;
+    } pairs;
     ~hgt_batch() {
         if (ctx) {
             cudaSetDevice(ctx->device);
@@ -2267,6 +2416,7 @@ static int batch_execute(hgt_batch *b, cudaStream_t st) {
     hgt_ctx *ctx = b->ctx;
     b->executed = false;
     b->finished = false;
+    b->pairs.valid = false;
     if (!b->units.empty()) {
         HGT_CHECK(reads_execute(b, st));
         HGT_CHECK(batch_alloc_tables(b, st));
@@ -2347,6 +2497,7 @@ static int batch_execute(hgt_batch *b, cudaStream_t st) {
 // ---- stage 3: results back; on the hla path the second-level EM over full-length alleles (core:1739-1782) -------
 static int batch_finish(hgt_batch *b, cudaStream_t st) {
     hgt_ctx *ctx = b->ctx;
+    b->pairs.valid = false;
     if (b->skip_em) {
         HGT_CUDA(cudaStreamSynchronize(st));
         b->timer.resolve();
@@ -2860,6 +3011,69 @@ extern "C" int hgt_batch_unit_table_dev(const hgt_batch *b, int64_t unit, int32_
     if (class_count) *class_count = lb.d_count.as<uint64_t>() + base;
     if (class_first) *class_first = lb.d_first.as<int32_t>() + base;
     if (n_classes) *n_classes = (int32_t)std::min<int64_t>(lb.ut_ncls[ut], lb.ut_base[ut + 1] - base);
+    return HGT_OK;
+}
+
+// Diploid pair calls of every unit (pair_batch.cu) on table 0, 1 or 2 of a finished batch, read in place.
+extern "C" int hgt_batch_pairs(hgt_batch *b, int32_t table, int64_t max_pairs, int32_t cap, int32_t *allele_lo,
+                               int32_t *allele_hi, double *prob, int32_t *n_total, int32_t *iters, int32_t *status) {
+    if (!b || !b->finished || table < 0 || table > 2 || max_pairs < 0 || cap < 0 || !n_total || !iters || !status ||
+        (cap > 0 && (!allele_lo || !allele_hi || !prob))) {
+        hgt_set_error("hgt_batch_pairs: bad argument, table outside 0..2 or batch not finished");
+        return HGT_ERR_ARG;
+    }
+    HGT_CUDA(cudaSetDevice(b->ctx->device));
+    std::vector<std::shared_ptr<NameRel>> names(b->lb.size());
+    for (size_t i = 0; i < b->lb.size(); i++)
+        if (!b->lb[i].units.empty()) HGT_CHECK(locus_names_dev(b->lb[i].loc, b->ctx->device, &names[i]));
+    auto &pc = b->pairs;
+    if (!(pc.valid && pc.table == table && pc.max_pairs == max_pairs && pc.names == names)) {
+        pc.valid = false;
+        std::vector<PairUnit> units(b->units.size());
+        for (size_t u = 0; u < b->units.size(); u++) {
+            const UnitHost &U = b->units[u];
+            const LocusBatch &lb = b->lb[U.locus];
+            const hgt_locus *loc = lb.loc;
+            const NameRel &rel = *names[U.locus];
+            const int ut = U.local * 4 + table;
+            const int64_t base = lb.ut_base[ut];
+            PairUnit &P = units[u];
+            P.C = (int32_t)std::min<int64_t>(lb.ut_ncls[ut], lb.ut_base[ut + 1] - base);
+            P.A = loc->A;
+            P.wp = loc->wp;
+            P.bits = lb.d_bits.as<uint64_t>() + (size_t)base * loc->wp;
+            P.count = lb.d_count.as<unsigned long long>() + base;
+            P.first = lb.d_first.as<int32_t>() + base;
+            P.sub_off = rel.d_sub_off; P.sub_idx = rel.d_sub_idx;
+            P.sup_off = rel.d_sup_off; P.sup_idx = rel.d_sup_idx;
+        }
+        HGT_CHECK(hgt_pair_batch_run(b->ctx, b->ctx->stream, units, max_pairs, std::max(cap, 16), &pc.r));
+        pc.table = table;
+        pc.max_pairs = max_pairs;
+        pc.names = std::move(names);
+        pc.valid = true;
+    }
+    const PairResult &r = pc.r;
+    for (size_t u = 0; u < b->units.size(); u++) {
+        n_total[u] = r.n_total[u];
+        iters[u] = r.iters[u];
+        status[u] = r.status[u];
+        const int64_t o = r.off[u];
+        for (int32_t k = 0; k < cap && k < r.n_total[u]; k++) {
+            allele_lo[u * (size_t)cap + k] = r.lo[o + k];
+            allele_hi[u * (size_t)cap + k] = r.hi[o + k];
+            prob[u * (size_t)cap + k] = r.p[o + k];
+        }
+    }
+    return HGT_OK;
+}
+
+extern "C" int hgt_batch_pair_sizes(const hgt_batch *b, int64_t *n_pairs) {
+    if (!b || !n_pairs || !b->pairs.valid) {
+        hgt_set_error("hgt_batch_pair_sizes: no hgt_batch_pairs result on this batch");
+        return HGT_ERR_ARG;
+    }
+    std::copy(b->pairs.r.n_pairs.begin(), b->pairs.r.n_pairs.end(), n_pairs);
     return HGT_OK;
 }
 

@@ -12,12 +12,14 @@ from __future__ import annotations
 
 import bisect
 import ctypes
+import threading
 
 import numpy as np
 
 from . import _lib
 
 _TYPE_CODE = {"single": 0, "deletion": 1, "insertion": 2}
+_NAMES_LOCK = threading.Lock()  # loci are shared by batches on several threads (typing_core.BatchPipeline)
 
 
 class LocusDesc(ctypes.Structure):
@@ -100,6 +102,14 @@ def _bind(L):
     L.hgt_walk_table.argtypes = [vp, i32, vp, vp, vp, vp, vp]
     L.hgt_walk_free.restype = None
     L.hgt_walk_free.argtypes = [vp]
+    L.hgt_locus_set_names.restype = ctypes.c_int
+    L.hgt_locus_set_names.argtypes = [vp, i32, P(ctypes.c_char_p)]
+    L.hgt_locus_name_subsets.restype = ctypes.c_int
+    L.hgt_locus_name_subsets.argtypes = [vp, vp, vp, P(i64)]
+    L.hgt_batch_pairs.restype = ctypes.c_int
+    L.hgt_batch_pairs.argtypes = [vp, i32, i64, i32, vp, vp, vp, vp, vp, vp]
+    L.hgt_batch_pair_sizes.restype = ctypes.c_int
+    L.hgt_batch_pair_sizes.argtypes = [vp, vp]
     L._hgt_typing_bound = True
     return L
 
@@ -353,6 +363,30 @@ class LocusTables:
         self.device = device
         ctx = None if host_only else _lib.ctx(device)
         _lib.check(lib().hgt_locus_create(ctx, ctypes.byref(d), ctypes.byref(self.handle)))
+
+    def ensure_names(self):
+        """Hand the allele names to the library (once): the batched pair model needs which names occur inside which."""
+        if getattr(self, "_names_set", False):
+            return
+        with _NAMES_LOCK:
+            if not getattr(self, "_names_set", False):
+                arr = (ctypes.c_char_p * self.A)(*[n.encode() for n in self.names])
+                _lib.check(lib().hgt_locus_set_names(self.handle, self.A, arr))
+                self._names_set = True
+
+    def name_subsets(self):
+        """(off[A + 1], idx): for allele a, idx[off[a]:off[a + 1]] = the alleles whose name is a substring of a's name."""
+        self.ensure_names()
+        n = ctypes.c_int64(0)
+        _lib.check(lib().hgt_locus_name_subsets(self.handle, None, None, ctypes.byref(n)))
+        off = np.zeros(self.A + 1, np.int64)
+        while True:  # (the names may be replaced by another thread between the size query and the read)
+            idx = np.zeros(max(n.value, 1), np.int32)
+            n.value = idx.size
+            rc = lib().hgt_locus_name_subsets(self.handle, _lib.ptr(off), _lib.ptr(idx), ctypes.byref(n))
+            if rc != _lib.HGT_ERR_ARG or n.value <= idx.size:
+                _lib.check(rc)
+                return off, idx[:n.value]
 
     def mask_of(self, names):
         m = np.zeros(self.wp, np.uint64)

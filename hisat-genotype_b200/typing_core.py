@@ -17,7 +17,7 @@ import numpy as np
 
 from . import _lib
 from .locus import LocusTables, Params, lib
-from .typing_common import rank_result
+from .typing_common import MAX_PAIRS, rank_result
 
 TABLE_GENE, TABLE_EXON, TABLE_PRIMARY = 0, 1, 2
 
@@ -245,9 +245,11 @@ class Batch:
         self._texts = []
 
     def execute(self, stream=None):
+        self._pairs = {}
         self._call(lib().hgt_batch_execute(self.handle, stream))
 
     def finish(self, stream=None):
+        self._pairs = {}
         self._call(lib().hgt_batch_finish(self.handle, stream))
 
     def run(self):
@@ -486,6 +488,93 @@ class Batch:
             names = t.names
             out.append([[names[idx_l[u][i]], prob_l[u][i]] for i in range(k)])
         return out
+
+    # ---- diploid pair calls (the legacy joint_abundance) on the device-resident class tables --------------------------
+    def pair_arrays(self, table=TABLE_GENE, max_pairs=None, cap=64):
+        """hgt_batch_pairs over all units: dict of arrays lo / hi / prob [n_units][cap] (sorted-name indices, pairs in
+        (-p, lo, hi) order), n_total, iters, status, n_pairs (pairs after the first pruning) [n_units].  When a unit has
+        more than cap pairs the call is repeated with a larger cap; the library then answers from the result it kept."""
+        max_pairs = MAX_PAIRS if max_pairs is None else int(max_pairs)
+        for t in {self.loci[i] for i in set(self.unit_locus)}:
+            t.ensure_names()
+        nu = len(self.unit_locus)
+        while True:
+            c = max(int(cap), 1)
+            lo = np.zeros((max(nu, 1), c), np.int32)
+            hi = np.zeros((max(nu, 1), c), np.int32)
+            prob = np.zeros((max(nu, 1), c), np.float64)
+            n = np.zeros(max(nu, 1), np.int32)
+            it = np.zeros(max(nu, 1), np.int32)
+            st = np.zeros(max(nu, 1), np.int32)
+            _lib.check(lib().hgt_batch_pairs(self.handle, int(table), max_pairs, c, _lib.ptr(lo), _lib.ptr(hi), _lib.ptr(prob),
+                                             _lib.ptr(n), _lib.ptr(it), _lib.ptr(st)))
+            need = int(n[:nu].max()) if nu else 0
+            if need <= c:
+                q = np.zeros(max(nu, 1), np.int64)
+                _lib.check(lib().hgt_batch_pair_sizes(self.handle, _lib.ptr(q)))
+                return dict(lo=lo[:nu], hi=hi[:nu], prob=prob[:nu], n_total=n[:nu], iters=it[:nu], status=st[:nu],
+                            n_pairs=q[:nu], max_pairs=max_pairs)
+            cap = need
+
+    def _pair_result(self, r, u, return_iters):
+        st = int(r["status"][u])
+        if st == _lib.HGT_ERR_UNSUPPORTED:
+            raise _lib.HgtError(_lib.HGT_ERR_UNSUPPORTED, "joint_abundance: more than %d allele pairs survive the first "
+                                "pruning" % r["max_pairs"])
+        _lib.check(st)
+        n, iters = int(r["n_total"][u]), int(r["iters"][u])
+        if n == 0:
+            return ({}, iters) if return_iters else {}
+        names = self.loci[self.unit_locus[u]].names
+        out = [["%s-%s" % (names[a], names[b]), p]
+               for a, b, p in zip(r["lo"][u, :n].tolist(), r["hi"][u, :n].tolist(), r["prob"][u, :n].tolist())]
+        # the device orders equal probabilities by index; the reference orders them by the key string
+        i = 0
+        while i < n:
+            j = i + 1
+            while j < n and out[j][1] == out[i][1]:
+                j += 1
+            if j - i > 1:
+                out[i:j] = sorted(out[i:j], key=lambda x: x[0])
+            i = j
+        return (out, iters) if return_iters else out
+
+    def _pairs_cached(self, table, max_pairs):
+        key = (int(table), MAX_PAIRS if max_pairs is None else int(max_pairs))
+        cache = getattr(self, "_pairs", None)
+        if cache is None:
+            cache = self._pairs = {}
+        if key not in cache:
+            cache[key] = self.pair_arrays(table, max_pairs)
+        return cache[key]
+
+    def pair_calls(self, table=TABLE_GENE, max_n=None, return_iters=False, max_pairs=None, errors="raise"):
+        """Diploid pair calls of every unit in one library call (hgt_batch_pairs): per unit what
+        typing_common.joint_abundance(self.unit_gene_cmpt(u, table)) returns - [["a-b", p], ...] by (-p, key), {} for an
+        empty table - cut to max_n entries when given; (value, iterations) with return_iters.  A unit where more than
+        max_pairs (default MAX_PAIRS) pairs survive the first pruning gets joint_abundance's HgtError: raised (errors=
+        "raise", the first such unit) or put in that unit's place in the list (errors="return"), next to the results of
+        the other units."""
+        if errors not in ("raise", "return"):
+            raise ValueError("errors must be 'raise' or 'return'")
+        r = self._pairs_cached(table, max_pairs)
+        out = []
+        for u in range(len(self.unit_locus)):
+            try:
+                v = self._pair_result(r, u, return_iters)
+            except _lib.HgtError as e:
+                if errors == "raise":
+                    raise
+                out.append(e)
+                continue
+            if max_n is not None:
+                v = (v[0][:max_n] if v[0] else v[0], v[1]) if return_iters else (v[:max_n] if v else v)
+            out.append(v)
+        return out
+
+    def unit_pair_calls(self, u, table=TABLE_GENE, return_iters=False, max_pairs=None):
+        """pair_calls for one unit (the batch's call is made once per table and kept until the next execute / finish)."""
+        return self._pair_result(self._pairs_cached(table, max_pairs), u, return_iters)
 
     def add_units_ptr(self, units):
         """[(locus_index, address, n_bytes), ...] in one library call."""

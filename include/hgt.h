@@ -181,6 +181,18 @@ int hgt_class_merge_dev(hgt_ctx *ctx, void *stream, const uint64_t *rows_in, con
 int hgt_pair_em(hgt_ctx *ctx, const uint64_t *class_bits, const int64_t *class_count, int32_t n_classes, int32_t wp,
                 const uint64_t *pair_bits, int32_t n_pairs, const double *p0, double *prob, int32_t *iters);
 
+/* Allele names of a locus, for the batched pair model below: names[n] in sorted-name order (the allele index space),
+ * n == n_alleles, distinct, none empty or containing '-' (the pair key's separator); anything else is HGT_ERR_ARG.  The
+ * library derives once per locus which names occur inside which (the legacy `allele in allele_pair` is a substring test):
+ * a hash set of the names and a lookup of every substring of every name.  Works on host-only loci; the device copy is made
+ * at the first hgt_batch_pairs call on the locus.  Setting the names again replaces the relation.
+ * hgt_locus_name_subsets reads it back as CSR in sorted-name index space: off[n_alleles + 1], idx[*n_idx]; the list of
+ * allele a = the alleles whose name is a substring of a's name, a included, ascending.  NULL arrays: only *n_idx.  With
+ * idx, *n_idx is its capacity in and the relation's length out; too small a capacity is HGT_ERR_ARG with nothing written
+ * (the names may have been replaced since the size query).  off and idx always come from one relation. */
+int hgt_locus_set_names(hgt_locus *loc, int32_t n, const char *const *names);
+int hgt_locus_name_subsets(const hgt_locus *loc, int64_t *off, int32_t *idx, int64_t *n_idx);
+
 /* ---- stage (a): per-read allele compatibility -----------------------------------------------------------
  * Replaces the per-read loop of typing() for index_type == "graph"
  *   reference hisatgenotype_modules/hisatgenotype_typing_core.py:598-1596 (add_count :626-677, add_stat
@@ -338,6 +350,26 @@ int hgt_batch_unit_abundance(const hgt_batch *b, int64_t unit, int32_t cap, int3
  * unit u (0, HGT_ERR_KEY, HGT_ERR_ZERODIV).  The function itself fails only on bad arguments. */
 int hgt_batch_abundances(const hgt_batch *b, int32_t cap, int32_t *allele, double *prob, int32_t *n_total,
                          int32_t *status);
+/* Diploid pair calls (the legacy joint_abundance, hgt_pair_em above) of every unit of a finished batch in one call, on the
+ * class table `table` (0, 1 or 2: the Gene, exon and primary-exon tables of hgt_batch_unit_table) read where the batch
+ * keeps it; no table leaves the device and the batch's rows are not moved.  Per unit, the pairs with p > 0 in
+ * (-p, lo, hi) order: allele_lo / allele_hi (sorted-name indices, lo <= hi) and prob are [n_units][cap], at most cap
+ * entries per unit; n_total[u] = the full count, iters[u] = loop iterations, status[u] = HGT_OK or HGT_ERR_UNSUPPORTED when
+ * more than max_pairs pairs survive the first pruning (that unit's result is then empty; the others are unaffected).  A
+ * unit with an empty table gets n_total 0 and HGT_OK.  HGT_ERR_ARG: batch not finished, table outside 0..2, a locus of the
+ * batch without names (hgt_locus_set_names).  The limit follows typing_common.joint_abundance exactly: that enumeration
+ * tests `total > max_pairs` after adding a candidate's partners, so pairs (a, a) counted after the last test do not count
+ * against it.  The masses, and with them the pruned pair set, are bit-identical to the host enumeration; repeated calls
+ * give bit-identical results and leave every other result of the batch unchanged.  Two synchronisations: the read-back of
+ * the pair counts, and the results (plus one when a unit has more than max(cap, 16) result pairs).  The complete result
+ * is kept on the batch until the next execute / finish: a repeated call with the same table, max_pairs and names (e.g.
+ * with a larger cap after n_total showed it was too small) launches nothing.  Loci may be shared by batches on several
+ * threads; hgt_locus_set_names may run meanwhile (a running call keeps the relation it started with). */
+int hgt_batch_pairs(hgt_batch *b, int32_t table, int64_t max_pairs, int32_t cap, int32_t *allele_lo, int32_t *allele_hi,
+                    double *prob, int32_t *n_total, int32_t *iters, int32_t *status);
+/* Pairs after the first pruning of every unit ([n_units]; 0 for an empty table) in the result hgt_batch_pairs keeps: the
+ * size the unit's loop works on.  HGT_ERR_ARG when the batch holds no such result. */
+int hgt_batch_pair_sizes(const hgt_batch *b, int64_t *n_pairs);
 
 /* ---- native SAM intake (host) -------------------------------------------------------------------------------
  * Replaces, for all loci of a sample at once, the external pipe the reference runs per locus
